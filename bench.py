@@ -6,6 +6,8 @@
                                                              # reference stack on the host cores
   python bench.py --env car --envs-per-gpu 16384            # BASELINE configs[3]
   python bench.py --gpus 8 --envs-per-gpu 8192 [--env car]  # BASELINE configs[4] (under torchrun)
+  python bench.py ... --dump-outputs DIR                     # also write the last timed step's outputs
+                                                             # as DIR/<name>.npy (see dump_outputs)
 
 A "step" is one PPO iteration of the workload (default: data/configs/point-ppo-b200.yaml) on every
 rank: rollout of n_steps x envs-per-gpu env-steps (point: ONE fused kernel), GAE, then 10 epochs of
@@ -67,7 +69,13 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the stand-alone env-step roofline and the "
                     "SB3-host-permutation e2e variant (they do not change value / e2e)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them computed as DIR/<name>.npy (rank 0)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA path's outputs: it needs --impl ours")
     d_envs, d_steps = DEFAULTS[a.env]
     a.envs_per_gpu = a.envs_per_gpu or d_envs
     a.n_steps = a.n_steps or d_steps
@@ -259,34 +267,57 @@ def run_ours(args):
     ctrl.ppo.tensorboard_log = None
     model = ctrl.ppo
     assert model.permutation == "device"
+    up = model.updater
+    built = [t.clone() for t in (up.params, up.exp_avg, up.exp_avg_sq, up.step)]
 
     def iteration():
         model.collect_rollouts()
         model.train()
 
+    def restart():
+        """Put the model back into the state it was built in: seeded parameters, zero Adam state and counters,
+        the environments' seeded first reset.  The update adds the CTAs' partial gradients in L2 in no fixed
+        order, so a minibatch is reproducible to rounding only, and over several iterations the rollouts of two
+        runs drift apart.  Every timed step therefore starts here: it then reads the same inputs in every run."""
+        for t, s in zip((up.params, up.exp_avg, up.exp_avg_sq, up.step), built):
+            t.copy_(s)
+        model._rollout_count = model._train_count = 0
+        model.env.seed(cfg["seed"])
+        model._last_obs = model.env.reset_tensor().clone()   # what collect_rollouts does on a new model
+        model._last_episode_starts = torch.ones(n_envs, dtype=torch.float32, device=dev)
+
     for _ in range(max(args.warmup, 3)):
         iteration()
     barrier()
 
-    # ---- value: device-resident, CUDA events, max over ranks -----------------------------------
+    # ---- value: device-resident, CUDA events around each step, max over ranks ------------------------
+    # restart() lies between the steps, outside the events; env.seed synchronises the stream, so a spin kernel
+    # keeps the device busy while the host enqueues the step (its launches then run back to back as before)
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    launches0 = _lib.launch_count()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    barrier()
-    e0.record()
+    ms, launches = 0.0, 0
     for _ in range(args.steps):
+        restart()
+        barrier()
+        torch.cuda._sleep(10_000_000)
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        launches0 = _lib.launch_count()
+        e0.record()
         iteration()
-    e1.record()
+        e1.record()
+        launches += _lib.launch_count() - launches0
+        e1.synchronize()
+        ms += e0.elapsed_time(e1)
     barrier()
-    ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
+    ms = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms = float(ms.item())
-    launches = _lib.launch_count() - launches0
     value = steps_per_iter * world * args.steps / (ms / 1e3)
     sampler.active = False
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model)   # before anything below steps the model further
 
     # ---- phase split and roofline of the dominant kernel (live CUDA events, same stream) -----------
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
@@ -427,6 +458,37 @@ EP_D2H_BYTES = 100 * 12 + 8
 # 126 MB L2 from one epoch to the next); a single-epoch launch 154.2 MB + 3.9 MB
 UPDATE_KERNEL_DRAM_BYTES = {10: 1152.8e6, 1: 158.05e6}
 ENV_STEP_DRAM_BYTES = 808.1e6      # 318.8 MB read + 489.3 MB written at 2^22 envs (profiles/r01_env_step_ncu_final.txt)
+
+
+DUMP_ROLLOUT_BYTES = 32 << 20
+
+
+def dump_outputs(out_dir, model):
+    """What one timed step hands its caller, as of the last timed step, written as float32 / float64 .npy:
+    the rollout buffer collect_rollouts() fills (observations, actions, rewards, episode starts, values, log
+    probabilities, GAE advantages and returns), the policy parameters train() leaves and the update's logger
+    statistics.  The buffer is n_steps x n_envs deep (107 MB for the default point workload), so it is written
+    for a fixed, seeded sample of environments, every time step of each, at most DUMP_ROLLOUT_BYTES;
+    sample_env_index holds which.  Every timed step starts from the seeded state the model was built in (see
+    restart in run_ours), so two runs with the same arguments feed the path identical inputs and two builds can
+    be compared array by array: the rollout bit for bit, the parameters to the rounding of the update's sums."""
+    import numpy as np
+    import torch
+
+    buf, n_steps, n_envs = model.buf, model.n_steps, model.env.num_envs
+    bytes_per_env = n_steps * sum(v[0, 0].numel() * v.element_size() for v in buf.values())
+    k = min(n_envs, max(1, DUMP_ROLLOUT_BYTES // bytes_per_env))
+    envs = np.sort(np.random.default_rng(0).choice(n_envs, k, replace=False))
+    idx = torch.as_tensor(envs, device=model.device)
+    arrays = {f"rollout_{name}": v.index_select(1, idx) for name, v in buf.items()}
+    arrays["policy_params"] = model.updater.params
+    arrays["train_stats"] = model._train_stats
+    arrays["sample_env_index"] = torch.as_tensor(envs, dtype=torch.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def time_update_kernel(model, dev, batch=BATCH):
