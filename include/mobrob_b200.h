@@ -286,6 +286,24 @@ int mr_ppo_prepare_epochs_device(uint64_t seed, const uint64_t* h_stream_ids, in
                                  int64_t n_samples, int64_t batch_size, int64_t N, int64_t T, double* stats,
                                  int32_t* rows, void* stream);
 
+/* Batched policy evaluation.  Replaces [SB3 2.0.0] common/evaluation.py: evaluate_policy(model, env,
+ * n_eval_episodes, deterministic) over the vectorised env, AFTER the caller's env.reset(): steps every env with the
+ * policy until each env i has finished its target of c_i = (n_episodes + i) / N episodes, exactly as SB3's loop does
+ * (all envs keep stepping until the last target is met), and records those episodes.
+ *   deterministic != 0: the action mean; else mu + exp(log_std) * z, z Philox4x32-10 keyed (seed; env_offset + n,
+ *        noise_offset + t) like the rollout kernels (t = step index within this call)
+ *   last_obs [N][O] f32 in/out: the observation the evaluation starts from; the one it ends on
+ *   ep_r [n_episodes] f64, ep_l [n_episodes] i32, ep_t [n_episodes] i64 out: Monitor's info["episode"] return and
+ *        length and the step index at which the episode ended.  Env i's records fill slots off_i .. off_i + c_i - 1,
+ *        off_i = c_0 + ... + c_{i-1}; SB3's list order is the records sorted by (ep_t, env index).
+ *   steps_taken [1] i64 out: steps S every env has taken.  status [1] i32 out: 1 if max_steps (mandatory: no call runs
+ *        unbounded) ended the evaluation before every target was met (the env is then consistent at S = max_steps).
+ * The point env with the default observation row runs in one fused kernel (two launches); the car and envs with
+ * optional observation keys take one launch plus mr_env_step per step, and synchronise the stream after each step. */
+int mr_evaluate(mr_env* env, const float* params, int deterministic, int64_t n_episodes, int64_t max_steps,
+                uint64_t seed, uint64_t noise_offset, int64_t env_offset, float* last_obs, double* ep_r,
+                int32_t* ep_l, int64_t* ep_t, int64_t* steps_taken, int* status, void* stream);
+
 /* Host-side minibatch index stream (no device work): out[0..n) <- a uniformly random permutation
  * of 0..n-1, a pure function of (seed, stream).  Replaces, for throughput runs, the
  * np.random.permutation call of [SB3 2.0.0] RolloutBuffer.get (reached from

@@ -57,7 +57,8 @@ class Logger:
             except Exception:
                 self.writer = None
 
-    def record(self, key, value):
+    def record(self, key, value, exclude=None):
+        """``exclude`` (SB3: output formats to leave out) is accepted and ignored."""
         self.name_to_value[key] = value
 
     def dump(self, step=0):
@@ -456,6 +457,10 @@ class PPO:
             if self.tensorboard_log:
                 self.logger = Logger(self.verbose, os.path.join(self.tensorboard_log, f"{tb_log_name}_1"))
         self._total_timesteps = total_timesteps + self._num_timesteps_at_start
+        if isinstance(callback, list):   # BaseAlgorithm._init_callback
+            from .callbacks import CallbackList
+
+            callback = CallbackList(callback)
         if callback is not None and hasattr(callback, "init_callback"):
             callback.init_callback(self)
             callback.on_training_start(locals(), globals())

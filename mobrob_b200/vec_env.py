@@ -84,6 +84,9 @@ class GpuVecEnv:
         self._actions = None
         self._needs_first_reset = True
         self._seed = None
+        # VecEnv steps taken so far by evaluate_policy's device path: the Philox counter at which the next stochastic
+        # evaluation on this env starts, so that consecutive evaluations never reuse a draw
+        self.eval_steps = 0
         self.t_start = time.time()
         if seed is not None:
             self.seed(seed)
