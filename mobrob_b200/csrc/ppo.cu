@@ -302,7 +302,7 @@ train_summary_kernel(const float* __restrict__ info, int n_rows, const float* __
     }
 }
 
-// One packed record per buffer row (tc::Rec): [obs | ret | 0.. | 1 | a0 a1 old_logp adv | ret 0 0 0].
+// One packed record per buffer row (tc::Rec): [obs | 0.. | 1 at KP-1 | a0 a1 old_logp adv | ret 0 0 0].
 // One thread per (row, 16-byte quad of the record): coalesced 16-byte stores, gathers hit L1 / L2.
 __global__ void __launch_bounds__(256)
 pack_samples_kernel(const float* __restrict__ obs, const float* __restrict__ act, const float* __restrict__ old_logp,
@@ -318,7 +318,7 @@ pack_samples_kernel(const float* __restrict__ obs, const float* __restrict__ act
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
             const int k = 4 * qd + e;
-            v[e] = k < O ? obs[r * O + k] : (k == O ? ret[r] : (k == KP - 1 ? 1.f : 0.f));
+            v[e] = k < O ? obs[r * O + k] : (k == KP - 1 ? 1.f : 0.f);
         }
     } else if (4 * qd == KP) {
         v[0] = act[2 * r]; v[1] = act[2 * r + 1]; v[2] = old_logp[r]; v[3] = adv[r];
@@ -666,7 +666,7 @@ __global__ void __launch_bounds__(tc::THREADS, 1) ppo_epoch_tc_kernel(EpochArgs 
         }
 
         // ---- the whole reduced gradient: clip coefficient, then Adam on the own tower -------------------
-        tc::BlockRegs gOwn, gOth;
+        tc::BlockRegs<KP> gOwn, gOth;
         tc::load_block(src + (size_t)C.tower * TL.size, TL, gOwn);
         tc::load_block(src + (size_t)(C.tower ^ 1) * TL.size, TL, gOth);
         MR_TR(30);
@@ -690,7 +690,7 @@ __global__ void __launch_bounds__(tc::THREADS, 1) ppo_epoch_tc_kernel(EpochArgs 
                 float* row = E.info + 8 * m;
                 if (tid == 0) { row[0] = total_norm; row[1] = K.coef; row[2] = (float)step; row[3] = ent_loss; }
 #pragma unroll
-                for (int k = 0; k < 2; ++k)
+                for (int k = 0; k < tc::BlockRegs<KP>::NR; ++k)
                     if (tid + k * tc::THREADS == q_st) {   // policy: loss, clipped count, kl; value: squared error
                         row[4] = gOwn.r[k].x * inv_cnt; row[5] = gOth.r[k].x * inv_cnt;
                         row[6] = gOwn.r[k].y * inv_cnt; row[7] = gOwn.r[k].z * inv_cnt;
@@ -706,7 +706,10 @@ __global__ void __launch_bounds__(tc::THREADS, 1) ppo_epoch_tc_kernel(EpochArgs 
                     const float v8[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
 #pragma unroll
                     for (int e = 0; e < 8; ++e) E.grad[p + e] = v8[e];
-                    const int qi = idx;
+                }
+#pragma unroll
+                for (int k = 0; k < tc::BlockRegs<KP>::NR; ++k) {
+                    const int qi = tid + k * tc::THREADS;
                     const float r4[4] = {gOwn.r[k].x, gOwn.r[k].y, gOwn.r[k].z, gOwn.r[k].w};
                     if (qi < ((TL.size - TL.w1) >> 2)) {
 #pragma unroll
@@ -996,7 +999,7 @@ int mr_ppo_record_floats(int obs_dim) { return (obs_dim + 1 <= 16 ? 16 : 32) + 8
 int mr_ppo_pack_samples(int obs_dim, const float* obs, const float* act, const float* old_logp, const float* adv,
                         const float* ret, int64_t n_rows, float* rec, void* stream) {
     MR_REQUIRE(obs && act && old_logp && adv && ret && rec, "NULL argument");
-    MR_REQUIRE(obs_dim > 0 && obs_dim < 31, "obs_dim out of range (the record keeps ret at column obs_dim and 1 at KP - 1)");
+    MR_REQUIRE(obs_dim > 0 && obs_dim < MAX_OBS, "obs_dim out of range (1..31: the record's row of X is obs and the ones column)");
     MR_REQUIRE(n_rows > 0, "empty buffer");
     const int kp = obs_dim + 1 <= 16 ? 16 : 32;
     const int64_t quads = n_rows * ((kp + 8) >> 2);
@@ -1014,7 +1017,7 @@ int mr_ppo_epoch_fused(float* params, float* exp_avg, float* exp_avg_sq, int64_t
                        float* grad, float* info, mr_xchg* xchg, void* stream) {
     MR_REQUIRE(params && exp_avg && exp_avg_sq && step && rec && rows && stats && partials && grad,
                "NULL argument");   // perm may be NULL: rows then already hold the epoch's samples (mr_ppo_prepare_epochs)
-    MR_REQUIRE(obs_dim > 0 && obs_dim < 31, "obs_dim out of range (the packed records need obs_dim < 31)");
+    MR_REQUIRE(obs_dim > 0 && obs_dim < MAX_OBS, "obs_dim out of range (1..31: the row of X is obs and the ones column)");
     MR_REQUIRE(batch_size > 0 && n_samples > 0, "empty batch");
     MR_REQUIRE(n_samples < (int64_t(1) << 31) && N * T < (int64_t(1) << 31), "samples are indexed with 32 bits");
     cudaStream_t s = (cudaStream_t)stream;

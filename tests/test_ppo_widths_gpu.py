@@ -1,0 +1,233 @@
+"""The PPO update at every observation width against autograd and SB3's arithmetic.
+
+The update kernels are instantiated for KP = 16 (O <= 15) and KP = 32 (16 <= O <= 31): the row of X is the
+observation padded to KP columns with the ones column (b1) at KP - 1.  What depends on the width -- the packed
+records, the odd-width gather of the per-launch path, the tower-local layout and its flat order, the dW1 staging,
+the ones column -- is held here to a reference at the edges: both instantiations and their boundary (15 / 16),
+odd widths, every width a real env config produces (14 - 23 point, 26 - 29 car) and the top of the range.
+"""
+import copy
+
+import numpy as np
+import pytest
+import torch
+
+from oracle import sb3_oracle
+from perm_ref import device_permutation
+from test_policy_gae_gpu import _forward
+from test_ppo_update_gpu import RTOL, _autograd_grad, _make_problem, _updater
+
+pytestmark = pytest.mark.gpu
+
+WIDTHS = [1, 2, 7, 13, 14, 15, 16, 17, 23, 26, 27, 29, 30, 31]
+KW = dict(clip_range=0.2, ent_coef=0.05, vf_coef=0.5, normalize_advantage=True)
+
+
+def _kp(O):
+    return 16 if O + 1 <= 16 else 32
+
+
+def _dev(buf):
+    return {k: torch.as_tensor(v).cuda().contiguous() for k, v in buf.items()}
+
+
+@pytest.mark.parametrize("O", range(1, 32))
+def test_packed_record_layout(cuda_lib, O):
+    """[obs | 0 .. | 1 at KP-1 | a0 a1 old_logp adv | ret 0 0 0], bit exact, on 7 x 13 = 91 rows."""
+    from mobrob_b200.updater import PpoUpdater
+
+    T, N = 7, 13
+    rng = np.random.default_rng(O)
+    buf = dict(obs=rng.standard_normal((T, N, O)), actions=rng.standard_normal((T, N, 2)),
+               log_probs=rng.standard_normal((T, N)), advantages=rng.standard_normal((T, N)),
+               returns=rng.standard_normal((T, N)) + 3.0)
+    buf = {k: v.astype(np.float32) for k, v in buf.items()}
+    up = PpoUpdater(O, torch.device("cuda", 0))
+    KP = _kp(O)
+    assert int(cuda_lib.mr_ppo_record_floats(O)) == KP + 8
+    rec = up.pack(_dev(buf)).cpu().numpy().reshape(T * N, KP + 8)
+    want = np.zeros((T * N, KP + 8), np.float32)
+    want[:, :O] = buf["obs"].reshape(T * N, O)   # buffer rows are time-major: row t * N + n
+    want[:, KP - 1] = 1.0
+    want[:, KP:KP + 2] = buf["actions"].reshape(T * N, 2)
+    want[:, KP + 2] = buf["log_probs"].reshape(-1)
+    want[:, KP + 3] = buf["advantages"].reshape(-1)
+    want[:, KP + 4] = buf["returns"].reshape(-1)
+    np.testing.assert_array_equal(rec, want)
+
+
+def test_obs_dim_32_is_refused(cuda_lib):
+    from mobrob_b200 import _lib
+    from mobrob_b200.updater import PpoUpdater
+
+    with pytest.raises(ValueError, match="1..31"):
+        PpoUpdater(32, torch.device("cuda", 0))
+    x = torch.zeros(64, device="cuda")
+    with pytest.raises(_lib.MobrobError, match="1..31"):
+        _lib.check(cuda_lib.mr_ppo_pack_samples(32, x.data_ptr(), x.data_ptr(), x.data_ptr(), x.data_ptr(),
+                                                x.data_ptr(), 1, x.data_ptr(), torch.cuda.current_stream().cuda_stream))
+
+
+def _assert_grad_matches(pol, gp, g_ref, g_64):
+    """test_minibatch_gradient_matches_autograd's rule: norm-wise within RTOL of torch's float32 gradient, and per
+    tensor within 3x torch's own float32 distance from the float64 gradient, on the tensor's scale (2e-6 at least).
+
+    That test also asks for 2x torch's distance or 1e-5; only its 3x assertion is kept here, because one tensor
+    exceeds 2x at one width.  It is the tensor that test documents as ill-conditioned in float32: d loss /
+    d value_net.bias = mean(V - R) cancels.  At O = 2, B = 999 (fused) torch's float32 result is 9.0e-6 from float64
+    on the tensor's scale and ours 1.9e-5 (2.1x), measured on a B200 (1000 W), and the same before the epoch
+    kernel's width fixes: its L2 adds the CTAs' partial sums in no fixed order."""
+    gmax = np.abs(g_ref).max()
+    err = np.abs(gp - g_ref).max() / gmax
+    assert err < RTOL, f"gradient error {err:.2e}"
+    off = 0
+    for name in sb3_oracle.PARAM_ORDER:
+        n = dict(pol.named_parameters())[name].numel()
+        sl = slice(off, off + n)
+        scale = max(np.abs(g_64[sl]).max(), 1e-2 * gmax)
+        e = np.abs(gp[sl] - g_64[sl]).max() / scale
+        e_torch = np.abs(g_ref[sl] - g_64[sl]).max() / scale
+        assert e < max(3 * e_torch, 2e-6), f"{name}: {e:.2e} (torch float32 vs float64: {e_torch:.2e})"
+        off += n
+
+
+def _assert_tail_matches(tail, st):
+    np.testing.assert_allclose(tail[0], st["policy_loss"], rtol=1e-4, atol=1e-6)
+    np.testing.assert_allclose(tail[1], st["value_loss"], rtol=1e-5)
+    np.testing.assert_allclose(tail[2], st["clip_fraction"], atol=1e-6)
+    np.testing.assert_allclose(tail[3], st["approx_kl"], rtol=1e-3, atol=1e-6)
+
+
+# (T, N, B): one partial tile; not a multiple of 128; more tiles (157) than CTAs, ragged last tile
+_SIZES = [(16, 64, 100), (16, 64, 999), (160, 128, 20000)]
+_CASES = [(O, *s) for O in WIDTHS for s in _SIZES] + [(O, 296, 64, 18944) for O in (15, 26)]   # + the bench minibatch
+
+
+@pytest.mark.parametrize("path", ["fused", "launches"])
+@pytest.mark.parametrize("O,T,N,B", _CASES)
+def test_one_minibatch_gradient_matches_autograd(cuda_lib, path, O, T, N, B):
+    """One minibatch through the epoch kernel (train_epoch_fused on a perm slice of exactly B samples: the kernel
+    leaves that minibatch's pre-clip mean-loss gradient, flat order, in `grad`) or through mr_ppo_grad."""
+    pol, buf = _make_problem(O, T, N, seed=O + T)
+    up = _updater(pol, O, **KW)
+    dbuf = _dev(buf)
+    perm = np.random.default_rng(O).permutation(N * T).astype(np.int64)[:B]
+    dperm = torch.as_tensor(perm).cuda()
+    stats = up.adv_stats(dbuf["advantages"], dperm, B, N, T)
+    g_ref, st = _autograd_grad(pol, buf, perm, KW, torch.float32)   # what SB3 computes
+    g_64, _ = _autograd_grad(pol, buf, perm, KW, torch.float64)     # what it approximates
+    assert st["clip_fraction"] > 0.0   # the problem exercises the clipped branch
+    if path == "fused":
+        info = torch.zeros((1, 8), device="cuda")
+        up.train_epoch_fused(dbuf, dperm, stats, B, N, T, info)
+        g = up.grad.cpu().numpy()
+        info = info.cpu().numpy()[0]
+        norm = np.linalg.norm(g_ref.astype(np.float64))
+        np.testing.assert_allclose(info[0], norm, rtol=1e-4)
+        np.testing.assert_allclose(info[1], min(0.5 / (norm + 1e-6), 1.0), rtol=1e-4)
+        assert info[2] == 1.0
+        np.testing.assert_allclose(info[3], st["entropy_loss"], rtol=1e-5)
+        _assert_tail_matches(info[4:], st)
+        assert int(up.step[0]) == 1
+    else:
+        g = up.compute_grad(dbuf, dperm, stats[0], N, T).cpu().numpy()
+    _assert_grad_matches(pol, g[:up.n_params], g_ref, g_64)
+    _assert_tail_matches(g[up.stride - 16:], st)
+
+
+@pytest.mark.parametrize("O", [15, 23, 26, 29, 31])
+def test_three_epochs_match_sb3_arithmetic(cuda_lib, O):
+    """3 epochs of 4.4 minibatches (the last one short) with host permutations: the epoch kernel and the per-minibatch
+    launches against SB3's PPO.train on torch CPU (float32): parameters, per-minibatch statistics, Adam moments."""
+    T, N, B, E = 64, 48, 700, 3
+    pol, buf = _make_problem(O, T, N, seed=O + 5)
+    p0 = pol.flat_params().numpy().copy()
+    a, b = _updater(pol, O, **KW), _updater(pol, O, **KW)
+    dbuf = _dev(buf)
+    rng = np.random.default_rng(O)
+    perms = [rng.permutation(N * T).astype(np.int64) for _ in range(E)]
+    n_mb = (N * T + B - 1) // B
+    ia, ib = torch.zeros((E * n_mb, 8), device="cuda"), torch.zeros((E * n_mb, 8), device="cuda")
+    for e, perm in enumerate(perms):
+        dperm = torch.as_tensor(perm).cuda()
+        stats = a.adv_stats(dbuf["advantages"], dperm, B, N, T)
+        a.train_epoch(dbuf, dperm, stats, B, N, T, ia[e * n_mb:(e + 1) * n_mb])
+        b.train_epoch_fused(dbuf, dperm, stats, B, N, T, ib[e * n_mb:(e + 1) * n_mb])
+    ref = copy.deepcopy(pol)
+    opt = sb3_oracle.make_adam(ref)
+    st = sb3_oracle.train_epochs(ref, opt, buf, E, B, perms=perms, clip_range=0.2, ent_coef=0.05, vf_coef=0.5)
+    p_ref = ref.flat_params().numpy()
+    m_ref = torch.cat([opt.state[q]["exp_avg"].reshape(-1) for q in opt.param_groups[0]["params"]]).numpy()
+    moved = np.abs(p_ref - p0).max()
+    assert moved > 5e-4
+    for name, up, info in (("launches", a, ia), ("fused", b, ib)):
+        assert int(up.step[0]) == E * n_mb, name
+        err = np.abs(up.params.cpu().numpy() - p_ref).max()
+        assert err < 2e-3 * moved + 1e-7, f"{name}: parameters {err:.2e} from SB3's (update {moved:.2e})"
+        info = info.cpu().numpy()
+        np.testing.assert_allclose(info[:, 0], [s["grad_norm"] for s in st], rtol=1e-3, err_msg=name)
+        np.testing.assert_allclose(info[:, 5], [s["value_loss"] for s in st], rtol=1e-3, err_msg=name)
+        np.testing.assert_allclose(up.exp_avg.cpu().numpy(), m_ref, rtol=1e-3, atol=1e-7, err_msg=name)
+
+
+_ALL = {"observe_goal_dist": True, "observe_qpos": True, "observe_qvel": True, "observe_ctrl": True}
+
+
+@pytest.mark.parametrize("env_name,cfg,O,B", [
+    ("point", {"observe_goal_dist": True}, 15, 512),
+    ("point", {"observe_goal_dist": True}, 15, 500),   # 2048 = 4 x 500 + 48: one launch per epoch
+    ("point", {"observe_ctrl": True}, 16, 512),
+    ("point", _ALL, 23, 512),
+    ("car", None, 26, 512),
+    ("car", {"observe_goal_dist": True, "observe_ctrl": True}, 29, 512),
+], ids=["point15", "point15-ragged", "point16", "point23", "car26", "car29"])
+def test_learn_iteration_matches_sb3_arithmetic(cuda_lib, env_name, cfg, O, B):
+    """One PPO.learn() iteration with the default settings -- device index streams; the whole update in one
+    cooperative launch when the minibatches are whole -- replayed by SB3's PPO.train on the rollout it collected,
+    with the permutations rebuilt from (seed, stream ids)."""
+    from mobrob_b200 import GpuVecEnv
+    from mobrob_b200.ppo import PPO
+
+    n_envs, T, E, seed = 64, 32, 3, 7
+    env = GpuVecEnv(env_name, n_envs, seed=None, time_limit=100, terminate_on_goal=True, robot_config=cfg)
+    model = PPO("MlpPolicy", env, n_steps=T, batch_size=B, n_epochs=E, seed=seed, gae_lambda=0.5, ent_coef=0.05)
+    assert model.updater.obs_dim == O
+    ref = sb3_oracle.MlpPolicyOracle(O)
+    ref.load_state_dict({k: v.cpu() for k, v in model.policy.state_dict().items()})
+    p0 = ref.flat_params().numpy().copy()
+    stream_ids = model._stream_ids()
+    model.learn(total_timesteps=n_envs * T)
+    torch.cuda.synchronize()
+    assert model._train_count == 1
+    buf = {k: v.cpu().numpy() for k, v in model.buf.items()}
+    perms = [device_permutation(seed, s, n_envs * T) for s in stream_ids]
+    opt = sb3_oracle.make_adam(ref)
+    st = sb3_oracle.train_epochs(ref, opt, buf, E, B, perms=perms, clip_range=0.2, ent_coef=0.05, vf_coef=0.5)
+    p_ref = ref.flat_params().numpy()
+    p = model.updater.params.cpu().numpy()
+    moved = np.abs(p_ref - p0).max()
+    assert moved > 5e-4
+    assert np.abs(p - p_ref).max() < 2e-3 * moved + 1e-7, (np.abs(p - p_ref).max(), moved)
+    tails, log = model._train_log
+    assert tails.shape[0] == len(st)
+    np.testing.assert_allclose(tails[:, 1].cpu().numpy(), [s["value_loss"] for s in st], rtol=1e-3)
+    np.testing.assert_allclose(log[:, 0].cpu().numpy(), [s["grad_norm"] for s in st], rtol=1e-3)
+
+
+@pytest.mark.parametrize("O", range(1, 32))
+def test_policy_forward_every_width(cuda_lib, O):
+    """mr_policy_forward (the rollout and evaluation kernels' MLP, mlp.cuh) at every width, incl. K % 4 != 0."""
+    torch.manual_seed(O)
+    pol = sb3_oracle.MlpPolicyOracle(O)
+    with torch.no_grad():
+        pol.log_std.copy_(torch.tensor([-0.3, 0.4]))
+    n = 333
+    obs = torch.randn(n, O) * 2.0
+    eps = torch.randn(n, 2)
+    with torch.no_grad():
+        a_ref, v_ref, lp_ref = pol.forward_with_noise(obs, eps)
+    act, logp, val = _forward(cuda_lib, pol.flat_params().cuda().contiguous(), O, obs.cuda(), eps.cuda())
+    scale = max(1.0, float(a_ref.abs().max()))
+    assert float((act - a_ref).abs().max()) <= 1e-5 * scale
+    np.testing.assert_allclose(val.numpy(), v_ref.numpy(), rtol=1e-5, atol=1e-5)
+    np.testing.assert_allclose(logp.numpy(), lp_ref.numpy(), rtol=1e-5, atol=1e-5)
