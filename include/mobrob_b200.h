@@ -242,9 +242,9 @@ void mr_xchg_destroy(mr_xchg* x);
 /* *timed_out <- 1 if an in-kernel exchange gave up waiting for a peer since creation (synchronous read) */
 int mr_xchg_status(mr_xchg* x, int* timed_out);
 /* The epoch kernel gathers its minibatches from PACKED sample records, one per buffer row (t * N + n):
- * mr_ppo_record_floats(obs_dim) floats = [obs | ret | 0.. | 1 | a0 a1 old_logp adv | ret 0 0 0] (96 B for
+ * mr_ppo_record_floats(obs_dim) floats = [obs | 0.. | 1 | a0 a1 old_logp adv | ret old_value 0 0] (96 B for
  * the point robot, 160 B for the car).  mr_ppo_pack_samples builds them once per rollout (after GAE) from
- * the RolloutBuffer arrays; rec is caller-owned, n_rows * mr_ppo_record_floats floats. */
+ * the RolloutBuffer arrays, with old_value = 0; rec is caller-owned, n_rows * mr_ppo_record_floats floats. */
 int mr_ppo_record_floats(int obs_dim);
 int mr_ppo_pack_samples(int obs_dim, const float* obs, const float* act, const float* old_logp, const float* adv,
                         const float* ret, int64_t n_rows, float* rec, void* stream);
@@ -254,6 +254,53 @@ int mr_ppo_epoch_fused(float* params, float* exp_avg, float* exp_avg_sq, int64_t
                        float clip_range, float ent_coef, float vf_coef, int normalize_adv, float lr,
                        float beta1, float beta2, float eps, float max_grad_norm, float* partials,
                        float* grad, float* info, mr_xchg* xchg, void* stream);
+
+/* ------------------------------------------------------------------------------------
+ * [SB3] PPO's clip_range_vf and target_kl.  The *_ex / *_vf entry points take the arguments of the calls above
+ * plus the following; with clip_range_vf <= 0, target_kl <= 0 and ctrl = NULL they compute exactly what those do.
+ *   clip_range_vf > 0: value_loss = mse(returns, old_value + clamp(V - old_value, -c, c)), old_value being the
+ *       rollout's values [T][N] (RolloutBuffer.values): passed as old_values to the per-launch calls, packed into
+ *       the records by mr_ppo_pack_samples_vf for the fused one.
+ *   target_kl > 0: per minibatch, after its losses and statistics, approx_kl > 1.5 * target_kl (compared in
+ *       double) stops the update: that minibatch is not applied and no later one runs.
+ *   ctrl: the update's control word, one int32 of caller-owned device memory, zero before the update's first
+ *       call (the caller clears it once per update).  A stop after the k-th minibatch of the update (counted over
+ *       all its calls from mb0 / mb_index = 0) sets it to k; every later call of the update then returns at entry
+ *       in its kernels and changes nothing.  Required with target_kl > 0.
+ * After a stop the info row of the stopping minibatch holds its statistics with the unchanged step count, and
+ * `grad` holds its gradient (the fused call: also when a later launch of the update returns at entry; the per-launch
+ * calls: on one GPU -- a host all-reduce of later minibatches still sums the unchanged vector). */
+int mr_ppo_pack_samples_vf(int obs_dim, const float* obs, const float* act, const float* old_logp, const float* adv,
+                           const float* ret, const float* values, int64_t n_rows, float* rec, void* stream);
+int mr_ppo_epoch_fused_ex(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
+                          const float* rec, const int64_t* perm, int32_t* rows, int64_t n_samples,
+                          int64_t batch_size, const double* stats, int64_t N, int64_t T,
+                          float clip_range, float ent_coef, float vf_coef, int normalize_adv, float lr,
+                          float beta1, float beta2, float eps, float max_grad_norm, float* partials,
+                          float* grad, float* info, mr_xchg* xchg, float clip_range_vf, float target_kl, int* ctrl,
+                          int64_t mb0, void* stream);
+int mr_ppo_grad_ex(const float* params, int obs_dim, const float* obs, const float* act,
+                   const float* old_logp, const float* adv, const float* ret, const int64_t* perm,
+                   int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
+                   float clip_range, float ent_coef, float vf_coef, int normalize_adv, float rank_share,
+                   float* partials, float* grad, const float* old_values, float clip_range_vf, const int* ctrl,
+                   void* stream);
+int mr_adam_step_ex(float* params, float* exp_avg, float* exp_avg_sq, const float* grad, int n_params,
+                    int64_t* step, float lr, float beta1, float beta2, float eps, float max_grad_norm,
+                    float* info, float target_kl, int* ctrl, int64_t mb_index, void* stream);
+int mr_ppo_train_epoch_ex(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
+                          const float* obs, const float* act, const float* old_logp, const float* adv,
+                          const float* ret, const int64_t* perm, int32_t* rows, int64_t n_samples,
+                          int64_t batch_size, const double* stats, int64_t N, int64_t T, float clip_range,
+                          float ent_coef, float vf_coef, int normalize_adv, float lr, float beta1, float beta2,
+                          float eps, float max_grad_norm, float* partials, float* grad, float* info,
+                          const float* old_values, float clip_range_vf, float target_kl, int* ctrl, int64_t mb0,
+                          void* stream);
+/* mr_ppo_train_summary over the minibatches the update evaluated: with ctrl != NULL recording a stop after k
+ * minibatches, the means cover rows [0, k), "last" is row k - 1, out[11] = k, and out[12] = row k - 1's
+ * approx_kl (out then has 13 floats).  ctrl = NULL: all n_rows, out [12], as mr_ppo_train_summary. */
+int mr_ppo_train_summary_ex(const float* info, int n_rows, const float* values, const float* returns, int64_t n,
+                            const float* params, float* out, double* scratch, const int* ctrl, void* stream);
 
 /* Same contract as mr_rollout, from the stand-alone env-step kernel plus ONE kernel between two env steps (the
  * finished step's RolloutBuffer.add bookkeeping -- time-out bootstrap, reward row, Monitor ring, start flags -- and

@@ -71,6 +71,19 @@ _SIGNATURES = {
     "mr_host_permutation": (c_int, [c_uint64, c_uint64, c_int64, _P]),
     "mr_adam_step": (c_int, [_P, _P, _P, _P, c_int, _P, c_float, c_float, c_float, c_float, c_float,
                              _P, _P]),
+    # clip_range_vf / target_kl (include/mobrob_b200.h): the calls above plus their trailing arguments
+    "mr_ppo_pack_samples_vf": (c_int, [c_int, _P, _P, _P, _P, _P, _P, c_int64, _P, _P]),
+    "mr_ppo_epoch_fused_ex": (c_int, [_P, _P, _P, _P, c_int, _P, _P, _P, c_int64, c_int64, _P,
+                                      c_int64, c_int64, c_float, c_float, c_float, c_int, c_float, c_float,
+                                      c_float, c_float, c_float, _P, _P, _P, _P, c_float, c_float, _P, c_int64, _P]),
+    "mr_ppo_grad_ex": (c_int, [_P, c_int, _P, _P, _P, _P, _P, _P, _P, c_int64, _P, c_int64, c_int64,
+                               c_float, c_float, c_float, c_int, c_float, _P, _P, _P, c_float, _P, _P]),
+    "mr_adam_step_ex": (c_int, [_P, _P, _P, _P, c_int, _P, c_float, c_float, c_float, c_float, c_float,
+                                _P, c_float, _P, c_int64, _P]),
+    "mr_ppo_train_epoch_ex": (c_int, [_P, _P, _P, _P, c_int, _P, _P, _P, _P, _P, _P, _P, c_int64, c_int64, _P,
+                                      c_int64, c_int64, c_float, c_float, c_float, c_int, c_float, c_float,
+                                      c_float, c_float, c_float, _P, _P, _P, _P, c_float, c_float, _P, c_int64, _P]),
+    "mr_ppo_train_summary_ex": (c_int, [_P, c_int, _P, _P, c_int64, _P, _P, _P, _P, _P]),
 }
 
 

@@ -41,22 +41,30 @@ struct GradArgs {
     float clip_range, ent_coef, vf_coef;
     int normalize_adv;
     float* partials;        // [gridDim.x][grad_stride]
+    const float* old_val;   // [T][N] the rollout's values (clip_range_vf; per-launch gather)
+    float clip_vf;          // SB3's clip_range_vf; <= 0: off
+    const int* ctrl;        // the update's control word (NULL: none); != 0 -> the update has stopped
 };
 
 // Tensor-core version (ppo_tc.cuh): even CTAs own the policy tower, odd CTAs the value tower.
-template <int KP>
+// VF: value clipping compiled in (A.clip_vf > 0).
+__device__ __forceinline__ bool update_stopped(const int* ctrl) {
+    return ctrl != nullptr && *reinterpret_cast<const volatile int*>(ctrl) != 0;
+}
+template <int KP, bool VF>
 __global__ void __launch_bounds__(tc::THREADS, 1) ppo_grad_tc_kernel(GradArgs A, int O) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
+    if (update_stopped(A.ctrl)) return;   // target_kl stopped the update at an earlier minibatch
     MR_TR(0);
     tc::Ctx C = tc::make_ctx(smem_raw, blockIdx.x & 1);
     tc::setup(C);
     tc::stage<KP>(C, A.params, O);
     const tc::Sched S{A.mb_size, A.mb_size, 1, (int)(blockIdx.x >> 1), (int)(gridDim.x >> 1)};
     tc::Pipe<KP> Q;
-    tc::pipe_start<KP, false>(Q, A, S, O, threadIdx.x & 127, threadIdx.x >> 7, C.tower == 0);
+    tc::pipe_start<KP, false, VF>(Q, A, S, O, threadIdx.x & 127, threadIdx.x >> 7, C.tower == 0);
     __syncthreads();
     const tc::MbConst MK = tc::mb_const(A.mb_stats, 0, A.normalize_adv);
-    tc::minibatch<KP>(C, A, S, MK, 0, Q, O, A.partials + (size_t)blockIdx.x * grad_stride(O));
+    tc::minibatch<KP, VF>(C, A, S, MK, 0, Q, O, A.partials + (size_t)blockIdx.x * grad_stride(O));
     tc::teardown(C);
 }
 
@@ -65,7 +73,9 @@ __global__ void __launch_bounds__(tc::THREADS, 1) ppo_grad_tc_kernel(GradArgs A,
 // combined in a fixed order (deterministic for a given n_parts).
 __global__ void __launch_bounds__(128)
 ppo_reduce_kernel(const float* __restrict__ partials, int n_parts, int O, float ent_coef,
-                  const double* __restrict__ mb_stats, float* __restrict__ grad, float rank_share) {
+                  const double* __restrict__ mb_stats, float* __restrict__ grad, float rank_share,
+                  const int* __restrict__ ctrl) {
+    if (update_stopped(ctrl)) return;   // grad keeps the stopping minibatch's gradient
     const int stride = grad_stride(O);
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= stride) return;
@@ -101,6 +111,9 @@ struct AdamArgs {
     float lr, beta1, beta2, eps, max_grad_norm;
     float* info;        // [8]: total_norm, clip_coef, step, entropy_loss, then the gradient's stats tail
     int n_params;       //      (policy_loss, value_loss, clip_fraction, approx_kl)
+    float target_kl;    // SB3's target_kl (<= 0: off); needs ctrl
+    int* ctrl;          // the update's control word (NULL: none)
+    int64_t mb;         // index of this minibatch in the update (what ctrl records on a stop)
 };
 
 constexpr int ADAM_THREADS = 256;
@@ -115,9 +128,13 @@ __device__ __forceinline__ float entropy_loss_of(float ls0, float ls1) {
 // The vector is only 42-48 KB, so the kernel is latency-bound: one parameter per thread,
 // every CTA recomputes the global norm from L2 in the same fixed order (bit-identical across
 // CTAs, no inter-CTA barrier), and the last CTA to finish bumps the step counter.
+// target_kl: SB3's early stop.  The approx_kl of the reduced gradient's tail (a global mean, after the
+// all-reduce when several ranks train) decides in every CTA alike; on a stop nothing is stepped, CTA 0 writes the
+// info row (step unchanged) and records mb + 1 in the control word, and every later launch of the update returns.
 __global__ void __launch_bounds__(ADAM_THREADS) adam_kernel(AdamArgs A) {
     __shared__ double s_part[ADAM_THREADS / 32];
     __shared__ double s_bc[2];
+    if (update_stopped(A.ctrl)) return;
     const int tid = threadIdx.x;
     const int64_t step = A.step[0] + 1;
     float ent_loss = 0.f;
@@ -153,6 +170,19 @@ __global__ void __launch_bounds__(ADAM_THREADS) adam_kernel(AdamArgs A) {
     for (int w = 0; w < ADAM_THREADS / 32; ++w) tot += s_part[w];
     const float total_norm = (float)sqrt(tot);
     const float coef = fminf(A.max_grad_norm / (total_norm + 1e-6f), 1.0f);
+    if (A.target_kl > 0.f && A.ctrl) {
+        const int sb = (A.n_params + 3) & ~3;
+        if ((double)__ldg(A.grad + sb + 3) > 1.5 * (double)A.target_kl) {
+            if (blockIdx.x == 0 && tid == 0) {
+                if (A.info) {
+                    A.info[0] = total_norm; A.info[1] = coef; A.info[2] = (float)(step - 1); A.info[3] = ent_loss;
+                    for (int q = 0; q < 4; ++q) A.info[4 + q] = A.grad[sb + q];
+                }
+                *A.ctrl = (int)(A.mb + 1);
+            }
+            return;   // every CTA: no parameter moves, the ticket is not taken
+        }
+    }
     tc::AdamK K;   // one arithmetic for the per-launch and the fused path (tc::adam1)
     K.coef = coef;
     K.beta1 = A.beta1; K.beta2 = A.beta2; K.omb1 = 1.f - A.beta1; K.omb2 = 1.f - A.beta2;
@@ -239,10 +269,13 @@ adv_stats_kernel(const float* __restrict__ adv, const int64_t* __restrict__ perm
 // approx_kl, [4:6] last minibatch's policy and value loss, [6] explained variance (nan if var(returns) = 0),
 // [7:9] log_std, [9] mean entropy_loss, [10] last minibatch's entropy_loss, [11] rows.
 // scratch: 4 doubles + a ticket (8 doubles in all), zero before the first call; the kernel re-arms it.
+// ctrl (target_kl; NULL = all rows): the update's control word.  When it records a stop after k minibatches, only
+// rows [0, k) are averaged, "last" means row k - 1, out[11] = k, and out[12] = row k - 1's approx_kl (out then
+// has 13 floats).
 __global__ void __launch_bounds__(256)
 train_summary_kernel(const float* __restrict__ info, int n_rows, const float* __restrict__ values,
                      const float* __restrict__ returns, int64_t n, const float* __restrict__ params,
-                     float* __restrict__ out, double* __restrict__ scratch) {
+                     float* __restrict__ out, double* __restrict__ scratch, const int* __restrict__ ctrl) {
     __shared__ double sh[8][8];
     __shared__ bool last;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -278,6 +311,10 @@ train_summary_kernel(const float* __restrict__ info, int n_rows, const float* __
     __syncthreads();
     if (!last) return;
     __threadfence();
+    if (ctrl) {
+        const int k = *reinterpret_cast<const volatile int*>(ctrl);
+        if (k > 0 && k < n_rows) n_rows = k;
+    }
     double r[6] = {0, 0, 0, 0, 0, 0};
     for (int row = tid; row < n_rows; row += blockDim.x) {
         const float* q = info + 8 * (size_t)row;
@@ -298,16 +335,18 @@ train_summary_kernel(const float* __restrict__ info, int n_rows, const float* __
         out[9] = (float)(r[4] * inv);
         out[10] = lastrow[3];
         out[11] = (float)n_rows;
+        if (ctrl) out[12] = lastrow[7];
         for (int k = 0; k < 5; ++k) scratch[k] = 0.0;   // re-arm (ticket included: it is slot 4)
     }
 }
 
-// One packed record per buffer row (tc::Rec): [obs | 0.. | 1 at KP-1 | a0 a1 old_logp adv | ret 0 0 0].
+// One packed record per buffer row (tc::Rec): [obs | 0.. | 1 at KP-1 | a0 a1 old_logp adv | ret old_value 0 0].
 // One thread per (row, 16-byte quad of the record): coalesced 16-byte stores, gathers hit L1 / L2.
+// values NULL: old_value = 0 (no value clipping).
 __global__ void __launch_bounds__(256)
 pack_samples_kernel(const float* __restrict__ obs, const float* __restrict__ act, const float* __restrict__ old_logp,
-                    const float* __restrict__ adv, const float* __restrict__ ret, int64_t n_rows, int O, int KP,
-                    float* __restrict__ rec) {
+                    const float* __restrict__ adv, const float* __restrict__ ret, const float* __restrict__ values,
+                    int64_t n_rows, int O, int KP, float* __restrict__ rec) {
     const int qpr = (KP + 8) >> 2;   // quads per record
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_rows * qpr) return;
@@ -323,7 +362,7 @@ pack_samples_kernel(const float* __restrict__ obs, const float* __restrict__ act
     } else if (4 * qd == KP) {
         v[0] = act[2 * r]; v[1] = act[2 * r + 1]; v[2] = old_logp[r]; v[3] = adv[r];
     } else {
-        v[0] = ret[r]; v[1] = v[2] = v[3] = 0.f;
+        v[0] = ret[r]; v[1] = values ? values[r] : 0.f; v[2] = v[3] = 0.f;
     }
     reinterpret_cast<float4*>(rec)[i] = make_float4(v[0], v[1], v[2], v[3]);
 }
@@ -435,6 +474,9 @@ struct EpochArgs {
     unsigned* barrier;         // [1], zero at launch
     unsigned seq0;             // exchange sequence number before this launch
     PeerXchg X;
+    float target_kl;           // SB3's target_kl (<= 0: off)           } read by the EXT instantiation only
+    int* ctrl;                 // the update's control word             }
+    int64_t mb0;               // index of this launch's first minibatch in the update
 };
 
 __device__ __forceinline__ unsigned ld_acquire_gpu(const unsigned* p) {
@@ -494,10 +536,20 @@ __device__ __forceinline__ void bulk_wait_all() {
     asm volatile("fence.proxy.async.global;" ::: "memory");   // async-proxy writes before the generic release below
 }
 
-template <int KP>
+// EXT: SB3's clip_range_vf and target_kl compiled in.  The default instantiation (EXT = false) is the kernel
+// without them, instruction for instruction.
+// Early stop (target_kl): after the barrier (and the exchange) of minibatch m every CTA of every rank holds the same
+// reduced statistics, so each computes approx_kl = kl_sum / count itself and takes the same decision without another
+// barrier.  On a stop, Adam is skipped (parameters, moments and step stay those after minibatch m - 1), CTA 0 still
+// writes info row m (step unchanged) and records mb0 + m + 1 in the control word, `grad` receives minibatch m's
+// gradient, and the CTAs leave the loop for the normal write-back.  A launch that finds the control word set returns
+// at entry in every CTA.
+template <int KP, bool EXT>
 __global__ void __launch_bounds__(tc::THREADS, 1) ppo_epoch_tc_kernel(EpochArgs E, int O) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
+    if (EXT && update_stopped(E.ctrl)) return;   // before any barrier: the update stopped in an earlier launch
     __shared__ double s_sq[tc::WARPS];
+    __shared__ float s_kl;
     __shared__ float4 s_x[8 * 32];   // peers' packets of the slice threads (tid < q4 <= 32)
     const ParamLayout L = make_layout(O);
     const tc::TowerLayout TL = tc::make_tl(O);
@@ -526,7 +578,7 @@ __global__ void __launch_bounds__(tc::THREADS, 1) ppo_epoch_tc_kernel(EpochArgs 
     GradArgs A = E.G;
     const tc::Sched S{E.n_samples, E.batch, n_mb, c >> 1, G >> 1};
     tc::Pipe<KP> Q;
-    tc::pipe_start<KP, true>(Q, A, S, O, tid & 127, tid >> 7, C.tower == 0);
+    tc::pipe_start<KP, true, EXT>(Q, A, S, O, tid & 127, tid >> 7, C.tower == 0);
 
     // the tower's parameters and Adam moments: flat global arrays -> shared memory, TL order
     for (int i = tid; i < TL.size; i += tc::THREADS) {
@@ -548,7 +600,7 @@ __global__ void __launch_bounds__(tc::THREADS, 1) ppo_epoch_tc_kernel(EpochArgs 
         if (m >= 2 && slice_t)
             __stcg(reinterpret_cast<float4*>(E.acc + (size_t)((m + 1) % 3) * acc_floats) + my_quad, make_float4(0.f, 0.f, 0.f, 0.f));
         MR_TR(2);
-        const tc::TileAcc T = tc::tiles<KP, true>(C, A, S, MK, m, Q, O);
+        const tc::TileAcc T = tc::tiles<KP, true, EXT>(C, A, S, MK, m, Q, O);
         if (T.any) {
             // the lane- and row-owned sums first (they do not need the last tile's dW1 GEMM, which finishes
             // meanwhile), then dW2 from TMEM and its bulk reduction, then dW1 and the sums
@@ -674,6 +726,13 @@ __global__ void __launch_bounds__(tc::THREADS, 1) ppo_epoch_tc_kernel(EpochArgs 
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) sq += __shfl_xor_sync(0xffffffffu, sq, o);
         if (lane == 0) s_sq[warp] = sq;
+        if (EXT) {
+            // the policy block's statistics quad: (loss, clipped count, kl sum, -)
+            const int q_st = (TL.st - TL.w1) >> 2;
+#pragma unroll
+            for (int k = 0; k < tc::BlockRegs<KP>::NR; ++k)
+                if (tid + k * tc::THREADS == q_st) s_kl = (C.tower == 0 ? gOwn.r[k].z : gOth.r[k].z) * inv_cnt;
+        }
         __syncthreads();
         double tot = 0.0;
 #pragma unroll
@@ -681,7 +740,9 @@ __global__ void __launch_bounds__(tc::THREADS, 1) ppo_epoch_tc_kernel(EpochArgs 
         const float total_norm = (float)sqrt(tot);
         K.coef = fminf(E.max_grad_norm / (total_norm + 1e-6f), 1.0f);
         MR_TR(31);
-        tc::adam_block(C, gOwn, K, TL, st_w, st_m, st_v);
+        const bool stop = EXT && E.target_kl > 0.f && (double)s_kl > 1.5 * (double)E.target_kl;
+        if (!stop) tc::adam_block(C, gOwn, K, TL, st_w, st_m, st_v);
+        else --step;   // SB3 breaks before optimizer.step(): the count stays that of minibatch m - 1
         MR_TR(7);
         // outputs of the API, off the other CTAs' critical path: statistics row (CTA 0), last gradient (CTAs 0, 1)
         if (c < 2) {
@@ -696,8 +757,12 @@ __global__ void __launch_bounds__(tc::THREADS, 1) ppo_epoch_tc_kernel(EpochArgs 
                         row[6] = gOwn.r[k].y * inv_cnt; row[7] = gOwn.r[k].z * inv_cnt;
                     }
             }
-            if (m == n_mb - 1) {
+            if (m == n_mb - 1 || stop) {
                 const int sb = stat_base(O);
+                if (EXT && c == 0) {   // the host does not clear `grad` for this instantiation: the pads here
+                    for (int p = L.total + tid; p < grad_stride(O); p += tc::THREADS)
+                        if (p < sb || p >= sb + 4) E.grad[p] = 0.f;
+                }
 #pragma unroll
                 for (int k = 0; k < 2; ++k) {
                     const int idx = tid + k * tc::THREADS;
@@ -725,7 +790,9 @@ __global__ void __launch_bounds__(tc::THREADS, 1) ppo_epoch_tc_kernel(EpochArgs 
                 }
             }
         }
+        if (stop && c == 0 && tid == 0) *E.ctrl = (int)(E.mb0 + m + 1);
         __syncthreads();   // the tower's new fp32 values (other threads' Adam) -> W1 panel, head vectors
+        if (stop) break;   // uniform: every CTA read the same s_kl
         if (m + 1 < n_mb) tc::panel_w1_from_tl<KP>(C, st_w, TL, O);
         MR_TR(37);
     }
@@ -818,21 +885,25 @@ int mr_ppo_prepare_epochs_device(uint64_t seed, const uint64_t* h_stream_ids, in
     return MR_OK;
 }
 
-int mr_ppo_grad_partials(const float* params, int obs_dim, const float* obs, const float* act,
+static int grad_partials(const float* params, int obs_dim, const float* obs, const float* act,
                          const float* old_logp, const float* adv, const float* ret, const int64_t* perm,
                          int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
                          float clip_range, float ent_coef, float vf_coef, int normalize_adv, float* partials,
-                         int* n_parts, void* stream) {
+                         int* n_parts, const float* old_values, float clip_range_vf, const int* ctrl, void* stream) {
     MR_REQUIRE(params && obs && act && old_logp && adv && ret && perm && rows && mb_stats && partials,
                "NULL argument");
     MR_REQUIRE(obs_dim > 0 && obs_dim <= MAX_OBS, "obs_dim out of range");
     MR_REQUIRE(mb_size > 0, "empty minibatch");
+    const bool vf = clip_range_vf > 0.f;
+    MR_REQUIRE(!vf || old_values, "clip_range_vf needs the rollout's values");
     GradArgs A{params, obs, act, old_logp, adv, ret, perm, nullptr, nullptr, mb_size, mb_stats, N, T,
-               clip_range, ent_coef, vf_coef, normalize_adv, partials};
+               clip_range, ent_coef, vf_coef, normalize_adv, partials, old_values, clip_range_vf, ctrl};
     static OncePerDevice once;
     if (once.first()) {
-        MR_CUDA(cudaFuncSetAttribute(ppo_grad_tc_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
-        MR_CUDA(cudaFuncSetAttribute(ppo_grad_tc_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+        MR_CUDA(cudaFuncSetAttribute(ppo_grad_tc_kernel<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+        MR_CUDA(cudaFuncSetAttribute(ppo_grad_tc_kernel<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+        MR_CUDA(cudaFuncSetAttribute(ppo_grad_tc_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+        MR_CUDA(cudaFuncSetAttribute(ppo_grad_tc_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
     }
     const int max_parts = mr_ppo_max_parts();
     cudaStream_t s = (cudaStream_t)stream;
@@ -845,10 +916,43 @@ int mr_ppo_grad_partials(const float* params, int obs_dim, const float* obs, con
     const int kp = obs_dim + 1 <= 16 ? 16 : 32;
     const int64_t tiles = (mb_size + tc::TILE - 1) / tc::TILE;
     const int grid = (int)std::min<int64_t>(2 * tiles, max_parts & ~1);
-    if (kp == 16) ppo_grad_tc_kernel<16><<<grid, tc::THREADS, tc::SMEM_BYTES, s>>>(A, obs_dim);
-    else ppo_grad_tc_kernel<32><<<grid, tc::THREADS, tc::SMEM_BYTES, s>>>(A, obs_dim);
+    if (kp == 16) {
+        if (vf) ppo_grad_tc_kernel<16, true><<<grid, tc::THREADS, tc::SMEM_BYTES, s>>>(A, obs_dim);
+        else ppo_grad_tc_kernel<16, false><<<grid, tc::THREADS, tc::SMEM_BYTES, s>>>(A, obs_dim);
+    } else {
+        if (vf) ppo_grad_tc_kernel<32, true><<<grid, tc::THREADS, tc::SMEM_BYTES, s>>>(A, obs_dim);
+        else ppo_grad_tc_kernel<32, false><<<grid, tc::THREADS, tc::SMEM_BYTES, s>>>(A, obs_dim);
+    }
     MR_CHECK_LAUNCH();
     if (n_parts) *n_parts = grid;
+    return MR_OK;
+}
+
+int mr_ppo_grad_partials(const float* params, int obs_dim, const float* obs, const float* act,
+                         const float* old_logp, const float* adv, const float* ret, const int64_t* perm,
+                         int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
+                         float clip_range, float ent_coef, float vf_coef, int normalize_adv, float* partials,
+                         int* n_parts, void* stream) {
+    return grad_partials(params, obs_dim, obs, act, old_logp, adv, ret, perm, rows, mb_size, mb_stats, N, T,
+                         clip_range, ent_coef, vf_coef, normalize_adv, partials, n_parts, nullptr, 0.f, nullptr, stream);
+}
+
+int mr_ppo_grad_ex(const float* params, int obs_dim, const float* obs, const float* act,
+                   const float* old_logp, const float* adv, const float* ret, const int64_t* perm,
+                   int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
+                   float clip_range, float ent_coef, float vf_coef, int normalize_adv, float rank_share,
+                   float* partials, float* grad, const float* old_values, float clip_range_vf, const int* ctrl,
+                   void* stream) {
+    MR_REQUIRE(grad, "NULL argument");
+    int grid = 0;
+    int rc = grad_partials(params, obs_dim, obs, act, old_logp, adv, ret, perm, rows, mb_size, mb_stats, N, T,
+                           clip_range, ent_coef, vf_coef, normalize_adv, partials, &grid, old_values, clip_range_vf,
+                           ctrl, stream);
+    if (rc != MR_OK) return rc;
+    const int stride = grad_stride(obs_dim);
+    ppo_reduce_kernel<<<ceil_div(stride, 128), 128, 0, (cudaStream_t)stream>>>(
+        partials, grid, obs_dim, ent_coef, mb_stats, grad, rank_share, ctrl);
+    MR_CHECK_LAUNCH();
     return MR_OK;
 }
 
@@ -857,14 +961,19 @@ int mr_ppo_grad(const float* params, int obs_dim, const float* obs, const float*
                 int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
                 float clip_range, float ent_coef, float vf_coef, int normalize_adv, float rank_share,
                 float* partials, float* grad, void* stream) {
-    MR_REQUIRE(grad, "NULL argument");
-    int grid = 0;
-    int rc = mr_ppo_grad_partials(params, obs_dim, obs, act, old_logp, adv, ret, perm, rows, mb_size, mb_stats,
-                                  N, T, clip_range, ent_coef, vf_coef, normalize_adv, partials, &grid, stream);
-    if (rc != MR_OK) return rc;
-    const int stride = grad_stride(obs_dim);
-    ppo_reduce_kernel<<<ceil_div(stride, 128), 128, 0, (cudaStream_t)stream>>>(
-        partials, grid, obs_dim, ent_coef, mb_stats, grad, rank_share);
+    return mr_ppo_grad_ex(params, obs_dim, obs, act, old_logp, adv, ret, perm, rows, mb_size, mb_stats, N, T,
+                          clip_range, ent_coef, vf_coef, normalize_adv, rank_share, partials, grad, nullptr, 0.f,
+                          nullptr, stream);
+}
+
+int mr_adam_step_ex(float* params, float* exp_avg, float* exp_avg_sq, const float* grad, int n_params,
+                    int64_t* step, float lr, float beta1, float beta2, float eps, float max_grad_norm,
+                    float* info, float target_kl, int* ctrl, int64_t mb_index, void* stream) {
+    MR_REQUIRE(params && exp_avg && exp_avg_sq && grad && step, "NULL argument");
+    MR_REQUIRE(!(target_kl > 0.f) || ctrl, "target_kl needs a control word");
+    AdamArgs A{params, exp_avg, exp_avg_sq, grad, step, lr, beta1, beta2, eps, max_grad_norm, info, n_params,
+               target_kl, ctrl, mb_index};
+    adam_kernel<<<ceil_div(n_params, ADAM_THREADS), ADAM_THREADS, 0, (cudaStream_t)stream>>>(A);
     MR_CHECK_LAUNCH();
     return MR_OK;
 }
@@ -872,20 +981,48 @@ int mr_ppo_grad(const float* params, int obs_dim, const float* obs, const float*
 int mr_adam_step(float* params, float* exp_avg, float* exp_avg_sq, const float* grad, int n_params,
                  int64_t* step, float lr, float beta1, float beta2, float eps, float max_grad_norm,
                  float* info, void* stream) {
-    MR_REQUIRE(params && exp_avg && exp_avg_sq && grad && step, "NULL argument");
-    AdamArgs A{params, exp_avg, exp_avg_sq, grad, step, lr, beta1, beta2, eps, max_grad_norm, info, n_params};
-    adam_kernel<<<ceil_div(n_params, ADAM_THREADS), ADAM_THREADS, 0, (cudaStream_t)stream>>>(A);
+    return mr_adam_step_ex(params, exp_avg, exp_avg_sq, grad, n_params, step, lr, beta1, beta2, eps, max_grad_norm,
+                           info, 0.f, nullptr, 0, stream);
+}
+
+int mr_ppo_train_summary_ex(const float* info, int n_rows, const float* values, const float* returns, int64_t n,
+                            const float* params, float* out, double* scratch, const int* ctrl, void* stream) {
+    MR_REQUIRE(info && values && returns && params && out && scratch, "NULL argument");
+    MR_REQUIRE(n_rows > 0 && n > 0, "empty summary");
+    const int grid = (int)std::min<int64_t>(sm_count(), (n + 255) / 256);
+    train_summary_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(info, n_rows, values, returns, n, params, out, scratch,
+                                                                 ctrl);
     MR_CHECK_LAUNCH();
     return MR_OK;
 }
 
 int mr_ppo_train_summary(const float* info, int n_rows, const float* values, const float* returns, int64_t n,
                          const float* params, float* out, double* scratch, void* stream) {
-    MR_REQUIRE(info && values && returns && params && out && scratch, "NULL argument");
-    MR_REQUIRE(n_rows > 0 && n > 0, "empty summary");
-    const int grid = (int)std::min<int64_t>(sm_count(), (n + 255) / 256);
-    train_summary_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(info, n_rows, values, returns, n, params, out, scratch);
-    MR_CHECK_LAUNCH();
+    return mr_ppo_train_summary_ex(info, n_rows, values, returns, n, params, out, scratch, nullptr, stream);
+}
+
+int mr_ppo_train_epoch_ex(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
+                          const float* obs, const float* act, const float* old_logp, const float* adv,
+                          const float* ret, const int64_t* perm, int32_t* rows, int64_t n_samples,
+                          int64_t batch_size, const double* stats, int64_t N, int64_t T, float clip_range,
+                          float ent_coef, float vf_coef, int normalize_adv, float lr, float beta1, float beta2,
+                          float eps, float max_grad_norm, float* partials, float* grad, float* info,
+                          const float* old_values, float clip_range_vf, float target_kl, int* ctrl, int64_t mb0,
+                          void* stream) {
+    MR_REQUIRE(batch_size > 0 && n_samples > 0, "empty batch");
+    const int n_params = make_layout(obs_dim).total;
+    const int64_t n_mb = (n_samples + batch_size - 1) / batch_size;
+    for (int64_t mb = 0; mb < n_mb; ++mb) {
+        const int64_t s0 = mb * batch_size;
+        const int64_t sz = std::min(batch_size, n_samples - s0);
+        int rc = mr_ppo_grad_ex(params, obs_dim, obs, act, old_logp, adv, ret, perm + s0, rows, sz, stats + 3 * mb,
+                                N, T, clip_range, ent_coef, vf_coef, normalize_adv, 1.0f, partials, grad, old_values,
+                                clip_range_vf, ctrl, stream);
+        if (rc != MR_OK) return rc;
+        rc = mr_adam_step_ex(params, exp_avg, exp_avg_sq, grad, n_params, step, lr, beta1, beta2, eps,
+                             max_grad_norm, info ? info + 8 * mb : nullptr, target_kl, ctrl, mb0 + mb, stream);
+        if (rc != MR_OK) return rc;
+    }
     return MR_OK;
 }
 
@@ -895,20 +1032,10 @@ int mr_ppo_train_epoch(float* params, float* exp_avg, float* exp_avg_sq, int64_t
                        int64_t batch_size, const double* stats, int64_t N, int64_t T, float clip_range,
                        float ent_coef, float vf_coef, int normalize_adv, float lr, float beta1, float beta2,
                        float eps, float max_grad_norm, float* partials, float* grad, float* info, void* stream) {
-    MR_REQUIRE(batch_size > 0 && n_samples > 0, "empty batch");
-    const int n_params = make_layout(obs_dim).total;
-    const int64_t n_mb = (n_samples + batch_size - 1) / batch_size;
-    for (int64_t mb = 0; mb < n_mb; ++mb) {
-        const int64_t s0 = mb * batch_size;
-        const int64_t sz = std::min(batch_size, n_samples - s0);
-        int rc = mr_ppo_grad(params, obs_dim, obs, act, old_logp, adv, ret, perm + s0, rows, sz, stats + 3 * mb,
-                             N, T, clip_range, ent_coef, vf_coef, normalize_adv, 1.0f, partials, grad, stream);
-        if (rc != MR_OK) return rc;
-        rc = mr_adam_step(params, exp_avg, exp_avg_sq, grad, n_params, step, lr, beta1, beta2, eps,
-                          max_grad_norm, info ? info + 8 * mb : nullptr, stream);
-        if (rc != MR_OK) return rc;
-    }
-    return MR_OK;
+    return mr_ppo_train_epoch_ex(params, exp_avg, exp_avg_sq, step, obs_dim, obs, act, old_logp, adv, ret, perm, rows,
+                                 n_samples, batch_size, stats, N, T, clip_range, ent_coef, vf_coef, normalize_adv, lr,
+                                 beta1, beta2, eps, max_grad_norm, partials, grad, info, nullptr, 0.f, 0.f, nullptr, 0,
+                                 stream);
 }
 
 #ifdef MR_TRACE
@@ -996,27 +1123,36 @@ void mr_xchg_destroy(mr_xchg* x) {
 
 int mr_ppo_record_floats(int obs_dim) { return (obs_dim + 1 <= 16 ? 16 : 32) + 8; }
 
-int mr_ppo_pack_samples(int obs_dim, const float* obs, const float* act, const float* old_logp, const float* adv,
-                        const float* ret, int64_t n_rows, float* rec, void* stream) {
+int mr_ppo_pack_samples_vf(int obs_dim, const float* obs, const float* act, const float* old_logp, const float* adv,
+                           const float* ret, const float* values, int64_t n_rows, float* rec, void* stream) {
     MR_REQUIRE(obs && act && old_logp && adv && ret && rec, "NULL argument");
     MR_REQUIRE(obs_dim > 0 && obs_dim < MAX_OBS, "obs_dim out of range (1..31: the record's row of X is obs and the ones column)");
     MR_REQUIRE(n_rows > 0, "empty buffer");
     const int kp = obs_dim + 1 <= 16 ? 16 : 32;
     const int64_t quads = n_rows * ((kp + 8) >> 2);
-    pack_samples_kernel<<<ceil_div(quads, 256), 256, 0, (cudaStream_t)stream>>>(obs, act, old_logp, adv, ret, n_rows,
-                                                                                obs_dim, kp, rec);
+    pack_samples_kernel<<<ceil_div(quads, 256), 256, 0, (cudaStream_t)stream>>>(obs, act, old_logp, adv, ret, values,
+                                                                                n_rows, obs_dim, kp, rec);
     MR_CHECK_LAUNCH();
     return MR_OK;
 }
 
-int mr_ppo_epoch_fused(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
-                       const float* rec, const int64_t* perm, int32_t* rows, int64_t n_samples,
-                       int64_t batch_size, const double* stats, int64_t N, int64_t T,
-                       float clip_range, float ent_coef, float vf_coef, int normalize_adv, float lr,
-                       float beta1, float beta2, float eps, float max_grad_norm, float* partials,
-                       float* grad, float* info, mr_xchg* xchg, void* stream) {
+int mr_ppo_pack_samples(int obs_dim, const float* obs, const float* act, const float* old_logp, const float* adv,
+                        const float* ret, int64_t n_rows, float* rec, void* stream) {
+    return mr_ppo_pack_samples_vf(obs_dim, obs, act, old_logp, adv, ret, nullptr, n_rows, rec, stream);
+}
+
+int mr_ppo_epoch_fused_ex(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
+                          const float* rec, const int64_t* perm, int32_t* rows, int64_t n_samples,
+                          int64_t batch_size, const double* stats, int64_t N, int64_t T,
+                          float clip_range, float ent_coef, float vf_coef, int normalize_adv, float lr,
+                          float beta1, float beta2, float eps, float max_grad_norm, float* partials,
+                          float* grad, float* info, mr_xchg* xchg, float clip_range_vf, float target_kl, int* ctrl,
+                          int64_t mb0, void* stream) {
     MR_REQUIRE(params && exp_avg && exp_avg_sq && step && rec && rows && stats && partials && grad,
                "NULL argument");   // perm may be NULL: rows then already hold the epoch's samples (mr_ppo_prepare_epochs)
+    MR_REQUIRE(!(target_kl > 0.f) || ctrl, "target_kl needs a control word");
+    // the extended instantiation (value clipping, early stop) only where asked for: the default one is unchanged
+    const bool ext = clip_range_vf > 0.f || target_kl > 0.f || ctrl != nullptr;
     MR_REQUIRE(obs_dim > 0 && obs_dim < MAX_OBS, "obs_dim out of range (1..31: the row of X is obs and the ones column)");
     MR_REQUIRE(batch_size > 0 && n_samples > 0, "empty batch");
     MR_REQUIRE(n_samples < (int64_t(1) << 31) && N * T < (int64_t(1) << 31), "samples are indexed with 32 bits");
@@ -1041,7 +1177,9 @@ int mr_ppo_epoch_fused(float* params, float* exp_avg, float* exp_avg_sq, int64_t
     E.gsum = partials + 3 * (size_t)acc_floats;
     E.barrier = reinterpret_cast<unsigned*>(partials + 4 * (size_t)acc_floats);
     MR_CUDA(cudaMemsetAsync(partials, 0, (4 * (size_t)acc_floats + 16) * sizeof(float), s));
-    MR_CUDA(cudaMemsetAsync(grad, 0, (size_t)stride * sizeof(float), s));
+    if (!ext) MR_CUDA(cudaMemsetAsync(grad, 0, (size_t)stride * sizeof(float), s));   // (ext: the kernel clears the pads)
+    E.G.clip_vf = clip_range_vf;   // the records carry old_value (mr_ppo_pack_samples_vf) when this is > 0
+    E.target_kl = target_kl; E.ctrl = ctrl; E.mb0 = mb0;
     E.X.world = 1; E.X.rank = 0; E.X.inbox = nullptr; E.X.err = nullptr;
     E.seq0 = 0;
     const int64_t n_mb = (n_samples + batch_size - 1) / batch_size;
@@ -1060,8 +1198,10 @@ int mr_ppo_epoch_fused(float* params, float* exp_avg, float* exp_avg_sq, int64_t
     static OncePerDevice once;
     if (once.first()) {
         const int smem_max = (int)((size_t)tc::SMEM_BYTES + 3 * (size_t)tc::make_tl(MAX_OBS - 1).size * sizeof(float));
-        MR_CUDA(cudaFuncSetAttribute(ppo_epoch_tc_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
-        MR_CUDA(cudaFuncSetAttribute(ppo_epoch_tc_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+        MR_CUDA(cudaFuncSetAttribute(ppo_epoch_tc_kernel<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+        MR_CUDA(cudaFuncSetAttribute(ppo_epoch_tc_kernel<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+        MR_CUDA(cudaFuncSetAttribute(ppo_epoch_tc_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+        MR_CUDA(cudaFuncSetAttribute(ppo_epoch_tc_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
     }
     if (perm) {
         perm_to_rows_kernel<<<ceil_div(n_samples, 256), 256, 0, s>>>(perm, n_samples, N, T, rows);
@@ -1069,10 +1209,22 @@ int mr_ppo_epoch_fused(float* params, float* exp_avg, float* exp_avg_sq, int64_t
     }
     int O = obs_dim;
     void* args[] = {&E, &O};
-    const void* fn = kp == 16 ? (const void*)ppo_epoch_tc_kernel<16> : (const void*)ppo_epoch_tc_kernel<32>;
+    const void* fn = kp == 16 ? (ext ? (const void*)ppo_epoch_tc_kernel<16, true> : (const void*)ppo_epoch_tc_kernel<16, false>)
+                              : (ext ? (const void*)ppo_epoch_tc_kernel<32, true> : (const void*)ppo_epoch_tc_kernel<32, false>);
     MR_CUDA(cudaLaunchCooperativeKernel(fn, dim3(n_cta), dim3(tc::THREADS), args, smem, s));
     mr::count_launch();
     return MR_OK;
+}
+
+int mr_ppo_epoch_fused(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
+                       const float* rec, const int64_t* perm, int32_t* rows, int64_t n_samples,
+                       int64_t batch_size, const double* stats, int64_t N, int64_t T,
+                       float clip_range, float ent_coef, float vf_coef, int normalize_adv, float lr,
+                       float beta1, float beta2, float eps, float max_grad_norm, float* partials,
+                       float* grad, float* info, mr_xchg* xchg, void* stream) {
+    return mr_ppo_epoch_fused_ex(params, exp_avg, exp_avg_sq, step, obs_dim, rec, perm, rows, n_samples, batch_size,
+                                 stats, N, T, clip_range, ent_coef, vf_coef, normalize_adv, lr, beta1, beta2, eps,
+                                 max_grad_norm, partials, grad, info, xchg, 0.f, 0.f, nullptr, 0, stream);
 }
 
 }  // extern "C"

@@ -91,8 +91,13 @@ class PPO:
                  host_permutation=None, update_mode="fused", permutation=None):
         if policy not in ("MlpPolicy", MlpPolicy):
             raise ValueError("only MlpPolicy is built (the only policy mobrob uses)")
-        if use_sde or clip_range_vf is not None or target_kl is not None:
-            raise NotImplementedError("use_sde / clip_range_vf / target_kl are not used by mobrob's configs")
+        if use_sde:
+            raise NotImplementedError("use_sde (gSDE) is not built: it is a different policy and rollout noise model")
+        if clip_range_vf is not None and not callable(clip_range_vf) and not float(clip_range_vf) > 0:
+            raise ValueError(f"clip_range_vf must be positive (got {clip_range_vf}); None turns value clipping off")
+        if target_kl is not None and not float(target_kl) > 0:
+            # SB3 would stop every update at its first minibatch; the kernels take target_kl <= 0 as "off"
+            raise ValueError(f"target_kl must be positive (got {target_kl}); None turns early stopping off")
         if policy_kwargs not in (None, {}):
             arch = (policy_kwargs or {}).get("net_arch")
             if arch not in (None, dict(pi=[64, 64], vf=[64, 64])):
@@ -100,6 +105,11 @@ class PPO:
         # SB3 schedules: callables of the remaining progress (1 -> 0), evaluated before every update
         self._lr_schedule = learning_rate if callable(learning_rate) else None
         self._clip_schedule = clip_range if callable(clip_range) else None
+        self._clip_vf_schedule = clip_range_vf if callable(clip_range_vf) else None
+        if callable(clip_range_vf):
+            clip_range_vf = float(clip_range_vf(1.0))
+        self.clip_range_vf = None if clip_range_vf is None else float(clip_range_vf)
+        self.target_kl = None if target_kl is None else float(target_kl)
         if callable(learning_rate):
             learning_rate = float(learning_rate(1.0))
         if callable(clip_range):
@@ -126,6 +136,9 @@ class PPO:
         self._train_meta = None
         self._snap_meta = None
         self._snap = None
+        # target_kl: updates whose epoch count is read back from the device lazily (_settle_updates)
+        self._pending_updates = deque()
+        self._n_updates_at = {}
         self._current_progress_remaining = 1.0
         self._stats_window_size = stats_window_size
         self.num_timesteps = 0
@@ -169,7 +182,8 @@ class PPO:
         O = env.obs_dim
         self.updater = PpoUpdater(O, self.device, lr=self.learning_rate, max_grad_norm=self.max_grad_norm,
                                   clip_range=self.clip_range, ent_coef=self.ent_coef, vf_coef=self.vf_coef,
-                                  normalize_advantage=self.normalize_advantage)
+                                  normalize_advantage=self.normalize_advantage, clip_range_vf=self.clip_range_vf,
+                                  target_kl=self.target_kl)
         self.policy = MlpPolicy(O, 2, device=self.device, flat=self.updater.params, init=True)
         d = _dist()
         if d is not None:  # every rank must start from rank 0's parameters
@@ -347,11 +361,14 @@ class PPO:
         rows = self.n_epochs * n_mb
         if getattr(self, "_log", None) is None or self._log.shape[0] != rows:
             # per-minibatch info rows (every row is written by the kernels), the 12 logger inputs of the
-            # update and the summary kernel's scratch: allocated once, no per-iteration torch launches
+            # update (+ the stopping minibatch's approx_kl with target_kl) and the summary kernel's scratch:
+            # allocated once, no per-iteration torch launches
             self._log = torch.zeros((rows, 8), dtype=torch.float32, device=self.device)
-            self._train_stats_buf = torch.zeros(12, dtype=torch.float32, device=self.device)
+            self._train_stats_buf = torch.zeros(13, dtype=torch.float32, device=self.device)
             self._sum_scratch = torch.zeros(8, dtype=torch.float64, device=self.device)
         log = self._log
+        self._settle_updates(block=False)
+        up.begin_update()   # target_kl: clear the control word (nothing otherwise)
         k = 0
         if self.update_mode == "fused":
             up.pack(b)   # packed sample records, once per rollout: what the epoch kernel gathers from
@@ -374,7 +391,8 @@ class PPO:
                 k = rows
             else:
                 for epoch in range(self.n_epochs):
-                    up.train_epoch_fused(None, None, stats_all[epoch], B, N, T, log[k:k + n_mb], self._xchg, rows=rows_all[epoch])
+                    up.train_epoch_fused(None, None, stats_all[epoch], B, N, T, log[k:k + n_mb], self._xchg, rows=rows_all[epoch],
+                                         mb0=k)
                     k += n_mb
             epochs = ()
         else:
@@ -389,10 +407,10 @@ class PPO:
             if d is not None:
                 stats, share = sharding.allreduce_adv_stats(stats)
             if self.update_mode == "fused":      # one cooperative launch per epoch (+ NVLink all-reduce)
-                up.train_epoch_fused(None, perm, stats, B, N, T, log[k:k + n_mb], self._xchg)
+                up.train_epoch_fused(None, perm, stats, B, N, T, log[k:k + n_mb], self._xchg, mb0=k)
                 k += n_mb
             elif d is None:                      # 3 launches per minibatch, looped in C
-                up.train_epoch(b, perm, stats, B, N, T, log[k:k + n_mb])
+                up.train_epoch(b, perm, stats, B, N, T, log[k:k + n_mb], mb0=k)
                 k += n_mb
             else:                                # NCCL all-reduce per minibatch (baseline path)
                 share_h = share.cpu().tolist()
@@ -400,20 +418,60 @@ class PPO:
                     sl = perm[mb * B:(mb + 1) * B]
                     up.compute_grad(b, sl, stats[mb], N, T, share_h[mb])
                     d.all_reduce(up.grad)
-                    up.adam_step(log[k])
+                    up.adam_step(log[k], mb_index=k)
                     k += 1
         if perms is None and self.permutation == "pool":
             self._feeder.release(self._train_count)
+        uid = self._train_count
         self._train_count += 1
-        self._n_updates += self.n_epochs
         self._train_log = (log[:, 4:], log[:, :4])
         # logger inputs of this update (mr_ppo_train_summary), read one iteration later -- SB3 records
         # train/* inside train() and dumps them with the NEXT iteration's rollout statistics
-        _lib.check(self.lib.mr_ppo_train_summary(log.data_ptr(), rows, b["values"].data_ptr(), b["returns"].data_ptr(),
-                                                 n, up.params.data_ptr(), self._train_stats_buf.data_ptr(),
-                                                 self._sum_scratch.data_ptr(), self._stream()))
-        self._train_stats = self._train_stats_buf
-        self._train_meta = dict(n_updates=self._n_updates, clip_range=self.clip_range, learning_rate=up.lr)
+        if self.target_kl is None:
+            self._n_updates += self.n_epochs
+            _lib.check(self.lib.mr_ppo_train_summary(log.data_ptr(), rows, b["values"].data_ptr(), b["returns"].data_ptr(),
+                                                     n, up.params.data_ptr(), self._train_stats_buf.data_ptr(),
+                                                     self._sum_scratch.data_ptr(), self._stream()))
+        else:
+            # statistics over the minibatches evaluated before the stop; how many epochs were entered is read
+            # back without blocking (the control word and the stopping approx_kl, into pinned memory)
+            _lib.check(self.lib.mr_ppo_train_summary_ex(log.data_ptr(), rows, b["values"].data_ptr(),
+                                                        b["returns"].data_ptr(), n, up.params.data_ptr(),
+                                                        self._train_stats_buf.data_ptr(), self._sum_scratch.data_ptr(),
+                                                        up.ctrl.data_ptr(), self._stream()))
+            ctrl_h = torch.zeros(1, dtype=torch.int32).pin_memory()
+            kl_h = torch.zeros(1, dtype=torch.float32).pin_memory()
+            ctrl_h.copy_(up.ctrl, non_blocking=True)
+            kl_h.copy_(self._train_stats_buf[12:13], non_blocking=True)
+            ev = torch.cuda.Event()
+            ev.record(torch.cuda.current_stream(self.device))
+            self._pending_updates.append((uid, ev, ctrl_h, kl_h, n_mb))
+        self._train_stats = self._train_stats_buf[:12]
+        self._train_meta = dict(update=uid, n_updates=self._n_updates if self.target_kl is None else None,
+                                clip_range=self.clip_range, clip_range_vf=self.clip_range_vf, learning_rate=up.lr)
+
+    def _settle_updates(self, upto=None, block=True):
+        """target_kl: add the epochs each finished update entered to _n_updates (SB3 counts every epoch it
+        enters, the one it stops in included) and print SB3's early-stopping message.  Updates are settled in
+        order: all of them, those up to update id `upto`, or (block=False) those already complete."""
+        while self._pending_updates:
+            uid, ev, ctrl_h, kl_h, n_mb = self._pending_updates[0]
+            if upto is not None and uid > upto:
+                break
+            if not block and not ev.query():
+                break
+            ev.synchronize()
+            self._pending_updates.popleft()
+            k = int(ctrl_h[0])
+            if k > 0:
+                epochs = (k + n_mb - 1) // n_mb
+                if self.verbose >= 1 and self._is_rank0():
+                    print(f"Early stopping at step {epochs - 1} due to reaching max kl: {float(kl_h[0]):.2f}")
+            else:
+                epochs = self.n_epochs
+            self._n_updates += epochs
+            self._n_updates_at[uid] = self._n_updates
+            self._n_updates_at.pop(uid - 8, None)
 
     def _update_schedules(self):
         """SB3's _update_learning_rate / clip_range(progress): constant values or callables of the
@@ -426,8 +484,12 @@ class PPO:
             self.learning_rate = float(self._lr_schedule(progress))
         if self._clip_schedule is not None:
             self.clip_range = float(self._clip_schedule(progress))
+        if self._clip_vf_schedule is not None:
+            self.clip_range_vf = float(self._clip_vf_schedule(progress))
         self.updater.lr = self.learning_rate
         self.updater.clip_range = self.clip_range
+        self.updater.clip_range_vf = self.clip_range_vf
+        self.updater.target_kl = self.target_kl
 
     def _log_train(self):
         """train/* keys of SB3's PPO.train, from the statistics snapshot of the previous update."""
@@ -442,8 +504,14 @@ class PPO:
         lg.record("train/loss", float(t[4] + self.ent_coef * t[10] + self.vf_coef * t[5]))
         lg.record("train/explained_variance", float(t[6]))
         lg.record("train/std", float(np.exp(t[7:9].astype(np.float32)).mean()))
-        lg.record("train/n_updates", meta["n_updates"])
+        n_updates = meta["n_updates"]
+        if n_updates is None:   # target_kl: the update's epoch count is in the snapshot's past, complete by now
+            self._settle_updates(upto=meta["update"])
+            n_updates = self._n_updates_at.get(meta["update"], self._n_updates)
+        lg.record("train/n_updates", n_updates)
         lg.record("train/clip_range", meta["clip_range"])
+        if meta.get("clip_range_vf") is not None:
+            lg.record("train/clip_range_vf", meta["clip_range_vf"])
         lg.record("train/learning_rate", meta["learning_rate"])
 
     # -- learn ----------------------------------------------------------------------------------------
@@ -542,7 +610,7 @@ class PPO:
                     "low": str(sp.low), "high": str(sp.high), "low_repr": str(sp.low.min()),
                     "high_repr": str(sp.high.max()), "_np_random": None}
 
-        lr, cr = self.learning_rate, self.clip_range
+        lr, cr, cvf = self.learning_rate, self.clip_range, self.clip_range_vf
         last_obs = None if self._last_obs is None else self._last_obs.cpu().numpy()
         starts = None if self._last_episode_starts is None else self._last_episode_starts.cpu().numpy().astype(bool)
         return {
@@ -568,7 +636,9 @@ class PPO:
             "max_grad_norm": self.max_grad_norm, "batch_size": self.batch_size, "n_epochs": self.n_epochs,
             "clip_range": {":type:": "<class 'function'>", ":serialized:": ser(self._clip_schedule or _Constant(cr)),
                            "value": cr},
-            "clip_range_vf": None, "normalize_advantage": self.normalize_advantage, "target_kl": None,
+            "clip_range_vf": None if cvf is None else {
+                ":type:": "<class 'function'>", ":serialized:": ser(self._clip_vf_schedule or _Constant(cvf)), "value": cvf},
+            "normalize_advantage": self.normalize_advantage, "target_kl": self.target_kl,
             "observation_space": space(self.observation_space), "action_space": space(self.action_space),
             "n_envs": self.n_envs,
             "lr_schedule": {":type:": "<class 'function'>", ":serialized:": ser(self._lr_schedule or _Constant(lr)),
@@ -580,6 +650,7 @@ class PPO:
         if not path.endswith(".zip"):
             path += ".zip"
         os.makedirs(os.path.dirname(os.path.abspath(path)), exist_ok=True)
+        self._settle_updates()   # target_kl: _n_updates of an update still in flight (waits for it)
         sd = {k: v.detach().cpu().clone() for k, v in self.policy.state_dict().items()}
         up = self.updater
         opt_state, off = {}, 0
@@ -632,6 +703,10 @@ class PPO:
         ctor = {k: data[k] for k in plain if k in data}
         ctor["learning_rate"] = _stored_schedule(data.get("learning_rate", 3e-4), "learning_rate")
         ctor["clip_range"] = _stored_schedule(data.get("clip_range", 0.2), "clip_range")
+        if data.get("clip_range_vf") is not None:
+            ctor["clip_range_vf"] = _stored_schedule(data["clip_range_vf"], "clip_range_vf")
+        if data.get("target_kl") is not None:
+            ctor["target_kl"] = float(data["target_kl"])
         ctor.update(kwargs)
         model = cls("MlpPolicy", env, _init_setup_model=False, **ctor)
         for k in ("num_timesteps", "_total_timesteps", "_num_timesteps_at_start", "_n_updates", "_episode_num"):
@@ -652,7 +727,8 @@ class PPO:
             up = PpoUpdater(obs_dim, dev, lr=ctor["learning_rate"], max_grad_norm=ctor.get("max_grad_norm", 0.5),
                             clip_range=ctor["clip_range"], ent_coef=ctor.get("ent_coef", 0.0),
                             vf_coef=ctor.get("vf_coef", 0.5),
-                            normalize_advantage=ctor.get("normalize_advantage", True))
+                            normalize_advantage=ctor.get("normalize_advantage", True),
+                            clip_range_vf=model.clip_range_vf, target_kl=model.target_kl)
             model.updater = up
             model.policy = MlpPolicy(obs_dim, 2, device=dev, flat=up.params, init=False)
         model.policy.load_state_dict(sd)

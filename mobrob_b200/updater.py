@@ -3,6 +3,10 @@
 Owns the flat parameter vector, the Adam moments and the gradient scratch as torch CUDA
 tensors (so ``state_dict`` views, NCCL all-reduce and checkpointing need no extra copies).
 Mirrors what [SB3] PPO.train does per minibatch; see include/mobrob_b200.h.
+
+clip_range_vf / target_kl (None = off, the default) select the *_ex entry points; without them every call is the
+one it always was.  With target_kl the update's control word (``self.ctrl``, one int32 on the device) records an
+early stop; ``begin_update()`` clears it and must be called before the first launch of every update.
 """
 from __future__ import annotations
 
@@ -14,7 +18,8 @@ from . import _lib
 class PpoUpdater:
     def __init__(self, obs_dim: int, device: torch.device, lr: float = 3e-4, betas=(0.9, 0.999),
                  eps: float = 1e-5, max_grad_norm: float = 0.5, clip_range: float = 0.2,
-                 ent_coef: float = 0.0, vf_coef: float = 0.5, normalize_advantage: bool = True):
+                 ent_coef: float = 0.0, vf_coef: float = 0.5, normalize_advantage: bool = True,
+                 clip_range_vf: float | None = None, target_kl: float | None = None):
         self.lib = _lib.load()
         if not 0 < obs_dim < 32:
             raise ValueError(f"the PPO kernels take observations of 1..31 floats (got {obs_dim}): with the optional "
@@ -25,6 +30,7 @@ class PpoUpdater:
         self.max_grad_norm = max_grad_norm
         self.clip_range, self.ent_coef, self.vf_coef = clip_range, ent_coef, vf_coef
         self.normalize_advantage = normalize_advantage
+        self.clip_range_vf, self.target_kl = clip_range_vf, target_kl
         self.n_params = int(self.lib.mr_ppo_num_params(obs_dim))
         self.stride = int(self.lib.mr_ppo_grad_stride(obs_dim))
         with torch.cuda.device(device):
@@ -39,6 +45,23 @@ class PpoUpdater:
         self.partials = torch.zeros((self.max_parts + 1, self.stride), **f32)
         self.grad = torch.zeros(self.stride, **f32)
         self._rows = torch.empty(0, dtype=torch.int32, device=device)
+        # target_kl: k > 0 once the update stopped after its k-th minibatch (caller-owned, like the barrier word)
+        self.ctrl = torch.zeros(1, dtype=torch.int32, device=device)
+
+    @property
+    def extended(self) -> bool:
+        """True when clip_range_vf or target_kl is on: the update goes through the *_ex entry points."""
+        return self.clip_range_vf is not None or self.target_kl is not None
+
+    def _ext_args(self):
+        """(clip_range_vf, target_kl, control word) as the *_ex entry points take them (0 / NULL = off)."""
+        return (float(self.clip_range_vf or 0.0), float(self.target_kl or 0.0),
+                self.ctrl.data_ptr() if self.target_kl is not None else None)
+
+    def begin_update(self):
+        """Clear the control word (target_kl): once per update, before its first launch."""
+        if self.target_kl is not None:
+            self.ctrl.zero_()
 
     def rows(self, n: int) -> torch.Tensor:
         """int32 scratch for the samples as buffer rows (owned here, not by the library)."""
@@ -59,7 +82,17 @@ class PpoUpdater:
 
     def compute_grad(self, buf: dict, perm_slice: torch.Tensor, mb_stats: torch.Tensor, N: int, T: int,
                      rank_share: float = 1.0):
-        """buf: time-major rollout tensors obs/actions/log_probs/advantages/returns."""
+        """buf: time-major rollout tensors obs/actions/log_probs/advantages/returns (+ values with clip_range_vf)."""
+        if self.extended:
+            cvf, _, ctrl = self._ext_args()
+            _lib.check(self.lib.mr_ppo_grad_ex(
+                self.params.data_ptr(), self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(),
+                buf["log_probs"].data_ptr(), buf["advantages"].data_ptr(), buf["returns"].data_ptr(),
+                perm_slice.data_ptr(), self.rows(perm_slice.numel()).data_ptr(), perm_slice.numel(),
+                mb_stats.data_ptr(), N, T, self.clip_range, self.ent_coef, self.vf_coef,
+                int(self.normalize_advantage), rank_share, self.partials.data_ptr(), self.grad.data_ptr(),
+                buf["values"].data_ptr() if cvf > 0 else None, cvf, ctrl, self._stream()))
+            return self.grad
         _lib.check(self.lib.mr_ppo_grad(
             self.params.data_ptr(), self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(),
             buf["log_probs"].data_ptr(), buf["advantages"].data_ptr(), buf["returns"].data_ptr(),
@@ -78,7 +111,16 @@ class PpoUpdater:
             mb_stats.data_ptr(), N, T, self.clip_range, self.ent_coef, self.vf_coef,
             int(self.normalize_advantage), self.partials.data_ptr(), None, self._stream()))
 
-    def adam_step(self, info: torch.Tensor | None = None):
+    def adam_step(self, info: torch.Tensor | None = None, mb_index: int = 0):
+        """mb_index: this minibatch's index in the update (what an early stop records)."""
+        if self.extended:
+            _, tkl, ctrl = self._ext_args()
+            _lib.check(self.lib.mr_adam_step_ex(
+                self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(),
+                self.grad.data_ptr(), self.n_params, self.step.data_ptr(), self.lr, self.betas[0],
+                self.betas[1], self.eps, self.max_grad_norm, None if info is None else info.data_ptr(), tkl, ctrl,
+                mb_index, self._stream()))
+            return
         _lib.check(self.lib.mr_adam_step(
             self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(),
             self.grad.data_ptr(), self.n_params, self.step.data_ptr(), self.lr, self.betas[0],
@@ -86,8 +128,21 @@ class PpoUpdater:
             self._stream()))
 
     def train_epoch(self, buf: dict, perm: torch.Tensor, stats: torch.Tensor, batch_size: int, N: int, T: int,
-                    info: torch.Tensor | None = None):
-        """All minibatches of one epoch, launched from C (single-GPU path)."""
+                    info: torch.Tensor | None = None, mb0: int = 0):
+        """All minibatches of one epoch, launched from C (single-GPU path).  mb0: index of the epoch's first
+        minibatch in the update (target_kl)."""
+        if self.extended:
+            cvf, tkl, ctrl = self._ext_args()
+            _lib.check(self.lib.mr_ppo_train_epoch_ex(
+                self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), self.step.data_ptr(),
+                self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(), buf["log_probs"].data_ptr(),
+                buf["advantages"].data_ptr(), buf["returns"].data_ptr(), perm.data_ptr(),
+                self.rows(min(perm.numel(), batch_size)).data_ptr(), perm.numel(), batch_size,
+                stats.data_ptr(), N, T, self.clip_range, self.ent_coef, self.vf_coef, int(self.normalize_advantage),
+                self.lr, self.betas[0], self.betas[1], self.eps, self.max_grad_norm, self.partials.data_ptr(),
+                self.grad.data_ptr(), None if info is None else info.data_ptr(),
+                buf["values"].data_ptr() if cvf > 0 else None, cvf, tkl, ctrl, mb0, self._stream()))
+            return
         _lib.check(self.lib.mr_ppo_train_epoch(
             self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), self.step.data_ptr(),
             self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(), buf["log_probs"].data_ptr(),
@@ -99,11 +154,18 @@ class PpoUpdater:
 
     def pack(self, buf: dict) -> torch.Tensor:
         """Packed sample records of a rollout (mr_ppo_pack_samples): what train_epoch_fused gathers from.
-        Build them once per rollout, after GAE; they stay valid for all epochs of the update."""
+        Build them once per rollout, after GAE; they stay valid for all epochs of the update.  With clip_range_vf
+        the records also carry buf["values"], the rollout's V(s) (mr_ppo_pack_samples_vf)."""
         n_rows = buf["log_probs"].numel()
         rf = int(self.lib.mr_ppo_record_floats(self.obs_dim))
         if getattr(self, "_rec", None) is None or self._rec.numel() != n_rows * rf:
             self._rec = torch.empty(n_rows * rf, dtype=torch.float32, device=self.device)
+        if self.clip_range_vf is not None:
+            _lib.check(self.lib.mr_ppo_pack_samples_vf(
+                self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(), buf["log_probs"].data_ptr(),
+                buf["advantages"].data_ptr(), buf["returns"].data_ptr(), buf["values"].data_ptr(), n_rows,
+                self._rec.data_ptr(), self._stream()))
+            return self._rec
         _lib.check(self.lib.mr_ppo_pack_samples(
             self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(), buf["log_probs"].data_ptr(),
             buf["advantages"].data_ptr(), buf["returns"].data_ptr(), n_rows, self._rec.data_ptr(), self._stream()))
@@ -135,13 +197,27 @@ class PpoUpdater:
         return stats, self._rows_all
 
     def train_epoch_fused(self, buf: dict | None, perm: torch.Tensor | None, stats: torch.Tensor, batch_size: int, N: int,
-                          T: int, info: torch.Tensor | None = None, xchg=None, rows: torch.Tensor | None = None):
+                          T: int, info: torch.Tensor | None = None, xchg=None, rows: torch.Tensor | None = None,
+                          mb0: int = 0):
         """One cooperative launch for the whole epoch; xchg (PeerExchange) adds the in-kernel
         NVLink all-reduce of the gradient (stats must then be the all-reduced, global sums).
         buf = the rollout arrays (packed here) or None to reuse the records of the last pack().
-        Either perm (int64 env-major sample ids) or rows (one row of prepare_epochs' output) names the samples."""
+        Either perm (int64 env-major sample ids) or rows (one row of prepare_epochs' output) names the samples.
+        mb0: index of the launch's first minibatch in the update (target_kl)."""
         rec = self.pack(buf) if buf is not None else self._rec
         n = perm.numel() if perm is not None else rows.numel()
+        if self.extended:
+            cvf, tkl, ctrl = self._ext_args()
+            _lib.check(self.lib.mr_ppo_epoch_fused_ex(
+                self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), self.step.data_ptr(),
+                self.obs_dim, rec.data_ptr(), None if perm is None else perm.data_ptr(),
+                self.rows(n).data_ptr() if rows is None else rows.data_ptr(), n,
+                batch_size, stats.data_ptr(), N, T, self.clip_range,
+                self.ent_coef, self.vf_coef, int(self.normalize_advantage), self.lr, self.betas[0], self.betas[1],
+                self.eps, self.max_grad_norm, self.partials.data_ptr(), self.grad.data_ptr(),
+                None if info is None else info.data_ptr(), None if xchg is None else xchg.handle, cvf, tkl, ctrl, mb0,
+                self._stream()))
+            return
         _lib.check(self.lib.mr_ppo_epoch_fused(
             self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), self.step.data_ptr(),
             self.obs_dim, rec.data_ptr(), None if perm is None else perm.data_ptr(),
