@@ -187,7 +187,8 @@ int mr_adam_step(float* params, float* exp_avg, float* exp_avg_sq, const float* 
 /* ------------------------------------------------------------------------------------
  * Fused rollout.  Replaces [SB3] OnPolicyAlgorithm.collect_rollouts (n_steps = T) over the
  * vectorised env, including the time-out bootstrap  reward += gamma * V(terminal_obs),
- * Monitor's episode statistics and RolloutBuffer.add, in one launch (point env).
+ * Monitor's episode statistics and RolloutBuffer.add, in one launch (point env; plus two
+ * launches that file the finished episodes).
  *   last_obs [N][O], last_starts [N] f32 : in/out, carried between rollouts (_last_obs,
  *                                          _last_episode_starts)
  *   obs [T][N][O], act [T][N][2] (unclipped), rew/starts/val/logp [T][N] f32 : RolloutBuffer
@@ -195,13 +196,18 @@ int mr_adam_step(float* params, float* exp_avg, float* exp_avg_sq, const float* 
  *   eps [T][N][2] f32 standard-normal draws (parity mode: torch's CPU generator cannot be
  *        reproduced on the device) or NULL -> Philox4x32-10 keyed (seed; env_offset + n,
  *        noise_offset + t)
- *   ep_r [ring_cap] f64, ep_l [ring_cap] i32, ep_count [1] u64 : ring of finished episodes
- *        (Monitor's info["episode"]), head = *ep_count. */
+ *   ep_ret [T][N] f64, ep_len [T][N] i32 : scratch, Monitor's info["episode"] return and length,
+ *        written only at the (t, n) where an episode ended; ep_steps [T] i32 : scratch
+ *   ep_r [ring_cap] f64, ep_l [ring_cap] i32, ep_count [1] u64 : ring of finished episodes in SB3's
+ *        order (by step, then env index).  Episode k (0-based, counted over all rollouts) sits in
+ *        slot k % ring_cap; *ep_count = number of episodes so far.  A rollout that ends more than
+ *        ring_cap episodes files its newest ring_cap. */
 int mr_rollout(mr_env* env, const float* params, int64_t T, float* last_obs, float* last_starts,
                float* obs, float* act, float* rew, float* starts, float* val, float* logp,
                float* last_val, uint8_t* last_done, const float* eps, uint64_t seed,
-               uint64_t noise_offset, int64_t env_offset, double gamma, double* ep_r,
-               int32_t* ep_l, unsigned long long* ep_count, int ring_cap, void* stream);
+               uint64_t noise_offset, int64_t env_offset, double gamma, double* ep_ret,
+               int32_t* ep_len, int32_t* ep_steps, double* ep_r, int32_t* ep_l,
+               unsigned long long* ep_count, int ring_cap, void* stream);
 
 /* What [SB3] PPO.train logs after its epochs (SURVEY A.5), in one launch and without a host round trip.
  * info [n_rows][8]: the info rows of every minibatch of the update; values / returns [n] the flat buffer;
@@ -303,14 +309,16 @@ int mr_ppo_train_summary_ex(const float* info, int n_rows, const float* values, 
                             const float* params, float* out, double* scratch, const int* ctrl, void* stream);
 
 /* Same contract as mr_rollout, from the stand-alone env-step kernel plus ONE kernel between two env steps (the
- * finished step's RolloutBuffer.add bookkeeping -- time-out bootstrap, reward row, Monitor ring, start flags -- and
- * the next step's policy forward, Gaussian sample and log-prob): 2 T + 1 launches.  Works for both env kinds and
+ * finished step's RolloutBuffer.add bookkeeping -- time-out bootstrap, reward row, Monitor's episode records, start
+ * flags -- and the next step's policy forward, Gaussian sample and log-prob), then the two episode-filing launches:
+ * 2 T + 3 launches and a copy.  Works for both env kinds and
  * for envs with optional observation keys (rows of mr_env_obs_dim floats, at most 32); the car uses this path. */
 int mr_rollout_unfused(mr_env* env, const float* params, int64_t T, float* last_obs, float* last_starts,
                        float* obs, float* act, float* rew, float* starts, float* val, float* logp,
                        float* last_val, uint8_t* last_done, const float* eps, uint64_t seed,
-                       uint64_t noise_offset, int64_t env_offset, double gamma, double* ep_r,
-                       int32_t* ep_l, unsigned long long* ep_count, int ring_cap, void* stream);
+                       uint64_t noise_offset, int64_t env_offset, double gamma, double* ep_ret,
+                       int32_t* ep_len, int32_t* ep_steps, double* ep_r, int32_t* ep_l,
+                       unsigned long long* ep_count, int ring_cap, void* stream);
 
 /* Device-side minibatch index stream: out[0..n) <- a keyed pseudo-random permutation of 0..n-1
  * (a pure function of (seed, stream_id); one thread per index, no sort).  For runs that keep

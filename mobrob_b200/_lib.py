@@ -57,11 +57,11 @@ _SIGNATURES = {
                                    c_int64, c_int64, c_float, c_float, c_float, c_int, c_float, c_float,
                                    c_float, c_float, c_float, _P, _P, _P, _P, _P]),
     "mr_rollout": (c_int, [_P, _P, c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_uint64,
-                           c_uint64, c_int64, c_double, _P, _P, _P, c_int, _P]),
+                           c_uint64, c_int64, c_double, _P, _P, _P, _P, _P, _P, c_int, _P]),
     "mr_ppo_grad_partials": (c_int, [_P, c_int, _P, _P, _P, _P, _P, _P, _P, c_int64, _P, c_int64, c_int64,
                                      c_float, c_float, c_float, c_int, _P, _P, _P]),
     "mr_rollout_unfused": (c_int, [_P, _P, c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_uint64,
-                                   c_uint64, c_int64, c_double, _P, _P, _P, c_int, _P]),
+                                   c_uint64, c_int64, c_double, _P, _P, _P, _P, _P, _P, c_int, _P]),
     "mr_evaluate": (c_int, [_P, _P, c_int, c_int64, c_int64, c_uint64, c_uint64, c_int64, _P, _P, _P, _P, _P, _P,
                             _P]),
     "mr_device_permutation": (c_int, [c_uint64, c_uint64, c_int64, _P, _P]),

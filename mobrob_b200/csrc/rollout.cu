@@ -46,10 +46,8 @@ struct RolloutArgs {
     uint64_t noise_offset; // rollout counter * T (Philox counter word)
     int64_t env_offset;    // global index of env 0 (multi-GPU sharding)
     float gamma;
-    double* ep_r;          // episode ring (Monitor): returns
-    int32_t* ep_l;         //                          lengths
-    unsigned long long* ep_count;  // total finished episodes (ring head)
-    int ring_cap;
+    double* ep_ret;        // [T][N] Monitor's return and length of the episode that ended at (t, n), written only
+    int32_t* ep_len;       //        there (episode_records puts them into the ring in SB3's order)
 };
 
 template <int RO_WARPS, int RO_E>
@@ -138,9 +136,8 @@ __global__ void __launch_bounds__(RO_WARPS * 32) point_rollout_kernel(RolloutArg
             A.starts[row] = start_flag;
             r = point_env_step(h, A.st.cold, n, a0, a1, A.cfg, o_new, o_term);
             if (r.done) {
-                unsigned long long slot = atomicAdd(A.ep_count, 1ull) % (unsigned long long)A.ring_cap;
-                A.ep_r[slot] = r.ep_r;
-                A.ep_l[slot] = r.ep_l;
+                A.ep_ret[row] = r.ep_r;
+                A.ep_len[row] = r.ep_l;
             }
             start_flag = r.done ? 1.f : 0.f;
             done_flag = r.done;
@@ -182,9 +179,96 @@ __global__ void __launch_bounds__(RO_WARPS * 32) point_rollout_kernel(RolloutArg
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Monitor's finished episodes in SB3's order.  DummyVecEnv steps its envs in index order and collect_rollouts appends
+// each step's infos to ep_info_buffer, so the episodes of a rollout are ordered by (step, env).  The rollout kernels
+// leave them in [T][N] side buffers at the (t, n) where they ended; the done mask tells which entries are valid:
+// episode_starts[t + 1], or last_done at the last step.  Two launches put the newest ring_cap of them into the ring
+// (slot = global episode index % ring_cap) and advance the episode counter, with no host synchronisation.
+constexpr int EPR_THREADS = 256;
+
+__device__ __forceinline__ bool episode_ended(const float* starts, const uint8_t* last_done, int64_t t, int64_t T,
+                                              int64_t N, int64_t n) {
+    return t + 1 < T ? starts[(t + 1) * N + n] != 0.f : last_done[n] != 0;
+}
+
+// block t: the number of episodes that ended at step t; the counter gets the rollout's total
+__global__ void __launch_bounds__(EPR_THREADS) episode_count_kernel(const float* starts, const uint8_t* last_done,
+                                                                    int64_t T, int64_t N, int32_t* ep_steps,
+                                                                    unsigned long long* ep_count) {
+    __shared__ int part[EPR_THREADS / 32];
+    const int64_t t = blockIdx.x;
+    int c = 0;
+    for (int64_t n = threadIdx.x; n < N; n += EPR_THREADS) c += episode_ended(starts, last_done, t, T, N, n);
+    c = __reduce_add_sync(0xffffffffu, c);
+    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = c;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int s = 0;
+        for (int w = 0; w < EPR_THREADS / 32; ++w) s += part[w];
+        ep_steps[t] = s;
+        if (s) atomicAdd(ep_count, (unsigned long long)s);
+    }
+}
+
+// block t: the episodes that ended at step t, in env order, into ring slots (first index of the step + rank) % cap
+__global__ void __launch_bounds__(EPR_THREADS) episode_ring_kernel(const float* starts, const uint8_t* last_done,
+                                                                   const double* ep_ret, const int32_t* ep_len,
+                                                                   int64_t T, int64_t N, const int32_t* ep_steps,
+                                                                   const unsigned long long* ep_count, double* ep_r,
+                                                                   int32_t* ep_l, int ring_cap) {
+    __shared__ long long part[EPR_THREADS / 32];
+    __shared__ int warp_cnt[EPR_THREADS / 32];
+    const int64_t t = blockIdx.x;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    long long later = 0;   // episodes that ended after step t
+    for (int64_t s = t + 1 + threadIdx.x; s < T; s += EPR_THREADS) later += ep_steps[s];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) later += __shfl_down_sync(0xffffffffu, later, o);
+    if (lane == 0) part[w] = later;
+    __syncthreads();
+    later = 0;
+    for (int i = 0; i < EPR_THREADS / 32; ++i) later += part[i];
+    const int mine = ep_steps[t];
+    if (mine == 0 || later >= ring_cap) return;   // nothing ended here, or newer episodes fill the ring
+    const unsigned long long first = *ep_count - (unsigned long long)(later + mine);   // global index of the step's first
+    const long long skip = later + mine - ring_cap;   // > 0: the step's oldest episodes do not fit
+    int base = 0;
+    for (int64_t n0 = 0; n0 < N && base < mine; n0 += EPR_THREADS) {
+        const int64_t n = n0 + threadIdx.x;
+        const bool d = n < N && episode_ended(starts, last_done, t, T, N, n);
+        const unsigned bal = __ballot_sync(0xffffffffu, d);
+        if (lane == 0) warp_cnt[w] = __popc(bal);
+        __syncthreads();
+        int rank = base + __popc(bal & ((1u << lane) - 1u)), tot = 0;
+        for (int i = 0; i < EPR_THREADS / 32; ++i) {
+            rank += i < w ? warp_cnt[i] : 0;
+            tot += warp_cnt[i];
+        }
+        if (d && rank >= skip) {
+            const unsigned long long slot = (first + (unsigned long long)rank) % (unsigned long long)ring_cap;
+            ep_r[slot] = ep_ret[t * N + n];
+            ep_l[slot] = ep_len[t * N + n];
+        }
+        base += tot;
+        __syncthreads();
+    }
+}
+
 }  // namespace mr
 
 using namespace mr;
+
+static int episode_records(const float* starts, const uint8_t* last_done, const double* ep_ret, const int32_t* ep_len,
+                           int64_t T, int64_t N, int32_t* ep_steps, double* ep_r, int32_t* ep_l,
+                           unsigned long long* ep_count, int ring_cap, cudaStream_t stream) {
+    episode_count_kernel<<<(unsigned)T, EPR_THREADS, 0, stream>>>(starts, last_done, T, N, ep_steps, ep_count);
+    MR_CHECK_LAUNCH();
+    episode_ring_kernel<<<(unsigned)T, EPR_THREADS, 0, stream>>>(starts, last_done, ep_ret, ep_len, T, N, ep_steps,
+                                                                 ep_count, ep_r, ep_l, ring_cap);
+    MR_CHECK_LAUNCH();
+    return MR_OK;
+}
 
 template <int RO_WARPS, int RO_E>
 static int launch_rollout_cfg(const RolloutArgs& A, int64_t n_envs, cudaStream_t stream) {
@@ -225,14 +309,15 @@ extern "C" int mr_rollout(mr_env* env, const float* params, int64_t T, float* la
                           float* last_starts, float* obs, float* act, float* rew, float* starts,
                           float* val, float* logp, float* last_val, uint8_t* last_done,
                           const float* eps, uint64_t seed, uint64_t noise_offset,
-                          int64_t env_offset, double gamma, double* ep_r, int32_t* ep_l,
-                          unsigned long long* ep_count, int ring_cap, void* stream) {
+                          int64_t env_offset, double gamma, double* ep_ret, int32_t* ep_len,
+                          int32_t* ep_steps, double* ep_r, int32_t* ep_l, unsigned long long* ep_count,
+                          int ring_cap, void* stream) {
     MR_REQUIRE(env && params && last_obs && last_starts && obs && act && rew && starts && val &&
-                   logp && last_val && last_done && ep_r && ep_l && ep_count,
+                   logp && last_val && last_done && ep_ret && ep_len && ep_steps && ep_r && ep_l && ep_count,
                "NULL argument");
     MR_REQUIRE(env->kind == MR_ENV_POINT, "fused rollout is built for the point env");
     MR_REQUIRE(env->cfg.obs_flags == 0, "fused rollout is built for the default observation (use mr_rollout_unfused)");
-    MR_REQUIRE(T > 0 && ring_cap > 0, "T and ring_cap must be positive");
+    MR_REQUIRE(T > 0 && T <= INT32_MAX && ring_cap > 0, "T must be in 1 .. 2^31 - 1 and ring_cap positive");
     RolloutArgs A;
     A.st = env->point;
     A.cfg = env->cfg;
@@ -245,8 +330,11 @@ extern "C" int mr_rollout(mr_env* env, const float* params, int64_t T, float* la
     A.last_val = last_val; A.last_done = last_done;
     A.eps = eps; A.seed = seed; A.noise_offset = noise_offset; A.env_offset = env_offset;
     A.gamma = (float)gamma;
-    A.ep_r = ep_r; A.ep_l = ep_l; A.ep_count = ep_count; A.ring_cap = ring_cap;
-    return launch_rollout(A, env->n, (cudaStream_t)stream);
+    A.ep_ret = ep_ret; A.ep_len = ep_len;
+    const int rc = launch_rollout(A, env->n, (cudaStream_t)stream);
+    if (rc != MR_OK) return rc;
+    return episode_records(starts, last_done, ep_ret, ep_len, T, env->n, ep_steps, ep_r, ep_l, ep_count, ring_cap,
+                           (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -262,7 +350,7 @@ struct StepArgs {
     const float* params;
     int O;
     int64_t N, t;
-    int record;            // finish step t - 1: time-out bootstrap, reward row, episode ring, start flags
+    int record;            // finish step t - 1: time-out bootstrap, reward row, episode records, start flags
     int forward;           // open step t: buffer rows, policy forward, sampling
     float* last_obs;       // [N][O]  observation the env returned (in), unchanged
     float* last_starts;    // [N]     _last_episode_starts (updated by the record half)
@@ -275,7 +363,7 @@ struct StepArgs {
     // outputs of the env step t - 1
     const float* rew_tmp; const uint8_t* done; const uint8_t* trunc; const float* term_obs;
     const double* ep_ret_n; const int32_t* ep_len_n;
-    double* ep_r; int32_t* ep_l; unsigned long long* ep_count; int ring_cap;
+    double* ep_ret; int32_t* ep_len;   // [T][N] episodes that ended at (t - 1, n), as in RolloutArgs
 };
 
 // Between two env steps: [RolloutBuffer.add bookkeeping of the step that just ran] + [policy forward, Gaussian
@@ -318,9 +406,8 @@ __global__ void __launch_bounds__(RS_WARPS * 32) rollout_step_kernel(StepArgs A)
                 start_flag = d ? 1.f : 0.f;
                 A.last_starts[n] = start_flag;
                 if (d) {
-                    const unsigned long long slot = atomicAdd(A.ep_count, 1ull) % (unsigned long long)A.ring_cap;
-                    A.ep_r[slot] = A.ep_ret_n[n];
-                    A.ep_l[slot] = A.ep_len_n[n];
+                    A.ep_ret[(A.t - 1) * A.N + n] = A.ep_ret_n[n];
+                    A.ep_len[(A.t - 1) * A.N + n] = A.ep_len_n[n];
                 }
             }
         }
@@ -371,11 +458,12 @@ extern "C" int mr_rollout_unfused(mr_env* env, const float* params, int64_t T, f
                                   float* last_starts, float* obs, float* act, float* rew, float* starts,
                                   float* val, float* logp, float* last_val, uint8_t* last_done,
                                   const float* eps, uint64_t seed, uint64_t noise_offset,
-                                  int64_t env_offset, double gamma, double* ep_r, int32_t* ep_l,
-                                  unsigned long long* ep_count, int ring_cap, void* stream) {
+                                  int64_t env_offset, double gamma, double* ep_ret, int32_t* ep_len,
+                                  int32_t* ep_steps, double* ep_r, int32_t* ep_l, unsigned long long* ep_count,
+                                  int ring_cap, void* stream) {
     MR_REQUIRE(env && params && last_obs && last_starts && obs && act && rew && starts && val && logp &&
-                   last_val && last_done && ep_r && ep_l && ep_count, "NULL argument");
-    MR_REQUIRE(T > 0 && ring_cap > 0, "T and ring_cap must be positive");
+                   last_val && last_done && ep_ret && ep_len && ep_steps && ep_r && ep_l && ep_count, "NULL argument");
+    MR_REQUIRE(T > 0 && T <= INT32_MAX && ring_cap > 0, "T must be in 1 .. 2^31 - 1 and ring_cap positive");
     cudaStream_t s = (cudaStream_t)stream;
     const int64_t N = env->n;
     const int O = mr_env_obs_dim(env);
@@ -408,7 +496,7 @@ extern "C" int mr_rollout_unfused(mr_env* env, const float* params, int64_t T, f
     A.obs = obs; A.act = act; A.rew = rew; A.starts = starts; A.val = val; A.logp = logp; A.last_val = last_val;
     A.eps = eps; A.seed = seed; A.noise_offset = noise_offset; A.env_offset = env_offset; A.gamma = (float)gamma;
     A.rew_tmp = rew_tmp; A.done = done; A.trunc = trunc; A.term_obs = term_obs; A.ep_ret_n = ep_ret_n; A.ep_len_n = ep_len_n;
-    A.ep_r = ep_r; A.ep_l = ep_l; A.ep_count = ep_count; A.ring_cap = ring_cap;
+    A.ep_ret = ep_ret; A.ep_len = ep_len;
     for (int64_t t = 0; t <= T; ++t) {
         A.t = t; A.record = t > 0; A.forward = t < T;
         mr::rollout_step_kernel<<<blocks, RS_WARPS * 32, smem, s>>>(A);
@@ -418,5 +506,5 @@ extern "C" int mr_rollout_unfused(mr_env* env, const float* params, int64_t T, f
         if (rc != MR_OK) return rc;
     }
     MR_CUDA(cudaMemcpyAsync(last_done, done, N, cudaMemcpyDeviceToDevice, s));
-    return MR_OK;
+    return episode_records(starts, last_done, ep_ret, ep_len, T, N, ep_steps, ep_r, ep_l, ep_count, ring_cap, s);
 }

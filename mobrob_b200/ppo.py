@@ -198,9 +198,14 @@ class PPO:
         self.last_done = torch.zeros(N, dtype=torch.uint8, device=self.device)
         self._last_obs = None
         self._last_episode_starts = None
+        # Monitor's finished episodes: the ring in SB3's (step, env) order, and the rollout kernels' [T][N] records
+        # it is filled from
         self.ep_r = torch.zeros(EP_RING, dtype=torch.float64, device=self.device)
         self.ep_l = torch.zeros(EP_RING, dtype=torch.int32, device=self.device)
         self.ep_count = torch.zeros(1, dtype=torch.int64, device=self.device)
+        self.ep_ret_tn = torch.zeros((T, N), dtype=torch.float64, device=self.device)
+        self.ep_len_tn = torch.zeros((T, N), dtype=torch.int32, device=self.device)
+        self.ep_steps = torch.zeros(T, dtype=torch.int32, device=self.device)
         self.lib = _lib.load()
 
     def get_env(self):
@@ -249,8 +254,9 @@ class PPO:
             b["rewards"].data_ptr(), b["episode_starts"].data_ptr(), b["values"].data_ptr(),
             b["log_probs"].data_ptr(), self.last_val.data_ptr(), self.last_done.data_ptr(),
             None if eps is None else eps.data_ptr(), seed, self._rollout_count * self.n_steps,
-            env.first_rank, float(self.gamma), self.ep_r.data_ptr(), self.ep_l.data_ptr(),
-            self.ep_count.data_ptr(), EP_RING, self._stream()))
+            env.first_rank, float(self.gamma), self.ep_ret_tn.data_ptr(), self.ep_len_tn.data_ptr(),
+            self.ep_steps.data_ptr(), self.ep_r.data_ptr(), self.ep_l.data_ptr(), self.ep_count.data_ptr(), EP_RING,
+            self._stream()))
         self._rollout_count += 1
         _lib.check(self.lib.mr_gae(b["rewards"].data_ptr(), b["values"].data_ptr(),
                                    b["episode_starts"].data_ptr(), self.last_val.data_ptr(),
@@ -264,8 +270,9 @@ class PPO:
         return d.get_world_size() if d is not None else 1
 
     def _snapshot_async(self):
-        """Enqueue the D2H reads one logging step needs -- Monitor's newest episodes (ep_info_buffer),
-        the previous train()'s statistics -- into pinned memory; returns the event to wait for.
+        """Enqueue the D2H reads one logging step needs -- Monitor's newest episodes (ep_info_buffer: the last W
+        slots of the ring, which the rollout fills in SB3's order), the previous train()'s statistics -- into pinned
+        memory; returns the event to wait for.
         Nothing here blocks the host: train() of this iteration is enqueued behind it."""
         W = self._stats_window_size
         if getattr(self, "_snap", None) is None:

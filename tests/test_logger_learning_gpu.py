@@ -106,13 +106,12 @@ def test_logger_keys_and_values_match_sb3(cuda_lib, golden_dir, tmp_path, monkey
             assert key in rec, key
             tol = dict(rtol=2e-2, atol=2e-5) if key in ("train/approx_kl", "train/clip_fraction") else dict(rtol=3e-3, atol=1e-6)
             np.testing.assert_allclose(rec[key], expect[k - 1][key], err_msg=f"{key} at dump {k}", **tol)
-    # Monitor's episode statistics: the last dump holds the mean over every episode finished so far (< 100),
-    # except those that ended on the final step of the final rollout (drained with the next iteration)
-    done_by_last_dump = [e for e in eps]
+    # Monitor's episode statistics: the last dump holds the mean over the newest 100 episodes finished so far, in
+    # SB3's order -- here every one of them (< 100), those that ended on the final step of the final rollout included
+    window = eps[-100:]
     got_l, got_r = dumps[-1][1]["rollout/ep_len_mean"], dumps[-1][1]["rollout/ep_rew_mean"]
-    cand_l = {round(float(np.mean([l for l, _ in done_by_last_dump[:m]])), 6) for m in range(max(1, len(eps) - n), len(eps) + 1)}
-    assert round(got_l, 6) in cand_l, (got_l, sorted(cand_l))
-    assert abs(got_r - np.mean([r for _, r in eps])) < 0.5
+    assert got_l == float(np.mean([l for l, _ in window])), (got_l, [l for l, _ in window])
+    assert abs(got_r - np.mean([r for _, r in window])) < 1e-3   # buffer rewards are Monitor's rounded to float32
     # tensorboard: events under <tensorboard_log>/PPO_1 (the reference's tensorboard_log + SB3's run naming)
     run = tmp_path / "tensorboard" / "PPO_1"
     assert run.is_dir() and any(f.startswith("events.out.tfevents") for f in os.listdir(run))

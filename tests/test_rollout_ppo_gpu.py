@@ -1,80 +1,14 @@
 """Fused rollout + GAE + PPO update vs the oracle's collect_rollouts / PPO.train restatement."""
-import copy
 import os
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import point_oracle as po, sb3_oracle
-from oracle.vec_oracle import GoalVecOracle
+from oracle import sb3_oracle
+from rollout_oracle import setup as _setup, teacher_forced_check as _teacher_forced_check
 
 pytestmark = pytest.mark.gpu
-
-
-def _setup(golden_dir, n, T, seed, time_limit, pretrained, **ppo_kw):
-    from mobrob_b200 import GpuVecEnv
-    from mobrob_b200.ppo import PPO
-
-    env = GpuVecEnv("point", n, seed=None, time_limit=time_limit, terminate_on_goal=True)
-    model = PPO("MlpPolicy", env, n_steps=T, seed=seed, gae_lambda=0.5, ent_coef=0.05, **ppo_kw)
-    ref_pol = sb3_oracle.MlpPolicyOracle(14)
-    if pretrained:
-        w = dict(np.load(os.path.join(golden_dir, "point_policy.npz")))
-        model.policy.load_state_dict({k: torch.as_tensor(v) for k, v in w.items()})
-        ref_pol.load_numpy(w)
-    else:
-        ref_pol.load_state_dict({k: v.cpu() for k, v in model.policy.state_dict().items()})
-    venv = GoalVecOracle(po.PointBody(n), seed=seed, time_limit=time_limit, terminate_on_goal=True)
-    return model, ref_pol, venv
-
-
-def _teacher_forced_check(model, ref_pol, venv, eps, first, last_obs_ref, gamma=0.99):
-    """Replay the device rollout through the oracle step by step.
-
-    The point robot's turning servo is stiff against the 2 ms timestep (explicit-Euler factor
-    about -3.9 per substep inside the un-saturated band), so trajectories are sensitive to
-    1e-6 differences in un-saturated actions (DESIGN.md "Sensitivity").  Parity is therefore
-    checked per component on identical inputs: the policy on the device's observations, the
-    environment on the device's float32 actions.
-    """
-    b = {k: v.cpu().numpy() for k, v in model.buf.items()}
-    T, n = b["rewards"].shape
-    obs_ref = last_obs_ref
-    n_trunc = 0
-    ep_infos = []
-    for t in range(T):
-        np.testing.assert_allclose(b["obs"][t], obs_ref, rtol=1e-5, atol=2e-6, err_msg=f"obs t={t}")
-        with torch.no_grad():
-            a_ref, v_ref, lp_ref = ref_pol.forward_with_noise(torch.as_tensor(b["obs"][t]), torch.as_tensor(eps[t]))
-        a_scale = max(1.0, float(a_ref.abs().max()))
-        assert np.abs(b["actions"][t] - a_ref.numpy()).max() <= 1e-5 * a_scale, f"actions t={t}"
-        np.testing.assert_allclose(b["values"][t], v_ref.numpy(), rtol=1e-5, atol=1e-5)
-        np.testing.assert_allclose(b["log_probs"][t], lp_ref.numpy(), rtol=1e-5, atol=1e-5)
-        obs_ref, rew, done, info = venv.step(np.clip(b["actions"][t], -1.0, 1.0))
-        trunc = done & info["truncated"]
-        if trunc.any():
-            with torch.no_grad():
-                _, tv = ref_pol.mean_value(torch.as_tensor(info["terminal_obs"][trunc]))
-            rew[trunc] += gamma * tv.numpy()
-            n_trunc += int(trunc.sum())
-        for i in np.nonzero(done)[0]:
-            ep_infos.append((float(info["ep_r"][i]), int(info["ep_l"][i])))
-        np.testing.assert_allclose(b["rewards"][t], rew, rtol=1e-5, atol=2e-6, err_msg=f"rewards t={t}")
-        nxt = b["episode_starts"][t + 1] if t + 1 < T else model._last_episode_starts.cpu().numpy()
-        np.testing.assert_array_equal(nxt.astype(bool), done, err_msg=f"done flags t={t}")
-    np.testing.assert_array_equal(b["episode_starts"][0].astype(bool), first)
-    np.testing.assert_allclose(model._last_obs.cpu().numpy(), obs_ref, rtol=1e-5, atol=2e-6)
-    with torch.no_grad():
-        _, lv = ref_pol.mean_value(torch.as_tensor(obs_ref))
-    np.testing.assert_allclose(model.last_val.cpu().numpy(), lv.numpy(), rtol=1e-5, atol=1e-5)
-    np.testing.assert_array_equal(model.last_done.cpu().numpy().astype(bool), done)
-    # GAE: bit exact on the device's own inputs
-    adv, ret = sb3_oracle.gae_numpy(b["rewards"], b["values"], b["episode_starts"],
-                                    model.last_val.cpu().numpy(), done, gamma, model.gae_lambda)
-    np.testing.assert_array_equal(b["advantages"], adv)
-    np.testing.assert_array_equal(b["returns"], ret)
-    return obs_ref, done, n_trunc, ep_infos
 
 
 @pytest.mark.parametrize("pretrained,time_limit", [(True, 1000), (False, 40)])
