@@ -164,15 +164,8 @@ int mr_ppo_grad(const float* params, int obs_dim, const float* obs, const float*
                 const float* old_logp, const float* adv, const float* ret, const int64_t* perm,
                 int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
                 float clip_range, float ent_coef, float vf_coef, int normalize_adv, float rank_share,
-                float* partials, float* grad, void* stream);
-
-/* The forward/backward kernel of mr_ppo_grad alone: per-CTA partial gradients, no reduction
- * (*n_parts rows of `partials` are valid).  Exposed so bench.py can time the dominant kernel. */
-int mr_ppo_grad_partials(const float* params, int obs_dim, const float* obs, const float* act,
-                         const float* old_logp, const float* adv, const float* ret, const int64_t* perm,
-                         int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
-                         float clip_range, float ent_coef, float vf_coef, int normalize_adv, float* partials,
-                         int* n_parts, void* stream);
+                float* partials, float* grad, const float* old_values, float clip_range_vf, const int* ctrl,
+                void* stream);
 
 /* clip_grad_norm_(max_grad_norm) then torch.optim.Adam.step (eps as given; SB3 uses 1e-5).
  * step: device int64[2]: [0] = Adam step count (state["step"]), incremented; [1] = launch-internal
@@ -182,7 +175,7 @@ int mr_ppo_grad_partials(const float* params, int obs_dim, const float* obs, con
  * logging needs no extra copy. */
 int mr_adam_step(float* params, float* exp_avg, float* exp_avg_sq, const float* grad, int n_params,
                  int64_t* step, float lr, float beta1, float beta2, float eps, float max_grad_norm,
-                 float* info, void* stream);
+                 float* info, float target_kl, int* ctrl, int64_t mb_index, void* stream);
 
 /* ------------------------------------------------------------------------------------
  * Fused rollout.  Replaces [SB3] OnPolicyAlgorithm.collect_rollouts (n_steps = T) over the
@@ -214,9 +207,10 @@ int mr_rollout(mr_env* env, const float* params, int64_t T, float* last_obs, flo
  * params: the flat parameter vector after the update.  out [12] f32: [0:4] mean policy_gradient_loss,
  * value_loss, clip_fraction, approx_kl; [4:6] the last minibatch's policy and value loss; [6]
  * explained_variance(values, returns) (nan if var(returns) == 0); [7:9] log_std; [9] mean entropy_loss;
- * [10] the last minibatch's entropy_loss; [11] n_rows.  scratch: 8 doubles, zero before the first call. */
+ * [10] the last minibatch's entropy_loss; [11] n_rows.  scratch: 8 doubles, zero before the first call.
+ * ctrl: the update's control word (target_kl, below) or NULL. */
 int mr_ppo_train_summary(const float* info, int n_rows, const float* values, const float* returns, int64_t n,
-                         const float* params, float* out, double* scratch, void* stream);
+                         const float* params, float* out, double* scratch, const int* ctrl, void* stream);
 
 /* One epoch of PPO.train on one GPU: for every minibatch of perm, mr_ppo_grad then mr_adam_step,
  * launched back to back from C (no host round trip between minibatches).  stats [n_mb][3] from
@@ -226,7 +220,9 @@ int mr_ppo_train_epoch(float* params, float* exp_avg, float* exp_avg_sq, int64_t
                        const float* ret, const int64_t* perm, int32_t* rows, int64_t n_samples,
                        int64_t batch_size, const double* stats, int64_t N, int64_t T, float clip_range,
                        float ent_coef, float vf_coef, int normalize_adv, float lr, float beta1, float beta2,
-                       float eps, float max_grad_norm, float* partials, float* grad, float* info, void* stream);
+                       float eps, float max_grad_norm, float* partials, float* grad, float* info,
+                       const float* old_values, float clip_range_vf, float target_kl, int* ctrl, int64_t mb0,
+                       void* stream);
 
 /* ------------------------------------------------------------------------------------
  * Fused epoch: every minibatch of one epoch of PPO.train in ONE cooperative launch (forward,
@@ -250,63 +246,34 @@ int mr_xchg_status(mr_xchg* x, int* timed_out);
 /* The epoch kernel gathers its minibatches from PACKED sample records, one per buffer row (t * N + n):
  * mr_ppo_record_floats(obs_dim) floats = [obs | 0.. | 1 | a0 a1 old_logp adv | ret old_value 0 0] (96 B for
  * the point robot, 160 B for the car).  mr_ppo_pack_samples builds them once per rollout (after GAE) from
- * the RolloutBuffer arrays, with old_value = 0; rec is caller-owned, n_rows * mr_ppo_record_floats floats. */
+ * the RolloutBuffer arrays; old_value = values (the rollout's V(s) [T][N], needed with clip_range_vf) or 0 when
+ * values = NULL.  rec is caller-owned, n_rows * mr_ppo_record_floats floats. */
 int mr_ppo_record_floats(int obs_dim);
 int mr_ppo_pack_samples(int obs_dim, const float* obs, const float* act, const float* old_logp, const float* adv,
-                        const float* ret, int64_t n_rows, float* rec, void* stream);
+                        const float* ret, const float* values, int64_t n_rows, float* rec, void* stream);
 int mr_ppo_epoch_fused(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
                        const float* rec, const int64_t* perm, int32_t* rows, int64_t n_samples,
                        int64_t batch_size, const double* stats, int64_t N, int64_t T,
                        float clip_range, float ent_coef, float vf_coef, int normalize_adv, float lr,
                        float beta1, float beta2, float eps, float max_grad_norm, float* partials,
-                       float* grad, float* info, mr_xchg* xchg, void* stream);
+                       float* grad, float* info, mr_xchg* xchg, float clip_range_vf, float target_kl, int* ctrl,
+                       int64_t mb0, void* stream);
 
-/* ------------------------------------------------------------------------------------
- * [SB3] PPO's clip_range_vf and target_kl.  The *_ex / *_vf entry points take the arguments of the calls above
- * plus the following; with clip_range_vf <= 0, target_kl <= 0 and ctrl = NULL they compute exactly what those do.
- *   clip_range_vf > 0: value_loss = mse(returns, old_value + clamp(V - old_value, -c, c)), old_value being the
- *       rollout's values [T][N] (RolloutBuffer.values): passed as old_values to the per-launch calls, packed into
- *       the records by mr_ppo_pack_samples_vf for the fused one.
- *   target_kl > 0: per minibatch, after its losses and statistics, approx_kl > 1.5 * target_kl (compared in
- *       double) stops the update: that minibatch is not applied and no later one runs.
- *   ctrl: the update's control word, one int32 of caller-owned device memory, zero before the update's first
- *       call (the caller clears it once per update).  A stop after the k-th minibatch of the update (counted over
- *       all its calls from mb0 / mb_index = 0) sets it to k; every later call of the update then returns at entry
- *       in its kernels and changes nothing.  Required with target_kl > 0.
- * After a stop the info row of the stopping minibatch holds its statistics with the unchanged step count, and
- * `grad` holds its gradient (the fused call: also when a later launch of the update returns at entry; the per-launch
- * calls: on one GPU -- a host all-reduce of later minibatches still sums the unchanged vector). */
-int mr_ppo_pack_samples_vf(int obs_dim, const float* obs, const float* act, const float* old_logp, const float* adv,
-                           const float* ret, const float* values, int64_t n_rows, float* rec, void* stream);
-int mr_ppo_epoch_fused_ex(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
-                          const float* rec, const int64_t* perm, int32_t* rows, int64_t n_samples,
-                          int64_t batch_size, const double* stats, int64_t N, int64_t T,
-                          float clip_range, float ent_coef, float vf_coef, int normalize_adv, float lr,
-                          float beta1, float beta2, float eps, float max_grad_norm, float* partials,
-                          float* grad, float* info, mr_xchg* xchg, float clip_range_vf, float target_kl, int* ctrl,
-                          int64_t mb0, void* stream);
-int mr_ppo_grad_ex(const float* params, int obs_dim, const float* obs, const float* act,
-                   const float* old_logp, const float* adv, const float* ret, const int64_t* perm,
-                   int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
-                   float clip_range, float ent_coef, float vf_coef, int normalize_adv, float rank_share,
-                   float* partials, float* grad, const float* old_values, float clip_range_vf, const int* ctrl,
-                   void* stream);
-int mr_adam_step_ex(float* params, float* exp_avg, float* exp_avg_sq, const float* grad, int n_params,
-                    int64_t* step, float lr, float beta1, float beta2, float eps, float max_grad_norm,
-                    float* info, float target_kl, int* ctrl, int64_t mb_index, void* stream);
-int mr_ppo_train_epoch_ex(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
-                          const float* obs, const float* act, const float* old_logp, const float* adv,
-                          const float* ret, const int64_t* perm, int32_t* rows, int64_t n_samples,
-                          int64_t batch_size, const double* stats, int64_t N, int64_t T, float clip_range,
-                          float ent_coef, float vf_coef, int normalize_adv, float lr, float beta1, float beta2,
-                          float eps, float max_grad_norm, float* partials, float* grad, float* info,
-                          const float* old_values, float clip_range_vf, float target_kl, int* ctrl, int64_t mb0,
-                          void* stream);
-/* mr_ppo_train_summary over the minibatches the update evaluated: with ctrl != NULL recording a stop after k
- * minibatches, the means cover rows [0, k), "last" is row k - 1, out[11] = k, and out[12] = row k - 1's
- * approx_kl (out then has 13 floats).  ctrl = NULL: all n_rows, out [12], as mr_ppo_train_summary. */
-int mr_ppo_train_summary_ex(const float* info, int n_rows, const float* values, const float* returns, int64_t n,
-                            const float* params, float* out, double* scratch, const int* ctrl, void* stream);
+/* [SB3] PPO's clip_range_vf and target_kl: the trailing arguments of mr_ppo_grad, mr_adam_step, mr_ppo_train_epoch,
+ * mr_ppo_epoch_fused and mr_ppo_train_summary.  clip_range_vf <= 0, target_kl <= 0 and ctrl = NULL turn both off
+ * (and launch the default kernels).  clip_range_vf > 0: value_loss = mse(returns, old_value + clamp(V - old_value,
+ * -c, c)), old_value being the rollout's values [T][N] (RolloutBuffer.values), passed as old_values to the
+ * per-launch calls and packed into the records by mr_ppo_pack_samples for the fused one.  target_kl > 0 (requires
+ * ctrl): per minibatch, after its losses and statistics, approx_kl > 1.5 * target_kl (compared in double) stops the
+ * update: that minibatch is not applied and no later one runs.  ctrl is the update's control word, one int32 of
+ * caller-owned device memory that the caller zeroes once per update; a stop after the k-th minibatch of the update
+ * (counted over all its calls from mb0 / mb_index = 0) sets it to k, and every later call of the update returns at
+ * entry in its kernels and changes nothing.  After a stop the info row of the stopping minibatch holds its
+ * statistics with the unchanged step count, and `grad` holds its gradient (the fused call: also when a later launch
+ * of the update returns at entry; the per-launch calls: on one GPU -- a host all-reduce of later minibatches still
+ * sums the unchanged vector).  mr_ppo_train_summary with a ctrl recording a stop after k minibatches averages rows
+ * [0, k), takes row k - 1 as "last", sets out[11] = k and out[12] = row k - 1's approx_kl (out then has 13 floats);
+ * with ctrl = NULL it covers all n_rows and writes 12 floats. */
 
 /* Same contract as mr_rollout, from the stand-alone env-step kernel plus ONE kernel between two env steps (the
  * finished step's RolloutBuffer.add bookkeeping -- time-out bootstrap, reward row, Monitor's episode records, start
@@ -320,11 +287,10 @@ int mr_rollout_unfused(mr_env* env, const float* params, int64_t T, float* last_
                        int32_t* ep_len, int32_t* ep_steps, double* ep_r, int32_t* ep_l,
                        unsigned long long* ep_count, int ring_cap, void* stream);
 
-/* Device-side minibatch index stream: out[0..n) <- a keyed pseudo-random permutation of 0..n-1
- * (a pure function of (seed, stream_id); one thread per index, no sort).  For runs that keep
- * RolloutBuffer.get's indices on the device (PPO(permutation="device")). */
-int mr_device_permutation(uint64_t seed, uint64_t stream_id, int64_t n, int64_t* out, void* stream);
-/* `count` (1..32) permutations in one launch: out [count][n], h_stream_ids [count] in host memory. */
+/* Device-side minibatch index streams: out[e][0..n) <- a keyed pseudo-random permutation of 0..n-1, a pure
+ * function of (seed, h_stream_ids[e]); one thread per index, no sort.  `count` (1..32) permutations in one launch:
+ * out [count][n], h_stream_ids [count] in host memory.  For runs that keep RolloutBuffer.get's indices on the
+ * device (PPO(permutation="device")). */
 int mr_device_permutations(uint64_t seed, const uint64_t* h_stream_ids, int count, int64_t n, int64_t* out,
                            void* stream);
 

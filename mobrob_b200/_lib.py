@@ -42,48 +42,32 @@ _SIGNATURES = {
     "mr_ppo_epoch_scratch_floats": (c_int, [c_int]),
     "mr_ppo_adv_stats": (c_int, [_P, _P, c_int64, c_int64, c_int64, c_int64, _P, _P]),
     "mr_ppo_grad": (c_int, [_P, c_int, _P, _P, _P, _P, _P, _P, _P, c_int64, _P, c_int64, c_int64,
-                            c_float, c_float, c_float, c_int, c_float, _P, _P, _P]),
+                            c_float, c_float, c_float, c_int, c_float, _P, _P, _P, c_float, _P, _P]),
     "mr_ppo_train_epoch": (c_int, [_P, _P, _P, _P, c_int, _P, _P, _P, _P, _P, _P, _P, c_int64, c_int64, _P,
                                    c_int64, c_int64, c_float, c_float, c_float, c_int, c_float, c_float,
-                                   c_float, c_float, c_float, _P, _P, _P, _P]),
-    "mr_ppo_train_summary": (c_int, [_P, c_int, _P, _P, c_int64, _P, _P, _P, _P]),
+                                   c_float, c_float, c_float, _P, _P, _P, _P, c_float, c_float, _P, c_int64, _P]),
+    "mr_ppo_train_summary": (c_int, [_P, c_int, _P, _P, c_int64, _P, _P, _P, _P, _P]),
     "mr_xchg_create": (c_int, [c_int, c_int, c_int, c_int, POINTER(c_void_p), _P]),
     "mr_xchg_connect": (c_int, [_P, _P]),
     "mr_xchg_destroy": (None, [_P]),
     "mr_xchg_status": (c_int, [_P, POINTER(c_int)]),
     "mr_ppo_record_floats": (c_int, [c_int]),
-    "mr_ppo_pack_samples": (c_int, [c_int, _P, _P, _P, _P, _P, c_int64, _P, _P]),
+    "mr_ppo_pack_samples": (c_int, [c_int, _P, _P, _P, _P, _P, _P, c_int64, _P, _P]),
     "mr_ppo_epoch_fused": (c_int, [_P, _P, _P, _P, c_int, _P, _P, _P, c_int64, c_int64, _P,
                                    c_int64, c_int64, c_float, c_float, c_float, c_int, c_float, c_float,
-                                   c_float, c_float, c_float, _P, _P, _P, _P, _P]),
+                                   c_float, c_float, c_float, _P, _P, _P, _P, c_float, c_float, _P, c_int64, _P]),
     "mr_rollout": (c_int, [_P, _P, c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_uint64,
                            c_uint64, c_int64, c_double, _P, _P, _P, _P, _P, _P, c_int, _P]),
-    "mr_ppo_grad_partials": (c_int, [_P, c_int, _P, _P, _P, _P, _P, _P, _P, c_int64, _P, c_int64, c_int64,
-                                     c_float, c_float, c_float, c_int, _P, _P, _P]),
     "mr_rollout_unfused": (c_int, [_P, _P, c_int64, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_uint64,
                                    c_uint64, c_int64, c_double, _P, _P, _P, _P, _P, _P, c_int, _P]),
     "mr_evaluate": (c_int, [_P, _P, c_int, c_int64, c_int64, c_uint64, c_uint64, c_int64, _P, _P, _P, _P, _P, _P,
                             _P]),
-    "mr_device_permutation": (c_int, [c_uint64, c_uint64, c_int64, _P, _P]),
     "mr_device_permutations": (c_int, [c_uint64, _P, c_int, c_int64, _P, _P]),
     "mr_ppo_prepare_epochs": (c_int, [_P, _P, c_int, c_int64, c_int64, c_int64, c_int64, _P, _P, _P]),
     "mr_ppo_prepare_epochs_device": (c_int, [c_uint64, _P, c_int, _P, c_int64, c_int64, c_int64, c_int64, _P, _P, _P]),
     "mr_host_permutation": (c_int, [c_uint64, c_uint64, c_int64, _P]),
     "mr_adam_step": (c_int, [_P, _P, _P, _P, c_int, _P, c_float, c_float, c_float, c_float, c_float,
-                             _P, _P]),
-    # clip_range_vf / target_kl (include/mobrob_b200.h): the calls above plus their trailing arguments
-    "mr_ppo_pack_samples_vf": (c_int, [c_int, _P, _P, _P, _P, _P, _P, c_int64, _P, _P]),
-    "mr_ppo_epoch_fused_ex": (c_int, [_P, _P, _P, _P, c_int, _P, _P, _P, c_int64, c_int64, _P,
-                                      c_int64, c_int64, c_float, c_float, c_float, c_int, c_float, c_float,
-                                      c_float, c_float, c_float, _P, _P, _P, _P, c_float, c_float, _P, c_int64, _P]),
-    "mr_ppo_grad_ex": (c_int, [_P, c_int, _P, _P, _P, _P, _P, _P, _P, c_int64, _P, c_int64, c_int64,
-                               c_float, c_float, c_float, c_int, c_float, _P, _P, _P, c_float, _P, _P]),
-    "mr_adam_step_ex": (c_int, [_P, _P, _P, _P, c_int, _P, c_float, c_float, c_float, c_float, c_float,
-                                _P, c_float, _P, c_int64, _P]),
-    "mr_ppo_train_epoch_ex": (c_int, [_P, _P, _P, _P, c_int, _P, _P, _P, _P, _P, _P, _P, c_int64, c_int64, _P,
-                                      c_int64, c_int64, c_float, c_float, c_float, c_int, c_float, c_float,
-                                      c_float, c_float, c_float, _P, _P, _P, _P, c_float, c_float, _P, c_int64, _P]),
-    "mr_ppo_train_summary_ex": (c_int, [_P, c_int, _P, _P, c_int64, _P, _P, _P, _P, _P]),
+                             _P, c_float, _P, c_int64, _P]),
 }
 
 

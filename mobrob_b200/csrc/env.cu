@@ -391,7 +391,7 @@ using namespace mr;
 // =======================================================================================
 extern "C" {
 
-int mr_version(void) { return 100; }
+int mr_version(void) { return 101; }
 const char* mr_last_error(void) { return mr::g_err; }
 uint64_t mr_launch_count(void) { return mr::g_launches.load(); }
 

@@ -1,4 +1,4 @@
-// The device index stream of RolloutBuffer.get (mr_device_permutation): key schedule and the keyed bijection, shared by
+// The device index stream of RolloutBuffer.get (mr_device_permutations): key schedule and the keyed bijection, shared by
 // the kernels of ppo.cu and -- __host__ __device__ -- by the host build of tests/host/perm_host.cu, which checks them
 // against the numpy restatement (tests/perm_ref.py) without a GPU.
 #pragma once

@@ -5,11 +5,13 @@
 // gradients of the two 64-64 tanh towers are formed analytically.
 //
 // Two forms, both on the tensor cores (ppo_tc.cuh):
-//   * per launch (mr_ppo_grad / mr_adam_step; parity tests, the NCCL baseline path):
+//   * per launch (mr_ppo_grad / mr_adam_step, looped by mr_ppo_train_epoch; parity tests, the NCCL baseline path):
 //     ppo_grad_tc_kernel writes one partial gradient per CTA, ppo_reduce_kernel sums them in a fixed
 //     order, adam_kernel clips by global norm and applies torch's Adam;
 //   * per epoch (mr_ppo_epoch_fused; the product path): ppo_epoch_tc_kernel, one persistent
 //     cooperative launch for all minibatches of an epoch.
+// The update's entry points take SB3's clip_range_vf / target_kl and the update's control word as trailing
+// arguments (include/mobrob_b200.h); with those off (<= 0 / NULL) they launch the default instantiations.
 #include "mlp.cuh"
 #include "perm.cuh"
 #include "ppo_tc.cuh"
@@ -844,10 +846,6 @@ int mr_device_permutations(uint64_t seed, const uint64_t* h_stream_ids, int coun
     return MR_OK;
 }
 
-int mr_device_permutation(uint64_t seed, uint64_t stream_id, int64_t n, int64_t* out, void* stream) {
-    return mr_device_permutations(seed, &stream_id, 1, n, out, stream);
-}
-
 // Everything the epochs of one update need besides the parameters, for ALL epochs in two launches: the
 // per-minibatch advantage sums (mr_ppo_adv_stats) and the samples as buffer rows.  perm [n_epochs][n_samples],
 // stats [n_epochs][n_mb][3], rows [n_epochs][n_samples].  The permutations do not depend on the update, so
@@ -885,12 +883,13 @@ int mr_ppo_prepare_epochs_device(uint64_t seed, const uint64_t* h_stream_ids, in
     return MR_OK;
 }
 
-static int grad_partials(const float* params, int obs_dim, const float* obs, const float* act,
-                         const float* old_logp, const float* adv, const float* ret, const int64_t* perm,
-                         int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
-                         float clip_range, float ent_coef, float vf_coef, int normalize_adv, float* partials,
-                         int* n_parts, const float* old_values, float clip_range_vf, const int* ctrl, void* stream) {
-    MR_REQUIRE(params && obs && act && old_logp && adv && ret && perm && rows && mb_stats && partials,
+int mr_ppo_grad(const float* params, int obs_dim, const float* obs, const float* act,
+                const float* old_logp, const float* adv, const float* ret, const int64_t* perm,
+                int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
+                float clip_range, float ent_coef, float vf_coef, int normalize_adv, float rank_share,
+                float* partials, float* grad, const float* old_values, float clip_range_vf, const int* ctrl,
+                void* stream) {
+    MR_REQUIRE(params && obs && act && old_logp && adv && ret && perm && rows && mb_stats && partials && grad,
                "NULL argument");
     MR_REQUIRE(obs_dim > 0 && obs_dim <= MAX_OBS, "obs_dim out of range");
     MR_REQUIRE(mb_size > 0, "empty minibatch");
@@ -924,51 +923,16 @@ static int grad_partials(const float* params, int obs_dim, const float* obs, con
         else ppo_grad_tc_kernel<32, false><<<grid, tc::THREADS, tc::SMEM_BYTES, s>>>(A, obs_dim);
     }
     MR_CHECK_LAUNCH();
-    if (n_parts) *n_parts = grid;
-    return MR_OK;
-}
-
-int mr_ppo_grad_partials(const float* params, int obs_dim, const float* obs, const float* act,
-                         const float* old_logp, const float* adv, const float* ret, const int64_t* perm,
-                         int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
-                         float clip_range, float ent_coef, float vf_coef, int normalize_adv, float* partials,
-                         int* n_parts, void* stream) {
-    return grad_partials(params, obs_dim, obs, act, old_logp, adv, ret, perm, rows, mb_size, mb_stats, N, T,
-                         clip_range, ent_coef, vf_coef, normalize_adv, partials, n_parts, nullptr, 0.f, nullptr, stream);
-}
-
-int mr_ppo_grad_ex(const float* params, int obs_dim, const float* obs, const float* act,
-                   const float* old_logp, const float* adv, const float* ret, const int64_t* perm,
-                   int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
-                   float clip_range, float ent_coef, float vf_coef, int normalize_adv, float rank_share,
-                   float* partials, float* grad, const float* old_values, float clip_range_vf, const int* ctrl,
-                   void* stream) {
-    MR_REQUIRE(grad, "NULL argument");
-    int grid = 0;
-    int rc = grad_partials(params, obs_dim, obs, act, old_logp, adv, ret, perm, rows, mb_size, mb_stats, N, T,
-                           clip_range, ent_coef, vf_coef, normalize_adv, partials, &grid, old_values, clip_range_vf,
-                           ctrl, stream);
-    if (rc != MR_OK) return rc;
     const int stride = grad_stride(obs_dim);
-    ppo_reduce_kernel<<<ceil_div(stride, 128), 128, 0, (cudaStream_t)stream>>>(
-        partials, grid, obs_dim, ent_coef, mb_stats, grad, rank_share, ctrl);
+    ppo_reduce_kernel<<<ceil_div(stride, 128), 128, 0, s>>>(partials, grid, obs_dim, ent_coef, mb_stats, grad,
+                                                            rank_share, ctrl);
     MR_CHECK_LAUNCH();
     return MR_OK;
 }
 
-int mr_ppo_grad(const float* params, int obs_dim, const float* obs, const float* act,
-                const float* old_logp, const float* adv, const float* ret, const int64_t* perm,
-                int32_t* rows, int64_t mb_size, const double* mb_stats, int64_t N, int64_t T,
-                float clip_range, float ent_coef, float vf_coef, int normalize_adv, float rank_share,
-                float* partials, float* grad, void* stream) {
-    return mr_ppo_grad_ex(params, obs_dim, obs, act, old_logp, adv, ret, perm, rows, mb_size, mb_stats, N, T,
-                          clip_range, ent_coef, vf_coef, normalize_adv, rank_share, partials, grad, nullptr, 0.f,
-                          nullptr, stream);
-}
-
-int mr_adam_step_ex(float* params, float* exp_avg, float* exp_avg_sq, const float* grad, int n_params,
-                    int64_t* step, float lr, float beta1, float beta2, float eps, float max_grad_norm,
-                    float* info, float target_kl, int* ctrl, int64_t mb_index, void* stream) {
+int mr_adam_step(float* params, float* exp_avg, float* exp_avg_sq, const float* grad, int n_params,
+                 int64_t* step, float lr, float beta1, float beta2, float eps, float max_grad_norm,
+                 float* info, float target_kl, int* ctrl, int64_t mb_index, void* stream) {
     MR_REQUIRE(params && exp_avg && exp_avg_sq && grad && step, "NULL argument");
     MR_REQUIRE(!(target_kl > 0.f) || ctrl, "target_kl needs a control word");
     AdamArgs A{params, exp_avg, exp_avg_sq, grad, step, lr, beta1, beta2, eps, max_grad_norm, info, n_params,
@@ -978,15 +942,8 @@ int mr_adam_step_ex(float* params, float* exp_avg, float* exp_avg_sq, const floa
     return MR_OK;
 }
 
-int mr_adam_step(float* params, float* exp_avg, float* exp_avg_sq, const float* grad, int n_params,
-                 int64_t* step, float lr, float beta1, float beta2, float eps, float max_grad_norm,
-                 float* info, void* stream) {
-    return mr_adam_step_ex(params, exp_avg, exp_avg_sq, grad, n_params, step, lr, beta1, beta2, eps, max_grad_norm,
-                           info, 0.f, nullptr, 0, stream);
-}
-
-int mr_ppo_train_summary_ex(const float* info, int n_rows, const float* values, const float* returns, int64_t n,
-                            const float* params, float* out, double* scratch, const int* ctrl, void* stream) {
+int mr_ppo_train_summary(const float* info, int n_rows, const float* values, const float* returns, int64_t n,
+                         const float* params, float* out, double* scratch, const int* ctrl, void* stream) {
     MR_REQUIRE(info && values && returns && params && out && scratch, "NULL argument");
     MR_REQUIRE(n_rows > 0 && n > 0, "empty summary");
     const int grid = (int)std::min<int64_t>(sm_count(), (n + 255) / 256);
@@ -996,46 +953,29 @@ int mr_ppo_train_summary_ex(const float* info, int n_rows, const float* values, 
     return MR_OK;
 }
 
-int mr_ppo_train_summary(const float* info, int n_rows, const float* values, const float* returns, int64_t n,
-                         const float* params, float* out, double* scratch, void* stream) {
-    return mr_ppo_train_summary_ex(info, n_rows, values, returns, n, params, out, scratch, nullptr, stream);
-}
-
-int mr_ppo_train_epoch_ex(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
-                          const float* obs, const float* act, const float* old_logp, const float* adv,
-                          const float* ret, const int64_t* perm, int32_t* rows, int64_t n_samples,
-                          int64_t batch_size, const double* stats, int64_t N, int64_t T, float clip_range,
-                          float ent_coef, float vf_coef, int normalize_adv, float lr, float beta1, float beta2,
-                          float eps, float max_grad_norm, float* partials, float* grad, float* info,
-                          const float* old_values, float clip_range_vf, float target_kl, int* ctrl, int64_t mb0,
-                          void* stream) {
+int mr_ppo_train_epoch(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
+                       const float* obs, const float* act, const float* old_logp, const float* adv,
+                       const float* ret, const int64_t* perm, int32_t* rows, int64_t n_samples,
+                       int64_t batch_size, const double* stats, int64_t N, int64_t T, float clip_range,
+                       float ent_coef, float vf_coef, int normalize_adv, float lr, float beta1, float beta2,
+                       float eps, float max_grad_norm, float* partials, float* grad, float* info,
+                       const float* old_values, float clip_range_vf, float target_kl, int* ctrl, int64_t mb0,
+                       void* stream) {
     MR_REQUIRE(batch_size > 0 && n_samples > 0, "empty batch");
     const int n_params = make_layout(obs_dim).total;
     const int64_t n_mb = (n_samples + batch_size - 1) / batch_size;
     for (int64_t mb = 0; mb < n_mb; ++mb) {
         const int64_t s0 = mb * batch_size;
         const int64_t sz = std::min(batch_size, n_samples - s0);
-        int rc = mr_ppo_grad_ex(params, obs_dim, obs, act, old_logp, adv, ret, perm + s0, rows, sz, stats + 3 * mb,
-                                N, T, clip_range, ent_coef, vf_coef, normalize_adv, 1.0f, partials, grad, old_values,
-                                clip_range_vf, ctrl, stream);
+        int rc = mr_ppo_grad(params, obs_dim, obs, act, old_logp, adv, ret, perm + s0, rows, sz, stats + 3 * mb, N, T,
+                             clip_range, ent_coef, vf_coef, normalize_adv, 1.0f, partials, grad, old_values,
+                             clip_range_vf, ctrl, stream);
         if (rc != MR_OK) return rc;
-        rc = mr_adam_step_ex(params, exp_avg, exp_avg_sq, grad, n_params, step, lr, beta1, beta2, eps,
-                             max_grad_norm, info ? info + 8 * mb : nullptr, target_kl, ctrl, mb0 + mb, stream);
+        rc = mr_adam_step(params, exp_avg, exp_avg_sq, grad, n_params, step, lr, beta1, beta2, eps,
+                          max_grad_norm, info ? info + 8 * mb : nullptr, target_kl, ctrl, mb0 + mb, stream);
         if (rc != MR_OK) return rc;
     }
     return MR_OK;
-}
-
-int mr_ppo_train_epoch(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
-                       const float* obs, const float* act, const float* old_logp, const float* adv,
-                       const float* ret, const int64_t* perm, int32_t* rows, int64_t n_samples,
-                       int64_t batch_size, const double* stats, int64_t N, int64_t T, float clip_range,
-                       float ent_coef, float vf_coef, int normalize_adv, float lr, float beta1, float beta2,
-                       float eps, float max_grad_norm, float* partials, float* grad, float* info, void* stream) {
-    return mr_ppo_train_epoch_ex(params, exp_avg, exp_avg_sq, step, obs_dim, obs, act, old_logp, adv, ret, perm, rows,
-                                 n_samples, batch_size, stats, N, T, clip_range, ent_coef, vf_coef, normalize_adv, lr,
-                                 beta1, beta2, eps, max_grad_norm, partials, grad, info, nullptr, 0.f, 0.f, nullptr, 0,
-                                 stream);
 }
 
 #ifdef MR_TRACE
@@ -1123,8 +1063,8 @@ void mr_xchg_destroy(mr_xchg* x) {
 
 int mr_ppo_record_floats(int obs_dim) { return (obs_dim + 1 <= 16 ? 16 : 32) + 8; }
 
-int mr_ppo_pack_samples_vf(int obs_dim, const float* obs, const float* act, const float* old_logp, const float* adv,
-                           const float* ret, const float* values, int64_t n_rows, float* rec, void* stream) {
+int mr_ppo_pack_samples(int obs_dim, const float* obs, const float* act, const float* old_logp, const float* adv,
+                        const float* ret, const float* values, int64_t n_rows, float* rec, void* stream) {
     MR_REQUIRE(obs && act && old_logp && adv && ret && rec, "NULL argument");
     MR_REQUIRE(obs_dim > 0 && obs_dim < MAX_OBS, "obs_dim out of range (1..31: the record's row of X is obs and the ones column)");
     MR_REQUIRE(n_rows > 0, "empty buffer");
@@ -1136,18 +1076,13 @@ int mr_ppo_pack_samples_vf(int obs_dim, const float* obs, const float* act, cons
     return MR_OK;
 }
 
-int mr_ppo_pack_samples(int obs_dim, const float* obs, const float* act, const float* old_logp, const float* adv,
-                        const float* ret, int64_t n_rows, float* rec, void* stream) {
-    return mr_ppo_pack_samples_vf(obs_dim, obs, act, old_logp, adv, ret, nullptr, n_rows, rec, stream);
-}
-
-int mr_ppo_epoch_fused_ex(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
-                          const float* rec, const int64_t* perm, int32_t* rows, int64_t n_samples,
-                          int64_t batch_size, const double* stats, int64_t N, int64_t T,
-                          float clip_range, float ent_coef, float vf_coef, int normalize_adv, float lr,
-                          float beta1, float beta2, float eps, float max_grad_norm, float* partials,
-                          float* grad, float* info, mr_xchg* xchg, float clip_range_vf, float target_kl, int* ctrl,
-                          int64_t mb0, void* stream) {
+int mr_ppo_epoch_fused(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
+                       const float* rec, const int64_t* perm, int32_t* rows, int64_t n_samples,
+                       int64_t batch_size, const double* stats, int64_t N, int64_t T,
+                       float clip_range, float ent_coef, float vf_coef, int normalize_adv, float lr,
+                       float beta1, float beta2, float eps, float max_grad_norm, float* partials,
+                       float* grad, float* info, mr_xchg* xchg, float clip_range_vf, float target_kl, int* ctrl,
+                       int64_t mb0, void* stream) {
     MR_REQUIRE(params && exp_avg && exp_avg_sq && step && rec && rows && stats && partials && grad,
                "NULL argument");   // perm may be NULL: rows then already hold the epoch's samples (mr_ppo_prepare_epochs)
     MR_REQUIRE(!(target_kl > 0.f) || ctrl, "target_kl needs a control word");
@@ -1178,7 +1113,7 @@ int mr_ppo_epoch_fused_ex(float* params, float* exp_avg, float* exp_avg_sq, int6
     E.barrier = reinterpret_cast<unsigned*>(partials + 4 * (size_t)acc_floats);
     MR_CUDA(cudaMemsetAsync(partials, 0, (4 * (size_t)acc_floats + 16) * sizeof(float), s));
     if (!ext) MR_CUDA(cudaMemsetAsync(grad, 0, (size_t)stride * sizeof(float), s));   // (ext: the kernel clears the pads)
-    E.G.clip_vf = clip_range_vf;   // the records carry old_value (mr_ppo_pack_samples_vf) when this is > 0
+    E.G.clip_vf = clip_range_vf;   // the records carry old_value (mr_ppo_pack_samples' values) when this is > 0
     E.target_kl = target_kl; E.ctrl = ctrl; E.mb0 = mb0;
     E.X.world = 1; E.X.rank = 0; E.X.inbox = nullptr; E.X.err = nullptr;
     E.seq0 = 0;
@@ -1214,17 +1149,6 @@ int mr_ppo_epoch_fused_ex(float* params, float* exp_avg, float* exp_avg_sq, int6
     MR_CUDA(cudaLaunchCooperativeKernel(fn, dim3(n_cta), dim3(tc::THREADS), args, smem, s));
     mr::count_launch();
     return MR_OK;
-}
-
-int mr_ppo_epoch_fused(float* params, float* exp_avg, float* exp_avg_sq, int64_t* step, int obs_dim,
-                       const float* rec, const int64_t* perm, int32_t* rows, int64_t n_samples,
-                       int64_t batch_size, const double* stats, int64_t N, int64_t T,
-                       float clip_range, float ent_coef, float vf_coef, int normalize_adv, float lr,
-                       float beta1, float beta2, float eps, float max_grad_norm, float* partials,
-                       float* grad, float* info, mr_xchg* xchg, void* stream) {
-    return mr_ppo_epoch_fused_ex(params, exp_avg, exp_avg_sq, step, obs_dim, rec, perm, rows, n_samples, batch_size,
-                                 stats, N, T, clip_range, ent_coef, vf_coef, normalize_adv, lr, beta1, beta2, eps,
-                                 max_grad_norm, partials, grad, info, xchg, 0.f, 0.f, nullptr, 0, stream);
 }
 
 }  // extern "C"

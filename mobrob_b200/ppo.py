@@ -8,12 +8,14 @@ Mirrors (same names, argument meaning, zip format):
   * ``.policy.state_dict() / load_state_dict()``           train.py:30-33
   * ``.predict(obs, deterministic=True)``                  examples/control.py:39
 One ``learn`` iteration = mr_rollout (T steps) -> mr_gae -> n_epochs x minibatches of
-(mr_ppo_grad [-> all-reduce] -> mr_adam_step).  Nothing here computes on the CPU except
-bookkeeping; there is no fallback path.
+(mr_ppo_grad [-> all-reduce] -> mr_adam_step), fused into mr_ppo_epoch_fused by default ->
+mr_ppo_train_summary; clip_range_vf / target_kl are the update calls' trailing arguments.
+Nothing here computes on the CPU except bookkeeping; there is no fallback path.
 """
 from __future__ import annotations
 
 import base64
+import ctypes
 import io
 import json
 import os
@@ -121,7 +123,7 @@ class PPO:
         self.normalize_advantage, self.ent_coef, self.vf_coef = normalize_advantage, ent_coef, vf_coef
         self.max_grad_norm, self.verbose, self.seed = max_grad_norm, verbose, seed
         self.tensorboard_log = tensorboard_log
-        # RolloutBuffer.get's index stream.  "device" (default): mr_device_permutation, a keyed Feistel
+        # RolloutBuffer.get's index stream.  "device" (default): mr_device_permutations, a keyed Feistel
         # bijection computed where the samples live -- nothing crosses PCIe.  "sb3": np.random.permutation
         # on the global MT19937, bit-for-bit SB3's stream, serial on the host (parity runs).  "pool": host
         # threads drawing streams keyed by (seed, iteration, epoch) one iteration ahead (permfeed.py).
@@ -346,7 +348,8 @@ class PPO:
         out = self._dperm
         d = _dist()
         key = ((d.get_rank() if d is not None else 0) << 48) ^ (self._train_count << 16) ^ epoch
-        _lib.check(self.lib.mr_device_permutation(int(self.seed or 0), key, n, out.data_ptr(), self._stream()))
+        _lib.check(self.lib.mr_device_permutations(int(self.seed or 0), (ctypes.c_uint64 * 1)(key), 1, n,
+                                                   out.data_ptr(), self._stream()))
         return out
 
     def _stream_ids(self):
@@ -434,18 +437,15 @@ class PPO:
         self._train_log = (log[:, 4:], log[:, :4])
         # logger inputs of this update (mr_ppo_train_summary), read one iteration later -- SB3 records
         # train/* inside train() and dumps them with the NEXT iteration's rollout statistics
+        # (target_kl: statistics over the minibatches evaluated before the stop)
+        _lib.check(self.lib.mr_ppo_train_summary(log.data_ptr(), rows, b["values"].data_ptr(), b["returns"].data_ptr(),
+                                                 n, up.params.data_ptr(), self._train_stats_buf.data_ptr(),
+                                                 self._sum_scratch.data_ptr(), up.ctrl_ptr(), self._stream()))
         if self.target_kl is None:
             self._n_updates += self.n_epochs
-            _lib.check(self.lib.mr_ppo_train_summary(log.data_ptr(), rows, b["values"].data_ptr(), b["returns"].data_ptr(),
-                                                     n, up.params.data_ptr(), self._train_stats_buf.data_ptr(),
-                                                     self._sum_scratch.data_ptr(), self._stream()))
         else:
-            # statistics over the minibatches evaluated before the stop; how many epochs were entered is read
-            # back without blocking (the control word and the stopping approx_kl, into pinned memory)
-            _lib.check(self.lib.mr_ppo_train_summary_ex(log.data_ptr(), rows, b["values"].data_ptr(),
-                                                        b["returns"].data_ptr(), n, up.params.data_ptr(),
-                                                        self._train_stats_buf.data_ptr(), self._sum_scratch.data_ptr(),
-                                                        up.ctrl.data_ptr(), self._stream()))
+            # how many epochs were entered is read back without blocking (the control word and the stopping
+            # approx_kl, into pinned memory)
             ctrl_h = torch.zeros(1, dtype=torch.int32).pin_memory()
             kl_h = torch.zeros(1, dtype=torch.float32).pin_memory()
             ctrl_h.copy_(up.ctrl, non_blocking=True)

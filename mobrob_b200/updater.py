@@ -4,9 +4,10 @@ Owns the flat parameter vector, the Adam moments and the gradient scratch as tor
 tensors (so ``state_dict`` views, NCCL all-reduce and checkpointing need no extra copies).
 Mirrors what [SB3] PPO.train does per minibatch; see include/mobrob_b200.h.
 
-clip_range_vf / target_kl (None = off, the default) select the *_ex entry points; without them every call is the
-one it always was.  With target_kl the update's control word (``self.ctrl``, one int32 on the device) records an
-early stop; ``begin_update()`` clears it and must be called before the first launch of every update.
+clip_range_vf / target_kl (None = off, the default) go to the entry points as their trailing arguments (0 / NULL
+when off, which launches the default kernels).  With target_kl the update's control word (``self.ctrl``, one int32 on
+the device) records an early stop; ``begin_update()`` clears it and must be called before the first launch of every
+update.  The control word is passed only when target_kl is set, so the default path never runs the extended kernels.
 """
 from __future__ import annotations
 
@@ -48,20 +49,14 @@ class PpoUpdater:
         # target_kl: k > 0 once the update stopped after its k-th minibatch (caller-owned, like the barrier word)
         self.ctrl = torch.zeros(1, dtype=torch.int32, device=device)
 
-    @property
-    def extended(self) -> bool:
-        """True when clip_range_vf or target_kl is on: the update goes through the *_ex entry points."""
-        return self.clip_range_vf is not None or self.target_kl is not None
-
-    def _ext_args(self):
-        """(clip_range_vf, target_kl, control word) as the *_ex entry points take them (0 / NULL = off)."""
-        return (float(self.clip_range_vf or 0.0), float(self.target_kl or 0.0),
-                self.ctrl.data_ptr() if self.target_kl is not None else None)
-
     def begin_update(self):
         """Clear the control word (target_kl): once per update, before its first launch."""
         if self.target_kl is not None:
             self.ctrl.zero_()
+
+    def ctrl_ptr(self):
+        """The control word as the entry points take it: only with target_kl (NULL otherwise)."""
+        return self.ctrl.data_ptr() if self.target_kl is not None else None
 
     def rows(self, n: int) -> torch.Tensor:
         """int32 scratch for the samples as buffer rows (owned here, not by the library)."""
@@ -83,66 +78,29 @@ class PpoUpdater:
     def compute_grad(self, buf: dict, perm_slice: torch.Tensor, mb_stats: torch.Tensor, N: int, T: int,
                      rank_share: float = 1.0):
         """buf: time-major rollout tensors obs/actions/log_probs/advantages/returns (+ values with clip_range_vf)."""
-        if self.extended:
-            cvf, _, ctrl = self._ext_args()
-            _lib.check(self.lib.mr_ppo_grad_ex(
-                self.params.data_ptr(), self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(),
-                buf["log_probs"].data_ptr(), buf["advantages"].data_ptr(), buf["returns"].data_ptr(),
-                perm_slice.data_ptr(), self.rows(perm_slice.numel()).data_ptr(), perm_slice.numel(),
-                mb_stats.data_ptr(), N, T, self.clip_range, self.ent_coef, self.vf_coef,
-                int(self.normalize_advantage), rank_share, self.partials.data_ptr(), self.grad.data_ptr(),
-                buf["values"].data_ptr() if cvf > 0 else None, cvf, ctrl, self._stream()))
-            return self.grad
+        cvf = float(self.clip_range_vf or 0.0)
         _lib.check(self.lib.mr_ppo_grad(
             self.params.data_ptr(), self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(),
             buf["log_probs"].data_ptr(), buf["advantages"].data_ptr(), buf["returns"].data_ptr(),
             perm_slice.data_ptr(), self.rows(perm_slice.numel()).data_ptr(), perm_slice.numel(),
             mb_stats.data_ptr(), N, T, self.clip_range, self.ent_coef, self.vf_coef,
             int(self.normalize_advantage), rank_share, self.partials.data_ptr(), self.grad.data_ptr(),
-            self._stream()))
+            buf["values"].data_ptr() if cvf > 0 else None, cvf, self.ctrl_ptr(), self._stream()))
         return self.grad
-
-    def compute_partials(self, buf: dict, perm_slice: torch.Tensor, mb_stats: torch.Tensor, N: int, T: int):
-        """Forward/backward kernel only (per-CTA partial gradients) -- used for kernel timing."""
-        _lib.check(self.lib.mr_ppo_grad_partials(
-            self.params.data_ptr(), self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(),
-            buf["log_probs"].data_ptr(), buf["advantages"].data_ptr(), buf["returns"].data_ptr(),
-            perm_slice.data_ptr(), self.rows(perm_slice.numel()).data_ptr(), perm_slice.numel(),
-            mb_stats.data_ptr(), N, T, self.clip_range, self.ent_coef, self.vf_coef,
-            int(self.normalize_advantage), self.partials.data_ptr(), None, self._stream()))
 
     def adam_step(self, info: torch.Tensor | None = None, mb_index: int = 0):
         """mb_index: this minibatch's index in the update (what an early stop records)."""
-        if self.extended:
-            _, tkl, ctrl = self._ext_args()
-            _lib.check(self.lib.mr_adam_step_ex(
-                self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(),
-                self.grad.data_ptr(), self.n_params, self.step.data_ptr(), self.lr, self.betas[0],
-                self.betas[1], self.eps, self.max_grad_norm, None if info is None else info.data_ptr(), tkl, ctrl,
-                mb_index, self._stream()))
-            return
         _lib.check(self.lib.mr_adam_step(
             self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(),
             self.grad.data_ptr(), self.n_params, self.step.data_ptr(), self.lr, self.betas[0],
             self.betas[1], self.eps, self.max_grad_norm, None if info is None else info.data_ptr(),
-            self._stream()))
+            float(self.target_kl or 0.0), self.ctrl_ptr(), mb_index, self._stream()))
 
     def train_epoch(self, buf: dict, perm: torch.Tensor, stats: torch.Tensor, batch_size: int, N: int, T: int,
                     info: torch.Tensor | None = None, mb0: int = 0):
         """All minibatches of one epoch, launched from C (single-GPU path).  mb0: index of the epoch's first
         minibatch in the update (target_kl)."""
-        if self.extended:
-            cvf, tkl, ctrl = self._ext_args()
-            _lib.check(self.lib.mr_ppo_train_epoch_ex(
-                self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), self.step.data_ptr(),
-                self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(), buf["log_probs"].data_ptr(),
-                buf["advantages"].data_ptr(), buf["returns"].data_ptr(), perm.data_ptr(),
-                self.rows(min(perm.numel(), batch_size)).data_ptr(), perm.numel(), batch_size,
-                stats.data_ptr(), N, T, self.clip_range, self.ent_coef, self.vf_coef, int(self.normalize_advantage),
-                self.lr, self.betas[0], self.betas[1], self.eps, self.max_grad_norm, self.partials.data_ptr(),
-                self.grad.data_ptr(), None if info is None else info.data_ptr(),
-                buf["values"].data_ptr() if cvf > 0 else None, cvf, tkl, ctrl, mb0, self._stream()))
-            return
+        cvf = float(self.clip_range_vf or 0.0)
         _lib.check(self.lib.mr_ppo_train_epoch(
             self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), self.step.data_ptr(),
             self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(), buf["log_probs"].data_ptr(),
@@ -150,25 +108,23 @@ class PpoUpdater:
             self.rows(min(perm.numel(), batch_size)).data_ptr(), perm.numel(), batch_size,
             stats.data_ptr(), N, T, self.clip_range, self.ent_coef, self.vf_coef, int(self.normalize_advantage),
             self.lr, self.betas[0], self.betas[1], self.eps, self.max_grad_norm, self.partials.data_ptr(),
-            self.grad.data_ptr(), None if info is None else info.data_ptr(), self._stream()))
+            self.grad.data_ptr(), None if info is None else info.data_ptr(),
+            buf["values"].data_ptr() if cvf > 0 else None, cvf, float(self.target_kl or 0.0), self.ctrl_ptr(), mb0,
+            self._stream()))
 
     def pack(self, buf: dict) -> torch.Tensor:
         """Packed sample records of a rollout (mr_ppo_pack_samples): what train_epoch_fused gathers from.
         Build them once per rollout, after GAE; they stay valid for all epochs of the update.  With clip_range_vf
-        the records also carry buf["values"], the rollout's V(s) (mr_ppo_pack_samples_vf)."""
+        the records also carry buf["values"], the rollout's V(s)."""
         n_rows = buf["log_probs"].numel()
         rf = int(self.lib.mr_ppo_record_floats(self.obs_dim))
         if getattr(self, "_rec", None) is None or self._rec.numel() != n_rows * rf:
             self._rec = torch.empty(n_rows * rf, dtype=torch.float32, device=self.device)
-        if self.clip_range_vf is not None:
-            _lib.check(self.lib.mr_ppo_pack_samples_vf(
-                self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(), buf["log_probs"].data_ptr(),
-                buf["advantages"].data_ptr(), buf["returns"].data_ptr(), buf["values"].data_ptr(), n_rows,
-                self._rec.data_ptr(), self._stream()))
-            return self._rec
+        values = buf["values"].data_ptr() if self.clip_range_vf is not None else None
         _lib.check(self.lib.mr_ppo_pack_samples(
             self.obs_dim, buf["obs"].data_ptr(), buf["actions"].data_ptr(), buf["log_probs"].data_ptr(),
-            buf["advantages"].data_ptr(), buf["returns"].data_ptr(), n_rows, self._rec.data_ptr(), self._stream()))
+            buf["advantages"].data_ptr(), buf["returns"].data_ptr(), values, n_rows, self._rec.data_ptr(),
+            self._stream()))
         return self._rec
 
     def prepare_epochs(self, adv: torch.Tensor, perms: torch.Tensor, batch_size: int, N: int, T: int):
@@ -206,18 +162,6 @@ class PpoUpdater:
         mb0: index of the launch's first minibatch in the update (target_kl)."""
         rec = self.pack(buf) if buf is not None else self._rec
         n = perm.numel() if perm is not None else rows.numel()
-        if self.extended:
-            cvf, tkl, ctrl = self._ext_args()
-            _lib.check(self.lib.mr_ppo_epoch_fused_ex(
-                self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), self.step.data_ptr(),
-                self.obs_dim, rec.data_ptr(), None if perm is None else perm.data_ptr(),
-                self.rows(n).data_ptr() if rows is None else rows.data_ptr(), n,
-                batch_size, stats.data_ptr(), N, T, self.clip_range,
-                self.ent_coef, self.vf_coef, int(self.normalize_advantage), self.lr, self.betas[0], self.betas[1],
-                self.eps, self.max_grad_norm, self.partials.data_ptr(), self.grad.data_ptr(),
-                None if info is None else info.data_ptr(), None if xchg is None else xchg.handle, cvf, tkl, ctrl, mb0,
-                self._stream()))
-            return
         _lib.check(self.lib.mr_ppo_epoch_fused(
             self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), self.step.data_ptr(),
             self.obs_dim, rec.data_ptr(), None if perm is None else perm.data_ptr(),
@@ -225,7 +169,8 @@ class PpoUpdater:
             batch_size, stats.data_ptr(), N, T, self.clip_range,
             self.ent_coef, self.vf_coef, int(self.normalize_advantage), self.lr, self.betas[0], self.betas[1],
             self.eps, self.max_grad_norm, self.partials.data_ptr(), self.grad.data_ptr(),
-            None if info is None else info.data_ptr(), None if xchg is None else xchg.handle, self._stream()))
+            None if info is None else info.data_ptr(), None if xchg is None else xchg.handle,
+            float(self.clip_range_vf or 0.0), float(self.target_kl or 0.0), self.ctrl_ptr(), mb0, self._stream()))
 
 
 class PeerExchange:

@@ -1,4 +1,4 @@
-// Host harness for tests/test_device_perm_host_cpu.py: the keyed Feistel bijection of mr_device_permutation
+// Host harness for tests/test_device_perm_host_cpu.py: the keyed Feistel bijection of mr_device_permutations
 // (mobrob_b200/csrc/perm.cuh, the functions device_perm_kernel / device_rows_kernel call) evaluated on the CPU.
 //   argv: seed stream n out.bin   ->   int64 perm[n]
 #include <stdlib.h>

@@ -1,4 +1,4 @@
-"""numpy restatement of mr_device_permutation (mobrob_b200/csrc/ppo.cu: 6-round Feistel network on the
+"""numpy restatement of mr_device_permutations (mobrob_b200/csrc/ppo.cu: 6-round Feistel network on the
 enclosing power-of-two domain, cycle-walked into [0, n)) -- integer work, so the CUDA kernel must match
 it bit for bit.  This is the repo's own algorithm (the reference draws np.random.permutation on the
 host; PPO(permutation="sb3") keeps that stream), restated only for the test."""

@@ -1,4 +1,6 @@
-"""mr_device_permutation: the keyed on-device index stream used by PPO(permutation="device")."""
+"""mr_device_permutations: the keyed on-device index stream used by PPO(permutation="device")."""
+import ctypes
+
 import numpy as np
 import pytest
 import torch
@@ -11,8 +13,9 @@ pytestmark = pytest.mark.gpu
 
 def _perm(seed, stream, n):
     out = torch.full((n,), -1, dtype=torch.int64, device="cuda")
-    _lib.check(_lib.load().mr_device_permutation(seed, stream, n, out.data_ptr(),
-                                                 torch.cuda.current_stream().cuda_stream))
+    key = (ctypes.c_uint64 * 1)(stream)
+    _lib.check(_lib.load().mr_device_permutations(seed, key, 1, n, out.data_ptr(),
+                                                  torch.cuda.current_stream().cuda_stream))
     return out.cpu().numpy()
 
 
@@ -81,8 +84,6 @@ def test_prepare_epochs_device_equals_the_two_step_form(cuda_lib):
     """mr_ppo_prepare_epochs_device (index streams generated on the fly) == mr_device_permutations followed by
     mr_ppo_prepare_epochs: same buffer rows bit for bit, same per-minibatch advantage sums; and the rows are
     what numpy makes of the restated permutation."""
-    import ctypes
-
     from mobrob_b200.updater import PpoUpdater
 
     N, T, B, E, seed = 37, 64, 300, 3, 11

@@ -1,4 +1,4 @@
-"""mr_device_permutation's keyed bijection (mobrob_b200/csrc/perm.cuh), compiled for the HOST, against its numpy
+"""mr_device_permutations' keyed bijection (mobrob_b200/csrc/perm.cuh), compiled for the HOST, against its numpy
 restatement (tests/perm_ref.py): integer work, bit for bit, no GPU needed.  The statistical quality of the stream is
 tested on the device output (tests/test_device_perm_gpu.py); this holds the arithmetic."""
 import os

@@ -65,7 +65,8 @@ def test_obs_dim_32_is_refused(cuda_lib):
     x = torch.zeros(64, device="cuda")
     with pytest.raises(_lib.MobrobError, match="1..31"):
         _lib.check(cuda_lib.mr_ppo_pack_samples(32, x.data_ptr(), x.data_ptr(), x.data_ptr(), x.data_ptr(),
-                                                x.data_ptr(), 1, x.data_ptr(), torch.cuda.current_stream().cuda_stream))
+                                                x.data_ptr(), None, 1, x.data_ptr(),
+                                                torch.cuda.current_stream().cuda_stream))
 
 
 def _assert_grad_matches(pol, gp, g_ref, g_64):
