@@ -58,14 +58,22 @@ int mr_env_obs_dim(const mr_env* env);   /* point 14, car 26 (engine.py:420-567)
 /* Optional keys of Engine.obs() (config flags engine.py:125,140-142; values engine.py:1179-1180, 1243-1248; the
  * reference sets them through MujocoGoalEnv.get_robot_config, wrapper.py:235-240): bit 0 observe_goal_dist
  * (exp(-|goal - pos|), 1 float), bit 1 observe_qpos (data.qpos: point 3, car 13), bit 2 observe_qvel (data.qvel:
- * point 3, car 11), bit 3 observe_ctrl (data.ctrl, 2).  The row stays the concatenation in sorted key order
- * (engine.py:1253-1259).  Call before the first reset; rows of obs / term_obs then have mr_env_obs_dim floats.
- * MR_ERR_UNSUPPORTED for other bits (lidar, vision, hazards are outside the path). */
+ * point 3, car 11), bit 3 observe_ctrl (data.ctrl, 2), bit 4 observe_goal_lidar (the pseudo-lidar of the goal,
+ * engine.py:1092-1172: lidar_num_bins floats, see mr_env_set_lidar).  The row stays the concatenation in sorted key
+ * order (engine.py:1253-1259).  Call before the first reset; rows of obs / term_obs then have mr_env_obs_dim floats.
+ * MR_ERR_UNSUPPORTED for other bits (the natural lidar, object lidars, vision and hazards are outside the path). */
 #define MR_OBS_GOAL_DIST 1u
 #define MR_OBS_QPOS 2u
 #define MR_OBS_QVEL 4u
 #define MR_OBS_CTRL 8u
+#define MR_OBS_GOAL_LIDAR 16u
 int mr_env_set_obs_flags(mr_env* env, unsigned flags);
+/* Engine's pseudo-lidar settings for MR_OBS_GOAL_LIDAR (config keys lidar_num_bins, lidar_max_dist, lidar_exp_gain,
+ * lidar_alias; lidar_type 'pseudo'): num_bins >= 1 (else MR_ERR_ARG); max_dist <= 0 means None (sensor =
+ * exp(-exp_gain * dist)), otherwise sensor = max(0, max_dist - dist) / max_dist; alias != 0 spreads each reading over
+ * the two neighbouring bins.  Defaults: 10 bins, None, 1.0, alias on.  Call before the first reset, like
+ * mr_env_set_obs_flags. */
+int mr_env_set_lidar(mr_env* env, int num_bins, double max_dist, double exp_gain, int alias);
 int mr_env_state_dim(const mr_env* env); /* doubles per env in get/set_state */
 
 /* Test hook (car): 0 disables the floor contacts, giving the contact-free trajectories on which

@@ -25,6 +25,7 @@ _SIGNATURES = {
     "mr_env_state_dim": (c_int, [_P]),
     "mr_env_set_contacts": (c_int, [_P, c_int]),
     "mr_env_set_obs_flags": (c_int, [_P, ctypes.c_uint]),
+    "mr_env_set_lidar": (c_int, [_P, c_int, c_double, c_double, c_int]),
     "mr_env_set_spaces": (c_int, [_P, _P, _P, _P]),
     "mr_env_seed": (c_int, [_P, _P, _P, _P, _P]),
     "mr_env_reset": (c_int, [_P, _P, c_int, _P, _P]),

@@ -105,34 +105,37 @@ point_step_ext_kernel(PointState st, EnvCfg cfg, const float2* __restrict__ act,
                       float* __restrict__ term_obs, double* __restrict__ ep_ret, int32_t* __restrict__ ep_len) {
     const int64_t i = (int64_t)blockIdx.x * STEP_THREADS + threadIdx.x;
     if (i >= st.n) return;
-    const int O = obs_dim_ext(point::OBS, 3, 3, cfg.obs_flags);
+    const int O = obs_dim_ext(point::OBS, 3, 3, cfg.obs_flags, cfg.lidar.num_bins);
     PointHot h = st.load_step(i);
     const float2 a = act[i];
     float o[point::OBS], tobs[point::OBS];
     PointExt x, tx;
     StepResult r = point_env_step(h, st.cold, i, a.x, a.y, cfg, o, tobs, &x, &tx);
     st.store_step(i, h, r.done);
-    emit_obs_row<point::OBS, POINT_OBS_PRE, 3, 3>(obs + i * O, o, x, cfg.obs_flags);
+    emit_obs_row<point::OBS, POINT_OBS_PRE, 3, 3>(obs + i * O, o, x, cfg.obs_flags, cfg.lidar);
     rew[i] = r.rew;
     done[i] = r.done ? 1 : 0;
     trunc[i] = r.trunc ? 1 : 0;
     if (r.done) {
-        if (term_obs) emit_obs_row<point::OBS, POINT_OBS_PRE, 3, 3>(term_obs + i * O, tobs, tx, cfg.obs_flags);
+        if (term_obs) emit_obs_row<point::OBS, POINT_OBS_PRE, 3, 3>(term_obs + i * O, tobs, tx, cfg.obs_flags, cfg.lidar);
         if (ep_ret) ep_ret[i] = r.ep_r;
         if (ep_len) ep_len[i] = r.ep_l;
     }
 }
 
 __device__ __forceinline__ void point_obs_row_ext(const PointState& st, const PointHot& h, int64_t i, const float (&o)[point::OBS],
-                                                  unsigned flags, float* __restrict__ obs) {
+                                                  const EnvCfg& cfg, float* __restrict__ obs) {
     PointExt x;
-    point_obs_ext(h, st.cold, i, x);
-    emit_obs_row<point::OBS, POINT_OBS_PRE, 3, 3>(obs + i * obs_dim_ext(point::OBS, 3, 3, flags), o, x, flags);
+    double s, c;
+    sincos(h.d.psi, &s, &c);
+    point_obs_ext(h, st.cold, i, c, s, x);
+    emit_obs_row<point::OBS, POINT_OBS_PRE, 3, 3>(obs + i * obs_dim_ext(point::OBS, 3, 3, cfg.obs_flags, cfg.lidar.num_bins),
+                                                  o, x, cfg.obs_flags, cfg.lidar);
 }
 
 __global__ void __launch_bounds__(STEP_THREADS)
 point_reset_kernel(PointState st, const uint8_t* __restrict__ mask, int first,
-                   float* __restrict__ obs, unsigned flags) {
+                   float* __restrict__ obs, EnvCfg cfg) {
     const int64_t i = (int64_t)blockIdx.x * STEP_THREADS + threadIdx.x;
     if (i >= st.n) return;
     if (mask && !mask[i]) return;
@@ -143,20 +146,20 @@ point_reset_kernel(PointState st, const uint8_t* __restrict__ mask, int first,
     if (obs) {
         float o[point::OBS];
         point::sensors(h.d, (double)h.cx, (double)h.cz, h.gx, h.gy, o);
-        if (flags) { point_obs_row_ext(st, h, i, o, flags, obs); return; }
+        if (cfg.obs_flags) { point_obs_row_ext(st, h, i, o, cfg, obs); return; }
 #pragma unroll
         for (int k = 0; k < point::OBS; ++k) obs[i * point::OBS + k] = o[k];
     }
 }
 
 __global__ void __launch_bounds__(STEP_THREADS)
-point_obs_ext_kernel(PointState st, float* __restrict__ obs, unsigned flags) {
+point_obs_ext_kernel(PointState st, float* __restrict__ obs, EnvCfg cfg) {
     const int64_t i = (int64_t)blockIdx.x * STEP_THREADS + threadIdx.x;
     if (i >= st.n) return;
     PointHot h = st.load(i);
     float o[point::OBS];
     point::sensors(h.d, (double)h.cx, (double)h.cz, h.gx, h.gy, o);
-    point_obs_row_ext(st, h, i, o, flags, obs);
+    point_obs_row_ext(st, h, i, o, cfg, obs);
 }
 
 __global__ void __launch_bounds__(STEP_THREADS)
@@ -265,30 +268,31 @@ car_step_ext_kernel(CarSoA st, car::Consts K, EnvCfg cfg, const float2* __restri
     MR_CAR_SCRATCH();
     const int64_t i = (int64_t)blockIdx.x * CAR_THREADS + threadIdx.x;
     if (i >= st.n) return;
-    const int O = obs_dim_ext(car::OBS, 13, 11, cfg.obs_flags);
+    const int O = obs_dim_ext(car::OBS, 13, 11, cfg.obs_flags, cfg.lidar.num_bins);
     CarHot h = st.load(i);
     float2 a = act[i];
     float o[car::OBS], tobs[car::OBS];
     CarExt x, tx;
     StepResult r = car_env_step(K, h, st.cold, i, a.x, a.y, cfg, st.contacts != 0, o, tobs, S, &x, &tx);
     st.store(i, h);
-    emit_obs_row<car::OBS, CAR_OBS_PRE, 13, 11>(obs + i * O, o, x, cfg.obs_flags);
+    emit_obs_row<car::OBS, CAR_OBS_PRE, 13, 11>(obs + i * O, o, x, cfg.obs_flags, cfg.lidar);
     rew[i] = r.rew;
     done[i] = r.done ? 1 : 0;
     trunc[i] = r.trunc ? 1 : 0;
     if (r.done) {
-        if (term_obs) emit_obs_row<car::OBS, CAR_OBS_PRE, 13, 11>(term_obs + i * O, tobs, tx, cfg.obs_flags);
+        if (term_obs) emit_obs_row<car::OBS, CAR_OBS_PRE, 13, 11>(term_obs + i * O, tobs, tx, cfg.obs_flags, cfg.lidar);
         if (ep_ret) ep_ret[i] = r.ep_r;
         if (ep_len) ep_len[i] = r.ep_l;
     }
 }
 
-__device__ __forceinline__ void car_obs_row(const CarHot& h, int64_t i, const float (&o)[car::OBS], unsigned flags,
+__device__ __forceinline__ void car_obs_row(const CarHot& h, int64_t i, const float (&o)[car::OBS], const EnvCfg& cfg,
                                             float* __restrict__ obs) {
-    if (flags) {
+    if (cfg.obs_flags) {
         CarExt x;
         car_obs_ext(h, x);
-        emit_obs_row<car::OBS, CAR_OBS_PRE, 13, 11>(obs + i * obs_dim_ext(car::OBS, 13, 11, flags), o, x, flags);
+        emit_obs_row<car::OBS, CAR_OBS_PRE, 13, 11>(obs + i * obs_dim_ext(car::OBS, 13, 11, cfg.obs_flags, cfg.lidar.num_bins),
+                                                    o, x, cfg.obs_flags, cfg.lidar);
     } else {
         for (int k = 0; k < car::OBS; ++k) obs[i * car::OBS + k] = o[k];
     }
@@ -296,7 +300,7 @@ __device__ __forceinline__ void car_obs_row(const CarHot& h, int64_t i, const fl
 
 __global__ void __launch_bounds__(CAR_THREADS)
 car_reset_kernel(CarSoA st, car::Consts K, const uint8_t* __restrict__ mask, int first, float* __restrict__ obs,
-                 unsigned flags) {
+                 EnvCfg cfg) {
     MR_CAR_SCRATCH();
     const int64_t i = (int64_t)blockIdx.x * CAR_THREADS + threadIdx.x;
     if (i >= st.n) return;
@@ -308,19 +312,19 @@ car_reset_kernel(CarSoA st, car::Consts K, const uint8_t* __restrict__ mask, int
     if (obs) {
         float o[car::OBS];
         car::sensors(K, h.s, (double)h.cx, (double)h.cz, h.gx, h.gy, st.contacts != 0, o, S);
-        car_obs_row(h, i, o, flags, obs);
+        car_obs_row(h, i, o, cfg, obs);
     }
 }
 
 __global__ void __launch_bounds__(CAR_THREADS)
-car_obs_kernel(CarSoA st, car::Consts K, float* __restrict__ obs, unsigned flags) {
+car_obs_kernel(CarSoA st, car::Consts K, float* __restrict__ obs, EnvCfg cfg) {
     MR_CAR_SCRATCH();
     const int64_t i = (int64_t)blockIdx.x * CAR_THREADS + threadIdx.x;
     if (i >= st.n) return;
     CarHot h = st.load(i);
     float o[car::OBS];
     car::sensors(K, h.s, (double)h.cx, (double)h.cz, h.gx, h.gy, st.contacts != 0, o, S);
-    car_obs_row(h, i, o, flags, obs);
+    car_obs_row(h, i, o, cfg, obs);
 }
 
 // reference view: qpos(13) = p quat thL thR qb ; qvel(11) = v w sL sR wb ; ctrl goal elapsed ep_ret
@@ -412,6 +416,7 @@ int mr_env_create(int kind, int64_t n_envs, int device, int time_limit, int term
     e->cfg.terminate_on_goal = terminate_on_goal ? 1 : 0;
     e->cfg.pk = point::make_k();
     e->cfg.obs_flags = 0;
+    e->cfg.lidar = make_lidar_cfg(10, 0.0, 1.0, 1);   // Safety Gym's defaults: 10 bins, max_dist None, exp_gain 1, alias
     size_t bytes = kind == MR_ENV_POINT ? PointState::slab_bytes(n_envs) : CarSoA::slab_bytes(n_envs);
     cudaError_t err = cudaMalloc(&e->slab, bytes);
     if (err != cudaSuccess) {
@@ -468,14 +473,16 @@ void mr_env_destroy(mr_env* env) {
 
 int mr_env_obs_dim(const mr_env* env) {
     if (!env) return 0;
-    return env->kind == MR_ENV_POINT ? obs_dim_ext(point::OBS, 3, 3, env->cfg.obs_flags)
-                                     : obs_dim_ext(car::OBS, 13, 11, env->cfg.obs_flags);
+    const int bins = env->cfg.lidar.num_bins;
+    return env->kind == MR_ENV_POINT ? obs_dim_ext(point::OBS, 3, 3, env->cfg.obs_flags, bins)
+                                     : obs_dim_ext(car::OBS, 13, 11, env->cfg.obs_flags, bins);
 }
 
 int mr_env_set_obs_flags(mr_env* env, unsigned flags) {
     MR_REQUIRE(env, "env is NULL");
     if (flags & ~OBS_ALL_FLAGS) {
-        set_error("unknown observation flag bits 0x%x (1 goal_dist, 2 qpos, 4 qvel, 8 ctrl)", flags & ~OBS_ALL_FLAGS);
+        set_error("unknown observation flag bits 0x%x (1 goal_dist, 2 qpos, 4 qvel, 8 ctrl, 16 goal_lidar)",
+                  flags & ~OBS_ALL_FLAGS);
         return MR_ERR_UNSUPPORTED;
     }
     if (env->scratch && flags != env->cfg.obs_flags) {   // mr_rollout_unfused sized its scratch for the old row length
@@ -485,6 +492,19 @@ int mr_env_set_obs_flags(mr_env* env, unsigned flags) {
         env->scratch = nullptr;
     }
     env->cfg.obs_flags = flags;
+    return MR_OK;
+}
+
+int mr_env_set_lidar(mr_env* env, int num_bins, double max_dist, double exp_gain, int alias) {
+    MR_REQUIRE(env, "env is NULL");
+    MR_REQUIRE(num_bins >= 1, "lidar_num_bins must be at least 1");
+    if (env->scratch && num_bins != env->cfg.lidar.num_bins && (env->cfg.obs_flags & OBS_GOAL_LIDAR)) {
+        DeviceGuard guard(env->device);   // as in mr_env_set_obs_flags: the rollout scratch has the old row length
+        MR_CUDA(cudaDeviceSynchronize());
+        MR_CUDA(cudaFree(env->scratch));
+        env->scratch = nullptr;
+    }
+    env->cfg.lidar = make_lidar_cfg(num_bins, max_dist, exp_gain, alias);
     return MR_OK;
 }
 int mr_env_state_dim(const mr_env* env) {
@@ -516,11 +536,11 @@ int mr_env_reset(mr_env* env, const uint8_t* mask, int first, float* obs_out, vo
     cudaStream_t s = (cudaStream_t)stream;
     if (env->kind == MR_ENV_POINT)
         point_reset_kernel<<<ceil_div(env->n, STEP_THREADS), STEP_THREADS, 0, s>>>(env->point, mask, first, obs_out,
-                                                                                   env->cfg.obs_flags);
+                                                                                   env->cfg);
     else {
         if (car_smem_optin() != MR_OK) return MR_ERR_CUDA;
         car_reset_kernel<<<ceil_div(env->n, CAR_THREADS), CAR_THREADS, CAR_SMEM, s>>>(env->car, env->carK, mask, first, obs_out,
-                                                                                      env->cfg.obs_flags);
+                                                                                      env->cfg);
     }
     MR_CHECK_LAUNCH();
     return MR_OK;
@@ -569,13 +589,13 @@ int mr_env_get_obs(mr_env* env, float* obs_out, void* stream) {
     cudaStream_t s = (cudaStream_t)stream;
     if (env->kind == MR_ENV_POINT) {
         if (env->cfg.obs_flags)
-            point_obs_ext_kernel<<<ceil_div(env->n, STEP_THREADS), STEP_THREADS, 0, s>>>(env->point, obs_out, env->cfg.obs_flags);
+            point_obs_ext_kernel<<<ceil_div(env->n, STEP_THREADS), STEP_THREADS, 0, s>>>(env->point, obs_out, env->cfg);
         else
             point_obs_kernel<<<ceil_div(env->n, STEP_THREADS), STEP_THREADS, 0, s>>>(env->point, obs_out);
     } else {
         if (car_smem_optin() != MR_OK) return MR_ERR_CUDA;
         car_obs_kernel<<<ceil_div(env->n, CAR_THREADS), CAR_THREADS, CAR_SMEM, s>>>(env->car, env->carK, obs_out,
-                                                                                    env->cfg.obs_flags);
+                                                                                    env->cfg);
     }
     MR_CHECK_LAUNCH();
     return MR_OK;

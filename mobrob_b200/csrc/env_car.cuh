@@ -109,9 +109,17 @@ constexpr int CAR_OBS_PRE = 15;
 
 // data.qpos = free joint (pos, quat) + wheel angles + rear ball quat; data.qvel = free joint (linear world, angular
 // body) + wheel rates + ball angular velocity: the order of mr_env_get_state's reference view.
+// The lidar drops the goal's height (engine.py ego_xy): R^T (goal_x - p_x, goal_y - p_y, -p_z), not goal_compass's
+// vector to the goal body at GOAL_Z -- the two differ once the chassis tilts.
 __host__ __device__ inline void car_obs_ext(const CarHot& h, CarExt& x) {
     const car::State& s = h.s;
     x.ctrl[0] = h.cx; x.ctrl[1] = h.cz;
+    double R[9], e[3];
+    car::quat2mat(s.q, R);
+    const double dv[3] = {(double)h.gx - s.p[0], (double)h.gy - s.p[1], -s.p[2]};
+    car::mat3tv(R, dv, e);
+    x.lidar_x = e[0];
+    x.lidar_y = e[1];
     x.goal_dist = (float)exp(-point::dist2((double)h.gx, (double)h.gy, s.p[0], s.p[1]));
 #pragma unroll
     for (int k = 0; k < 3; ++k) { x.qpos[k] = (float)s.p[k]; x.qvel[k] = (float)s.v[k]; x.qvel[3 + k] = (float)s.w[k]; x.qvel[8 + k] = (float)s.wb[k]; }

@@ -128,7 +128,8 @@ class MujocoGoalEnv(EnvWrapper, ABC):
 
     def get_robot_config(self) -> dict:
         """Engine config of the robot (wrapper.py:235-240, 293-317).  A subclass may switch on observe_goal_dist /
-        observe_qpos / observe_qvel / observe_ctrl (engine.py:125, 140-142); other observation keys are fixed."""
+        observe_qpos / observe_qvel / observe_ctrl (engine.py:125, 140-142) and observe_goal_lidar with its
+        lidar_num_bins / lidar_max_dist / lidar_exp_gain / lidar_alias settings; other observation keys are fixed."""
         return {"robot_base": f"xmls/{self.ENV_NAME}.xml", "sensors_obs": self.BASE_SENSORS,
                 "observe_com": False, "observe_goal_comp": True}
 

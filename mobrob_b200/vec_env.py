@@ -20,8 +20,8 @@ ENV_KINDS = {"point": 0, "car": 1}
 OBS_DIMS = {"point": 14, "car": 26}
 # Engine config keys (engine.py:124-144) the batched env implements -> mr_env_set_obs_flags bits; every other
 # observe_* key must keep the value the reference's get_robot_config leaves it at
-OBS_FLAG_BITS = {"observe_goal_dist": 1, "observe_qpos": 2, "observe_qvel": 4, "observe_ctrl": 8}
-_FIXED_OBSERVE = {"observe_sensors": True, "observe_goal_comp": True, "observe_com": False, "observe_goal_lidar": False,
+OBS_FLAG_BITS = {"observe_goal_dist": 1, "observe_qpos": 2, "observe_qvel": 4, "observe_ctrl": 8, "observe_goal_lidar": 16}
+_FIXED_OBSERVE = {"observe_sensors": True, "observe_goal_comp": True, "observe_com": False,
                   "observe_box_comp": False, "observe_box_lidar": False, "observe_circle": False,
                   "observe_remaining": False, "observe_walls": False, "observe_hazards": False, "observe_vases": False,
                   "observe_pillars": False, "observe_buttons": False, "observe_gremlins": False,
@@ -38,6 +38,29 @@ def obs_flags_of(robot_config: dict | None) -> int:
         elif key in _FIXED_OBSERVE and bool(value) != _FIXED_OBSERVE[key]:
             raise NotImplementedError(f"{key}={value!r}: only {sorted(OBS_FLAG_BITS)} can be switched on the B200 path")
     return flags
+
+
+# Safety Gym's Engine.DEFAULT pseudo-lidar settings (parity unpinned: restated, the reference's source is not at hand)
+LIDAR_DEFAULTS = {"lidar_num_bins": 10, "lidar_max_dist": None, "lidar_exp_gain": 1.0, "lidar_alias": True,
+                  "lidar_type": "pseudo"}
+
+
+def lidar_of(robot_config: dict | None) -> tuple[int, float | None, float, bool]:
+    """Engine(config) lidar keys -> (num_bins, max_dist, exp_gain, alias) for observe_goal_lidar, defaults filled in.
+    Only the pseudo-lidar exists here: lidar_type 'natural' ray-casts against the model's geoms."""
+    cfg = {**LIDAR_DEFAULTS, **{k: v for k, v in (robot_config or {}).items() if k in LIDAR_DEFAULTS}}
+    if cfg["lidar_type"] == "natural":
+        raise NotImplementedError("lidar_type='natural' (ray-cast lidar) is not available on the B200 path; use 'pseudo'")
+    if cfg["lidar_type"] != "pseudo":
+        raise ValueError(f"lidar_type={cfg['lidar_type']!r}: must be 'pseudo' or 'natural'")
+    bins = cfg["lidar_num_bins"]
+    if isinstance(bins, bool) or not isinstance(bins, (int, np.integer)) or bins < 1:
+        raise ValueError(f"lidar_num_bins={bins!r}: must be an integer >= 1")
+    max_dist = cfg["lidar_max_dist"]
+    if max_dist is not None and not float(max_dist) > 0:
+        raise ValueError(f"lidar_max_dist={max_dist!r}: must be None or positive")
+    return (int(bins), None if max_dist is None else float(max_dist), float(cfg["lidar_exp_gain"]),
+            bool(cfg["lidar_alias"]))
 
 
 class GpuVecEnv:
@@ -66,6 +89,11 @@ class GpuVecEnv:
         self.obs_flags = obs_flags_of(robot_config)
         if self.obs_flags:
             _lib.check(self.lib.mr_env_set_obs_flags(h, self.obs_flags))
+        # the lidar keys are read only with observe_goal_lidar on (the Engine ignores them otherwise)
+        self.lidar = lidar_of(robot_config) if self.obs_flags & OBS_FLAG_BITS["observe_goal_lidar"] else None
+        if self.lidar:
+            bins, max_dist, gain, alias = self.lidar
+            _lib.check(self.lib.mr_env_set_lidar(h, bins, max_dist or 0.0, gain, int(alias)))
         self.obs_dim = int(self.lib.mr_env_obs_dim(h))
         self.state_dim = int(self.lib.mr_env_state_dim(h))
         self.observation_space = Box(-np.inf, np.inf, (self.obs_dim,), np.float32)
