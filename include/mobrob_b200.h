@@ -112,6 +112,14 @@ int mr_env_step(mr_env* env, const float* act, float* obs, float* rew, uint8_t* 
 
 /* EnvWrapper.get_obs (wrapper.py:272-273 -> Engine.obs, engine.py:1174-1263). */
 int mr_env_get_obs(mr_env* env, float* obs_out, void* stream);
+/* EnvWrapper.set_goal (wrapper.py:115-117) for the masked envs, then their get_obs() rows.
+ *   mask [N] u8 on the device, NULL = every env; goals [N][2] f32 on the device (rows of unmasked envs unread)
+ *   obs_out [N][obs_dim] f32, may be NULL: the masked envs' rows are written with the new goal and everything else as
+ *        it was, the ctrl of the last step included (a goal-only reset's row); the other rows are left alone
+ * Only the goal changes: no reset count, elapsed step or episode return moves, and the next step's reward is paid from
+ * the position before it, as reward_fn's _prev_pos.  Valid between steps and after a reset, for both robots and every
+ * observation row. */
+int mr_env_set_goals(mr_env* env, const uint8_t* mask, const float* goals, float* obs_out, void* stream);
 /* Reference-view state, [N][state_dim] float64.
  * point (15): qpos(3) qvel(3) body_pos_xy(2) start_heading(1) ctrl(2) goal_xy(2) elapsed(1) ep_ret(1)
  * car (30):   qpos(13) qvel(11) ctrl(2) goal_xy(2) elapsed(1) ep_ret(1), MuJoCo joint order */
@@ -332,6 +340,30 @@ int mr_ppo_prepare_epochs_device(uint64_t seed, const uint64_t* h_stream_ids, in
 int mr_evaluate(mr_env* env, const float* params, int deterministic, int64_t n_episodes, int64_t max_steps,
                 uint64_t seed, uint64_t noise_offset, int64_t env_offset, float* last_obs, double* ep_r,
                 int32_t* ep_l, int64_t* ep_t, int64_t* steps_taken, int* status, void* stream);
+
+/* Waypoint following: for each env i independently, from its current state, the loop a planner runs with
+ * EnvWrapper.set_goal / model.predict / env.step / reached() over waypoints W[i][0..K-1]:
+ *     set_goal(W[i][0]); obs = get_obs(); k = t = 0
+ *     while k < K and t < max_steps:
+ *         step with the policy's action on obs; t += 1; ret += reward
+ *         if reached():  arrival[i][k] = t; k += 1; if k < K: set_goal(W[i][k]); obs = get_obs()
+ * An env whose loop has ended takes no further step: its state stays where its own loop left it.
+ *   deterministic, seed, noise_offset, env_offset: the actions of mr_evaluate (Philox keyed (seed; env_offset + n,
+ *        noise_offset + t), t = step index within this call)
+ *   waypoints [N][K][2] f32 world xy; K >= 1; max_steps >= 1 (mandatory, as in mr_evaluate)
+ *   last_obs [N][obs_dim] f32 out: the observation each env's loop ended on
+ *   arrival [N][K] i32 out: the step (1-based) at which waypoint k was reached, -1 if it was not
+ *   ret [N] f64 out: the sum of the env's float64 rewards (reward_fn, reach bonus included)
+ *   steps_taken [N] i32 out: steps the env took; the call used max_i steps_taken[i] Philox counters
+ *   positions [max_steps + 1][N][2] f32 out or NULL: row t = the world xy after step t (row 0: the start); rows past an
+ *        env's end repeat its final position
+ * The env must have been created with terminate_on_goal = 0 and no time limit (MR_ERR_ARG otherwise): its
+ * auto-reset would draw a random goal.  The point env with the default observation row runs in one fused launch; the
+ * car and envs with optional observation keys take two launches per step (forward, then a masked env step) and read
+ * a device count of finished envs every 16 steps to stop early. */
+int mr_follow_waypoints(mr_env* env, const float* params, int deterministic, const float* waypoints, int K,
+                        int64_t max_steps, uint64_t seed, uint64_t noise_offset, int64_t env_offset, float* last_obs,
+                        int32_t* arrival, double* ret, int32_t* steps_taken, float* positions, void* stream);
 
 /* Host-side minibatch index stream (no device work): out[0..n) <- a uniformly random permutation
  * of 0..n-1, a pure function of (seed, stream).  Replaces, for throughput runs, the

@@ -31,6 +31,7 @@ _SIGNATURES = {
     "mr_env_reset": (c_int, [_P, _P, c_int, _P, _P]),
     "mr_env_step": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "mr_env_get_obs": (c_int, [_P, _P, _P]),
+    "mr_env_set_goals": (c_int, [_P, _P, _P, _P, _P]),
     "mr_env_get_state": (c_int, [_P, _P, _P]),
     "mr_env_set_state": (c_int, [_P, _P, _P]),
     "mr_env_get_pos": (c_int, [_P, _P, _P]),
@@ -63,6 +64,8 @@ _SIGNATURES = {
                                    c_uint64, c_int64, c_double, _P, _P, _P, _P, _P, _P, c_int, _P]),
     "mr_evaluate": (c_int, [_P, _P, c_int, c_int64, c_int64, c_uint64, c_uint64, c_int64, _P, _P, _P, _P, _P, _P,
                             _P]),
+    "mr_follow_waypoints": (c_int, [_P, _P, c_int, _P, c_int, c_int64, c_uint64, c_uint64, c_int64, _P, _P, _P, _P,
+                                    _P, _P]),
     "mr_device_permutations": (c_int, [c_uint64, _P, c_int, c_int64, _P, _P]),
     "mr_ppo_prepare_epochs": (c_int, [_P, _P, c_int, c_int64, c_int64, c_int64, c_int64, _P, _P, _P]),
     "mr_ppo_prepare_epochs_device": (c_int, [c_uint64, _P, c_int, _P, c_int64, c_int64, c_int64, c_int64, _P, _P, _P]),

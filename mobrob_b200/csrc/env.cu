@@ -229,11 +229,7 @@ __global__ void point_get_pos_kernel(PointState st, double* __restrict__ out) {
 
 // ---------------------------------------------------------------------------------------
 // car: same VecEnv kernels, one thread per env (state in fp64 registers; the contact solver's Delassus matrix
-// in shared memory, car::SCRATCH_DOUBLES per thread)
-constexpr int CAR_THREADS = 64;
-constexpr size_t CAR_SMEM = (size_t)car::SCRATCH_DOUBLES * sizeof(double) * CAR_THREADS;   // 112.5 KB: two CTAs per SM
-#define MR_CAR_SCRATCH() extern __shared__ __align__(16) double car_smem[]; \
-    const car::Scratch S{(uint32_t)__cvta_generic_to_shared(car_smem + threadIdx.x), (uint32_t)(CAR_THREADS * sizeof(double))}
+// in shared memory, car::SCRATCH_DOUBLES per thread; CAR_THREADS, CAR_SMEM, MR_CAR_SCRATCH in env_state.cuh)
 
 __global__ void __launch_bounds__(CAR_THREADS)
 car_step_kernel(CarSoA st, car::Consts K, EnvCfg cfg, const float2* __restrict__ act,
@@ -599,6 +595,11 @@ int mr_env_get_obs(mr_env* env, float* obs_out, void* stream) {
     }
     MR_CHECK_LAUNCH();
     return MR_OK;
+}
+
+int mr_env_set_goals(mr_env* env, const uint8_t* mask, const float* goals, float* obs_out, void* stream) {
+    MR_REQUIRE(env && goals, "NULL argument");
+    return env_set_goals(env, mask, goals, 2, obs_out, (cudaStream_t)stream);
 }
 
 int mr_env_get_state(mr_env* env, double* state_out, void* stream) {

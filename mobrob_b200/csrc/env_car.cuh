@@ -151,6 +151,7 @@ __host__ __device__ inline StepResult car_env_step(const car::Consts& K, CarHot&
     r.done = term || tl;
     r.trunc = tl && !term;
     h.ep_ret = rn::add(h.ep_ret, reward);
+    r.reward = reward;
     r.rew = (float)reward;
     r.ep_r = h.ep_ret;
     r.ep_l = h.elapsed;

@@ -149,6 +149,7 @@ struct PointHot {
 struct StepResult {
     float rew;
     bool done, trunc, reach;
+    double reward;   // rew before the float32 rounding (mr_follow_waypoints sums these)
     double ep_r;
     int ep_l;
 };
@@ -247,6 +248,7 @@ __host__ __device__ inline StepResult point_env_step(PointHot& h, const EnvCold&
     r.done = term || tl;
     r.trunc = tl && !term;
     h.ep_ret = rn::add(h.ep_ret, reward);
+    r.reward = reward;
     r.rew = (float)reward;
     r.ep_r = h.ep_ret;
     r.ep_l = h.elapsed;

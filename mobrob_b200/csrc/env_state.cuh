@@ -133,3 +133,36 @@ struct mr_env {
     void* scratch = nullptr;  // lazily allocated by mr_rollout_unfused
     int step_flip = 0;        // env-step kernels alternate the block order (L2 keeps the tail of the last step)
 };
+
+namespace mr {
+
+// car env kernels (env.cu, waypoints.cu): one thread per env, the contact solver's scratch in shared memory
+constexpr int CAR_THREADS = 64;
+constexpr size_t CAR_SMEM = (size_t)car::SCRATCH_DOUBLES * sizeof(double) * CAR_THREADS;   // 112.5 KB: two CTAs per SM
+#define MR_CAR_SCRATCH() extern __shared__ __align__(16) double car_smem[]; \
+    const car::Scratch S{(uint32_t)__cvta_generic_to_shared(car_smem + threadIdx.x), (uint32_t)(CAR_THREADS * sizeof(double))}
+
+// EnvWrapper.set_goal for the masked envs (mask NULL: all): env i's goal <- goals[i * goal_stride + 0..1]; obs (may be
+// NULL) receives the masked envs' get_obs() rows.  mr_env_set_goals and mr_follow_waypoints' first waypoint.
+int env_set_goals(mr_env* env, const uint8_t* mask, const float* goals, int64_t goal_stride, float* obs,
+                  cudaStream_t s);
+
+// mr_follow_waypoints' per-step path: the per-env loop state, advanced by env_step_waypoints (waypoints.cu)
+struct WaypointStep {
+    const float* wp;                 // [N][K][2]
+    int K;
+    int64_t max_steps;
+    int64_t t;                       // step index of this launch (0-based)
+    int32_t* cursor;                 // [N] next waypoint; K once the last one is reached
+    int32_t* steps;                  // [N] steps the env has taken
+    double* ret;                     // [N] sum of the rewards
+    int32_t* arrival;                // [N][K]
+    float* pos;                      // [max_steps + 1][N][2] or NULL
+    unsigned long long* n_finished;  // envs whose loop has ended
+};
+
+// one step of the envs whose loop is still running (the others are not touched): env step with act, the step's
+// arrival / return bookkeeping, the next waypoint's goal and get_obs() row for envs that just reached one
+int env_step_waypoints(mr_env* env, const float* act, float* obs, const WaypointStep& w, cudaStream_t s);
+
+}  // namespace mr

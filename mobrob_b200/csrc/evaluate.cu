@@ -213,6 +213,120 @@ __global__ void __launch_bounds__(ES_WARPS * 32) eval_step_kernel(EvalStepArgs A
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Waypoint following (mr_follow_waypoints).  Fused path for the point's default row: point_eval_kernel's structure,
+// each env with its own waypoint cursor and its own end; a warp ends when its envs have ended.
+struct WaypointArgs {
+    PointState st;
+    EnvCfg cfg;
+    const float* params;
+    int O, K;
+    int64_t N, max_steps;
+    int stochastic;
+    const float* wp;       // [N][K][2]
+    float* last_obs;       // [N][O] out
+    int32_t* arrival;      // [N][K] out (pre-filled with -1)
+    double* ret;           // [N] out
+    int32_t* steps;        // [N] out
+    float2* pos;           // [max_steps + 1][N] out, or NULL
+    uint64_t seed, noise_offset;
+    int64_t env_offset;
+};
+
+template <int W_, int E_>
+__global__ void __launch_bounds__(W_ * 32) point_waypoint_kernel(WaypointArgs A) {
+    extern __shared__ __align__(16) float smem[];
+    const int O = A.O;
+    SmemW W = stage_weights(smem, A.params, O);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    float* obsT = smem + smem_w_floats(O) + warp * (MAX_OBS * E_ + 128 * E_);
+    float* hbuf = obsT + MAX_OBS * E_;
+    __syncthreads();
+
+    const int64_t n0 = ((int64_t)blockIdx.x * W_ + warp) * E_;
+    if (n0 >= A.N) return;
+    const int n_live = (int)min((int64_t)E_, A.N - n0);
+    const bool phys = lane < n_live;
+    const int64_t n = n0 + lane;
+    const float sig0 = expf(W.logstd[0]), sig1 = expf(W.logstd[1]);
+
+    // set_goal(W[n, 0]); obs = get_obs()
+    PointHot h;
+    int k = 0, my_t = 0;
+    double ret = 0.0;
+    bool running = phys;
+    if (phys) {
+        h = A.st.load(n);
+        h.gx = A.wp[n * A.K * 2];
+        h.gy = A.wp[n * A.K * 2 + 1];
+        float o[point::OBS];
+        point::sensors(h.d, (double)h.cx, (double)h.cz, h.gx, h.gy, o);
+#pragma unroll
+        for (int j = 0; j < point::OBS; ++j) obsT[j * E_ + lane] = o[j];
+        if (A.pos) A.pos[n] = make_float2((float)h.d.px, (float)h.d.py);
+    } else if (lane < E_) {
+        for (int j = 0; j < O; ++j) obsT[j * E_ + lane] = 0.f;
+    }
+    __syncwarp();
+
+    const int e_of = lane / 3, j_of = lane - 3 * e_of;
+    const int src = 3 * (lane % E_);
+    int64_t t = 0;
+    for (; t < A.max_steps; ++t) {
+        if (!__any_sync(0xffffffffu, running)) break;
+        const float out = warp_mlp_forward<E_>(W, O, obsT, hbuf, lane);
+        float a = out;
+        if (lane < 3 * E_ && e_of < n_live && j_of < 2)
+            a = eval_action(out, j_of == 0 ? sig0 : sig1, A.stochastic, A.seed, (uint64_t)(A.env_offset + n0 + e_of),
+                            A.noise_offset + (uint64_t)t, j_of);
+        const float a0 = __shfl_sync(0xffffffffu, a, src);
+        const float a1 = __shfl_sync(0xffffffffu, a, src + 1);
+        float o_new[point::OBS], o_term[point::OBS];
+        const bool stepped = running;
+        if (stepped) {
+            const StepResult r = point_env_step(h, A.st.cold, n, a0, a1, A.cfg, o_new, o_term);
+            my_t = (int)t + 1;
+            ret = rn::add(ret, r.reward);
+            if (r.reach) {
+                A.arrival[n * A.K + k] = my_t;
+                if (++k < A.K) {   // set_goal(W[n, k]); obs = get_obs()
+                    h.gx = A.wp[(n * A.K + k) * 2];
+                    h.gy = A.wp[(n * A.K + k) * 2 + 1];
+                    point::sensors(h.d, (double)h.cx, (double)h.cz, h.gx, h.gy, o_new);
+                }
+            }
+            running = k < A.K && my_t < A.max_steps;
+        }
+        if (phys && A.pos) A.pos[(t + 1) * A.N + n] = make_float2((float)h.d.px, (float)h.d.py);
+        __syncwarp();
+        if (stepped) {
+#pragma unroll
+            for (int j = 0; j < point::OBS; ++j) obsT[j * E_ + lane] = o_new[j];
+        }
+        __syncwarp();
+    }
+
+    if (phys) {
+        if (A.pos)   // rows past the warp's end repeat the final position
+            for (int64_t r = t + 1; r <= A.max_steps; ++r) A.pos[r * A.N + n] = make_float2((float)h.d.px, (float)h.d.py);
+        A.st.store(n, h);
+        A.ret[n] = ret;
+        A.steps[n] = my_t;
+    }
+    for (int idx = lane; idx < n_live * O; idx += 32) {
+        const int e = idx / O, j = idx - e * O;
+        A.last_obs[n0 * O + idx] = obsT[j * E_ + e];
+    }
+}
+
+// per-step path: positions rows from_row .. max_steps repeat row from_row - 1
+__global__ void fill_positions_kernel(float2* pos, int64_t N, int64_t from_row, int64_t max_steps) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    const float2 p = pos[(from_row - 1) * N + i];
+    for (int64_t r = from_row; r <= max_steps; ++r) pos[r * N + i] = p;
+}
+
 }  // namespace mr
 
 using namespace mr;
@@ -329,4 +443,111 @@ extern "C" int mr_evaluate(mr_env* env, const float* params, int deterministic, 
         return eval_fused(env, A, s);
     }
     return eval_per_step(env, A, s);
+}
+
+// Per-step path (the car, point envs with optional keys): per step, eval_step_kernel (forward + sample for every env,
+// with no episode to record) then the masked env step, which leaves envs whose loop has ended untouched and does the
+// waypoint bookkeeping itself -- it is the kernel that holds the car's contact scratch, which the post-switch get_obs()
+// row needs.  The loop reads the device count of finished envs every WP_POLL steps: each read synchronises the stream,
+// which costs about as much as a step of a few thousand envs, while a late stop costs at most WP_POLL - 1 pairs of
+// launches whose threads all return at once.
+constexpr int64_t WP_POLL = 16;
+
+static int waypoints_per_step(mr_env* env, const float* params, int stochastic, const float* wp, int K,
+                              int64_t max_steps, uint64_t seed, uint64_t noise_offset, int64_t env_offset,
+                              float* last_obs, int32_t* arrival, double* ret, int32_t* steps, float* pos,
+                              cudaStream_t s) {
+    const int64_t N = env->n;
+    const int O = mr_env_obs_dim(env);
+    char* scratch = nullptr;
+    size_t off = 0;
+    auto carve = [&](size_t bytes) { const size_t at = off; off += (bytes + 255) & ~size_t(255); return at; };
+    const size_t o_act = carve(N * 8), o_cur = carve(N * 4), o_done = carve(N), o_fin = carve(8);
+    MR_CUDA(cudaMallocAsync((void**)&scratch, off, s));
+    MR_CUDA(cudaMemsetAsync(scratch + o_cur, 0, off - o_cur, s));   // cursors, eval_step_kernel's done flags, count
+
+    const size_t smem = (smem_w_floats(O) + ES_WARPS * (MAX_OBS * ES_E + 128 * ES_E)) * sizeof(float);
+    static OncePerDevice once;
+    if (once.first())
+        MR_CUDA(cudaFuncSetAttribute(mr::eval_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+    const int64_t tiles = (N + ES_E - 1) / ES_E;
+    const int blocks = (int)std::min<int64_t>((tiles + ES_WARPS - 1) / ES_WARPS, (int64_t)sm_count() * 2);
+    EvalStepArgs A{};
+    A.params = params; A.O = O; A.N = N; A.E = 0; A.stochastic = stochastic;
+    A.obs = last_obs; A.act = (float*)(scratch + o_act);
+    A.done = (const uint8_t*)(scratch + o_done);   // all zero: no episode ever ends (no reset, no time limit)
+    A.seed = seed; A.noise_offset = noise_offset; A.env_offset = env_offset;
+
+    WaypointStep w;
+    w.wp = wp; w.K = K; w.max_steps = max_steps;
+    w.cursor = (int32_t*)(scratch + o_cur); w.steps = steps; w.ret = ret; w.arrival = arrival; w.pos = pos;
+    w.n_finished = (unsigned long long*)(scratch + o_fin);
+
+    int rc = env_set_goals(env, nullptr, wp, 2 * (int64_t)K, last_obs, s);
+    unsigned long long finished = 0;
+    int64_t t = 0;
+    for (; rc == MR_OK && t < max_steps; ++t) {
+        A.t = t;
+        mr::eval_step_kernel<<<blocks, ES_WARPS * 32, smem, s>>>(A);
+        count_launch();
+        w.t = t;
+        rc = env_step_waypoints(env, A.act, last_obs, w, s);
+        if (rc == MR_OK && (t + 1) % WP_POLL == 0) {
+            cudaError_t e = cudaMemcpyAsync(&finished, w.n_finished, 8, cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+            if (e != cudaSuccess) {
+                set_error("waypoint step %lld: %s", (long long)t, cudaGetErrorString(e));
+                rc = MR_ERR_CUDA;
+            } else if (finished >= (unsigned long long)N) {
+                ++t;
+                break;
+            }
+        }
+    }
+    if (rc == MR_OK && pos && t < max_steps) {   // rows 0 .. t are written
+        fill_positions_kernel<<<ceil_div(N, 128), 128, 0, s>>>(reinterpret_cast<float2*>(pos), N, t + 1, max_steps);
+        count_launch();
+    }
+    cudaFreeAsync(scratch, s);
+    if (rc != MR_OK) return rc;
+    MR_CHECK_LAUNCH();
+    return MR_OK;
+}
+
+extern "C" int mr_follow_waypoints(mr_env* env, const float* params, int deterministic, const float* waypoints,
+                                   int K, int64_t max_steps, uint64_t seed, uint64_t noise_offset, int64_t env_offset,
+                                   float* last_obs, int32_t* arrival, double* ret, int32_t* steps_taken,
+                                   float* positions, void* stream) {
+    MR_REQUIRE(env && params && waypoints && last_obs && arrival && ret && steps_taken, "NULL argument");
+    MR_REQUIRE(K >= 1, "K must be at least 1");
+    MR_REQUIRE(max_steps >= 1 && max_steps <= INT32_MAX, "max_steps must be in 1 .. 2^31 - 1");
+    MR_REQUIRE(!env->cfg.terminate_on_goal && env->cfg.time_limit <= 0,
+               "mr_follow_waypoints needs an env created with terminate_on_goal = 0 and no time limit (its "
+               "auto-reset would draw a random goal)");
+    const int O = mr_env_obs_dim(env);
+    MR_REQUIRE(O <= MAX_OBS, "the policy kernels take observations of at most 32 floats");
+    cudaStream_t s = (cudaStream_t)stream;
+    DeviceGuard guard(env->device);
+    const int64_t N = env->n;
+    MR_CUDA(cudaMemsetAsync(arrival, 0xff, (size_t)N * K * sizeof(int32_t), s));   // -1: not reached
+    MR_CUDA(cudaMemsetAsync(ret, 0, (size_t)N * sizeof(double), s));
+    MR_CUDA(cudaMemsetAsync(steps_taken, 0, (size_t)N * sizeof(int32_t), s));
+    const int stochastic = deterministic ? 0 : 1;
+    if (env->kind != MR_ENV_POINT || env->cfg.obs_flags != 0)
+        return waypoints_per_step(env, params, stochastic, waypoints, K, max_steps, seed, noise_offset, env_offset,
+                                  last_obs, arrival, ret, steps_taken, positions, s);
+    WaypointArgs A;
+    A.st = env->point; A.cfg = env->cfg; A.params = params; A.O = O; A.K = K; A.N = N; A.max_steps = max_steps;
+    A.stochastic = stochastic; A.wp = waypoints; A.last_obs = last_obs; A.arrival = arrival; A.ret = ret;
+    A.steps = steps_taken; A.pos = reinterpret_cast<float2*>(positions);
+    A.seed = seed; A.noise_offset = noise_offset; A.env_offset = env_offset;
+    const size_t smem = (smem_w_floats(O) + EV_WARPS * (MAX_OBS * EV_E + 128 * EV_E)) * sizeof(float);
+    static OncePerDevice once;
+    if (once.first())
+        MR_CUDA(cudaFuncSetAttribute(point_waypoint_kernel<EV_WARPS, EV_E>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     100 * 1024));
+    const int64_t warps = (N + EV_E - 1) / EV_E;
+    point_waypoint_kernel<EV_WARPS, EV_E><<<(int)((warps + EV_WARPS - 1) / EV_WARPS), EV_WARPS * 32, smem, s>>>(A);
+    MR_CHECK_LAUNCH();
+    return MR_OK;
 }

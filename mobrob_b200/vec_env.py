@@ -112,8 +112,8 @@ class GpuVecEnv:
         self._actions = None
         self._needs_first_reset = True
         self._seed = None
-        # VecEnv steps taken so far by evaluate_policy's device path: the Philox counter at which the next stochastic
-        # evaluation on this env starts, so that consecutive evaluations never reuse a draw
+        # VecEnv steps taken so far by evaluate_policy's device path and follow_waypoints: the Philox counter at which
+        # the next stochastic evaluation on this env starts, so that consecutive calls never reuse a draw
         self.eval_steps = 0
         self.t_start = time.time()
         if seed is not None:
@@ -216,6 +216,39 @@ class GpuVecEnv:
         """Later resets draw the goal from `goal_space` (a 2-d Box)."""
         self.goal_space = goal_space
         self._set_spaces()
+
+    # -- EnvWrapper.set_goal / get_goal (wrapper.py:115-123) for the batch ---------------------------------------------
+    def set_goals(self, goals, indices=None):
+        """Give env ``indices[j]`` (every env when None) the goal ``goals[j]`` (float32 xy), as EnvWrapper.set_goal does:
+        nothing else changes, and the next step's reward is paid from the position before it.  The env-owned ``obs``
+        tensor receives those envs' new ``get_obs()`` rows.  ``goals``: numpy (copied to the device) or a CUDA tensor
+        (used in place when it is a contiguous float32 [num_envs, 2] on this env's device)."""
+        n = self.num_envs
+        idx = None
+        if indices is not None:
+            idx = np.asarray(indices.cpu() if isinstance(indices, torch.Tensor) else list(indices), np.int64).reshape(-1)
+        rows = n if idx is None else len(idx)
+        if tuple(goals.shape) != (rows, 2):
+            raise ValueError(f"goals must have shape ({rows}, 2), got {tuple(goals.shape)}")
+        if idx is not None and len(idx) and (idx.min() < -n or idx.max() >= n):
+            raise IndexError(f"env index out of range for {n} envs")
+        g = torch.as_tensor(goals).to(device=self.device, dtype=torch.float32)
+        if idx is not None:
+            full = torch.zeros((n, 2), dtype=torch.float32, device=self.device)
+            mask = torch.zeros(n, dtype=torch.uint8, device=self.device)
+            dev_idx = torch.as_tensor(idx % n, device=self.device)
+            full[dev_idx] = g
+            mask[dev_idx] = 1
+            g = full
+        g = g.contiguous()
+        # temporaries are released to the caching allocator in stream order: no synchronisation needed
+        _lib.check(self.lib.mr_env_set_goals(self._h, None if idx is None else mask.data_ptr(), g.data_ptr(),
+                                             self.obs.data_ptr(), self._stream()))
+
+    def get_goals(self) -> torch.Tensor:
+        """[num_envs, 2] float32 on the device: each env's current goal (EnvWrapper.get_goal)."""
+        slot = 11 if self.env_name == "point" else 26   # goal_xy in the reference-view state
+        return self.get_state()[:, slot:slot + 2].to(torch.float32)
 
     def set_contacts(self, enabled: bool):
         """car only: switch the floor contacts off for contact-free parity trajectories."""
