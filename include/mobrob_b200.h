@@ -59,14 +59,17 @@ int mr_env_obs_dim(const mr_env* env);   /* point 14, car 26 (engine.py:420-567)
  * reference sets them through MujocoGoalEnv.get_robot_config, wrapper.py:235-240): bit 0 observe_goal_dist
  * (exp(-|goal - pos|), 1 float), bit 1 observe_qpos (data.qpos: point 3, car 13), bit 2 observe_qvel (data.qvel:
  * point 3, car 11), bit 3 observe_ctrl (data.ctrl, 2), bit 4 observe_goal_lidar (the pseudo-lidar of the goal,
- * engine.py:1092-1172: lidar_num_bins floats, see mr_env_set_lidar).  The row stays the concatenation in sorted key
- * order (engine.py:1253-1259).  Call before the first reset; rows of obs / term_obs then have mr_env_obs_dim floats.
- * MR_ERR_UNSUPPORTED for other bits (the natural lidar, object lidars, vision and hazards are outside the path). */
+ * engine.py:1092-1172: lidar_num_bins floats, see mr_env_set_lidar), bit 5 observe_hazards (the pseudo-lidar of the
+ * hazards, lidar_num_bins floats between gyro and magnetometer; only present when mr_env_set_hazards gave the env
+ * hazards).  The row stays the concatenation in sorted key order (engine.py:1253-1259).  Call before the first reset;
+ * rows of obs / term_obs then have mr_env_obs_dim floats.  MR_ERR_UNSUPPORTED for other bits (the natural lidar, the
+ * vase / pillar / gremlin lidars and vision are outside the path). */
 #define MR_OBS_GOAL_DIST 1u
 #define MR_OBS_QPOS 2u
 #define MR_OBS_QVEL 4u
 #define MR_OBS_CTRL 8u
 #define MR_OBS_GOAL_LIDAR 16u
+#define MR_OBS_HAZARDS_LIDAR 32u
 int mr_env_set_obs_flags(mr_env* env, unsigned flags);
 /* Engine's pseudo-lidar settings for MR_OBS_GOAL_LIDAR (config keys lidar_num_bins, lidar_max_dist, lidar_exp_gain,
  * lidar_alias; lidar_type 'pseudo'): num_bins >= 1 (else MR_ERR_ARG); max_dist <= 0 means None (sensor =
@@ -74,6 +77,30 @@ int mr_env_set_obs_flags(mr_env* env, unsigned flags);
  * the two neighbouring bins.  Defaults: 10 bins, None, 1.0, alias on.  Call before the first reset, like
  * mr_env_set_obs_flags. */
 int mr_env_set_lidar(mr_env* env, int num_bins, double max_dist, double exp_gain, int alias);
+
+/* Safety Gym's hazards (Engine config keys hazards_num, hazards_size, hazards_keepout, hazards_cost,
+ * hazards_locations, constrain_hazards, constrain_indicator).  Hazards do not collide; they change three things:
+ *   - every full reset lays out robot, goal and the num hazards by the Engine's rejection sampling (build_layout) on
+ *     the device, and the start heading is the one drawn after that layout (set_pos / set_goal then move the robot and
+ *     the goal, not the hazards); a goal-only reset keeps the hazards;
+ *   - MR_OBS_HAZARDS_LIDAR adds their pseudo-lidar (the mr_env_set_lidar settings) to the row;
+ *   - with constrain != 0 each step's Engine.cost, sum over hazards within `size` of cost * (size - dist), or its
+ *     indicator (x > 0) with indicator != 0, is kept per env (mr_env_get_cost).
+ * locations: host [n_loc][2] float64, hazard i < n_loc is drawn from a box of side ~2e-9 around locations[i].
+ * MR_ERR_ARG for num outside 0 .. MR_MAX_HAZARDS, n_loc outside 0 .. num, a negative size or keepout, and (with
+ * constrain) size >= robot_keepout + placements_margin + keepout = 0.4 + keepout, where the Engine's reset asserts
+ * "World has starting cost!".  num = 0 removes the hazards.  Call before the first reset, like mr_env_set_lidar. */
+#define MR_MAX_HAZARDS 32
+int mr_env_set_hazards(mr_env* env, int num, double size, double keepout, double cost, int constrain, int indicator,
+                       const double* locations, int n_loc);
+/* hazard xy of every env, [N][num][2] float64 on the device (nothing is written without hazards) */
+int mr_env_get_hazards(mr_env* env, double* out, void* stream);
+/* info["cost"] of each env's last step, [N] float64 on the device: 0 before the first step and without
+ * constrain_hazards */
+int mr_env_get_cost(mr_env* env, double* out, void* stream);
+/* Synchronises the device and returns in *out the number of full resets that found no layout in 10 000 attempts
+ * (the Engine raises ResamplingError "Failed to sample layout of objects"); such an env keeps a partial layout. */
+int mr_env_layout_failures(mr_env* env, int64_t* out);
 int mr_env_state_dim(const mr_env* env); /* doubles per env in get/set_state */
 
 /* Test hook (car): 0 disables the floor contacts, giving the contact-free trajectories on which

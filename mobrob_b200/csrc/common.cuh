@@ -184,6 +184,38 @@ struct MtHead {
     }
 };
 
+// The same generator with its whole 624-word state, for any number of draws (hazard_layout).  Word k of each round is
+// twisted when it is drawn, from mt[k + 1] of the previous round and mt[k + 397] of whichever round wrote it last --
+// what the reference's block twist computes.  2.5 KB: local memory, for the full resets of hazard envs only.
+struct Mt19937 {
+    uint32_t mt[624];
+    int k;
+    __host__ __device__ explicit Mt19937(uint32_t seed) {
+        mt[0] = seed;
+        for (int j = 1; j < 624; ++j) mt[j] = 1812433253u * (mt[j - 1] ^ (mt[j - 1] >> 30)) + (uint32_t)j;
+        k = 0;
+    }
+    __host__ __device__ uint32_t next32() {
+        const int k1 = k + 1 == 624 ? 0 : k + 1, km = k < 227 ? k + 397 : k - 227;
+        const uint32_t y = (mt[k] & 0x80000000u) | (mt[k1] & 0x7fffffffu);
+        uint32_t v = mt[km] ^ (y >> 1) ^ ((y & 1u) ? 0x9908b0dfu : 0u);
+        mt[k] = v;
+        k = k1;
+        v ^= v >> 11;
+        v ^= (v << 7) & 0x9d2c5680u;
+        v ^= (v << 15) & 0xefc60000u;
+        v ^= v >> 18;
+        return v;
+    }
+    __host__ __device__ double next_double() {
+        uint32_t x = next32() >> 5, y = next32() >> 6;
+        return ((double)x * 67108864.0 + (double)y) / 9007199254740992.0;
+    }
+    __host__ __device__ double uniform(double low, double high) {
+        return rn::add(low, rn::mul(rn::sub(high, low), next_double()));
+    }
+};
+
 // Engine.reset -> build_layout -> build_world_config: the heading is the first uniform after
 // the robot xy pair and the accepted goal xy pair.
 __host__ __device__ inline double engine_heading(uint32_t engine_seed) {

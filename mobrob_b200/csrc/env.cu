@@ -97,42 +97,52 @@ point_step_kernel(PointState st, EnvCfg cfg, const float2* __restrict__ act,
     store_rows_coalesced(obs, s_obs, block_start, rows);
 }
 
-// Step with optional observation keys (EnvCfg::obs_flags != 0): same per-env logic, rows of obs_dim_ext floats
-// written row by row (this variant is not the measured hot path; the default configuration keeps the kernel above).
+// Step with optional observation keys (EnvCfg::obs_flags != 0) or hazards (HAZ, EnvCfg::haz.num > 0): same per-env
+// logic, rows of row_dim floats written row by row (this variant is not the measured hot path; the default
+// configuration keeps the kernel above).
+template <bool HAZ>
 __global__ void __launch_bounds__(STEP_THREADS)
 point_step_ext_kernel(PointState st, EnvCfg cfg, const float2* __restrict__ act, float* __restrict__ obs,
                       float* __restrict__ rew, uint8_t* __restrict__ done, uint8_t* __restrict__ trunc,
                       float* __restrict__ term_obs, double* __restrict__ ep_ret, int32_t* __restrict__ ep_len) {
     const int64_t i = (int64_t)blockIdx.x * STEP_THREADS + threadIdx.x;
     if (i >= st.n) return;
-    const int O = obs_dim_ext(point::OBS, 3, 3, cfg.obs_flags, cfg.lidar.num_bins);
+    const int O = row_dim<HAZ>(point::OBS, 3, 3, cfg);
     PointHot h = st.load_step(i);
     const float2 a = act[i];
     float o[point::OBS], tobs[point::OBS];
     PointExt x, tx;
-    StepResult r = point_env_step(h, st.cold, i, a.x, a.y, cfg, o, tobs, &x, &tx);
+    StepResult r = point_env_step<HAZ>(h, st.cold, i, a.x, a.y, cfg, o, tobs, &x, &tx,
+                                       hazards_block<HAZ, POINT_OBS_PRE>(obs + i * O, cfg),
+                                       hazards_block<HAZ, POINT_OBS_PRE>(term_obs ? term_obs + i * O : nullptr, cfg));
     st.store_step(i, h, r.done);
-    emit_obs_row<point::OBS, POINT_OBS_PRE, 3, 3>(obs + i * O, o, x, cfg.obs_flags, cfg.lidar);
+    emit_obs_row<point::OBS, POINT_OBS_PRE, 3, 3, HAZ>(obs + i * O, o, x, cfg.obs_flags, cfg.lidar);
     rew[i] = r.rew;
     done[i] = r.done ? 1 : 0;
     trunc[i] = r.trunc ? 1 : 0;
     if (r.done) {
-        if (term_obs) emit_obs_row<point::OBS, POINT_OBS_PRE, 3, 3>(term_obs + i * O, tobs, tx, cfg.obs_flags, cfg.lidar);
+        if (term_obs)
+            emit_obs_row<point::OBS, POINT_OBS_PRE, 3, 3, HAZ>(term_obs + i * O, tobs, tx, cfg.obs_flags, cfg.lidar);
         if (ep_ret) ep_ret[i] = r.ep_r;
         if (ep_len) ep_len[i] = r.ep_l;
     }
 }
 
+template <bool HAZ>
 __device__ __forceinline__ void point_obs_row_ext(const PointState& st, const PointHot& h, int64_t i, const float (&o)[point::OBS],
                                                   const EnvCfg& cfg, float* __restrict__ obs) {
     PointExt x;
     double s, c;
     sincos(h.d.psi, &s, &c);
     point_obs_ext(h, st.cold, i, c, s, x);
-    emit_obs_row<point::OBS, POINT_OBS_PRE, 3, 3>(obs + i * obs_dim_ext(point::OBS, 3, 3, cfg.obs_flags, cfg.lidar.num_bins),
-                                                  o, x, cfg.obs_flags, cfg.lidar);
+    float* row = obs + i * row_dim<HAZ>(point::OBS, 3, 3, cfg);
+    emit_obs_row<point::OBS, POINT_OBS_PRE, 3, 3, HAZ>(row, o, x, cfg.obs_flags, cfg.lidar);
+    if constexpr (HAZ) {
+        if (float* hb = hazards_block<HAZ, POINT_OBS_PRE>(row, cfg)) point_hazards_lidar(hb, h, cfg, i);
+    }
 }
 
+template <bool HAZ>
 __global__ void __launch_bounds__(STEP_THREADS)
 point_reset_kernel(PointState st, const uint8_t* __restrict__ mask, int first,
                    float* __restrict__ obs, EnvCfg cfg) {
@@ -141,17 +151,18 @@ point_reset_kernel(PointState st, const uint8_t* __restrict__ mask, int first,
     if (mask && !mask[i]) return;
     PointHot h = st.load(i);
     bool reach = point::dist2((double)h.gx, (double)h.gy, h.d.px, h.d.py) < REACH_RADIUS;
-    point_reset(h, st.cold, i, first || !reach);
+    point_reset<HAZ>(h, st.cold, i, first || !reach, &cfg.haz);
     st.store(i, h);
     if (obs) {
         float o[point::OBS];
         point::sensors(h.d, (double)h.cx, (double)h.cz, h.gx, h.gy, o);
-        if (cfg.obs_flags) { point_obs_row_ext(st, h, i, o, cfg, obs); return; }
+        if (HAZ || cfg.obs_flags) { point_obs_row_ext<HAZ>(st, h, i, o, cfg, obs); return; }
 #pragma unroll
         for (int k = 0; k < point::OBS; ++k) obs[i * point::OBS + k] = o[k];
     }
 }
 
+template <bool HAZ>
 __global__ void __launch_bounds__(STEP_THREADS)
 point_obs_ext_kernel(PointState st, float* __restrict__ obs, EnvCfg cfg) {
     const int64_t i = (int64_t)blockIdx.x * STEP_THREADS + threadIdx.x;
@@ -159,7 +170,7 @@ point_obs_ext_kernel(PointState st, float* __restrict__ obs, EnvCfg cfg) {
     PointHot h = st.load(i);
     float o[point::OBS];
     point::sensors(h.d, (double)h.cx, (double)h.cz, h.gx, h.gy, o);
-    point_obs_row_ext(st, h, i, o, cfg, obs);
+    point_obs_row_ext<HAZ>(st, h, i, o, cfg, obs);
 }
 
 __global__ void __launch_bounds__(STEP_THREADS)
@@ -255,7 +266,8 @@ car_step_kernel(CarSoA st, car::Consts K, EnvCfg cfg, const float2* __restrict__
     }
 }
 
-// optional observation keys (EnvCfg::obs_flags != 0), see point_step_ext_kernel
+// optional observation keys (EnvCfg::obs_flags != 0) or hazards (HAZ), see point_step_ext_kernel
+template <bool HAZ>
 __global__ void __launch_bounds__(CAR_THREADS)
 car_step_ext_kernel(CarSoA st, car::Consts K, EnvCfg cfg, const float2* __restrict__ act,
                     float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ done,
@@ -264,36 +276,44 @@ car_step_ext_kernel(CarSoA st, car::Consts K, EnvCfg cfg, const float2* __restri
     MR_CAR_SCRATCH();
     const int64_t i = (int64_t)blockIdx.x * CAR_THREADS + threadIdx.x;
     if (i >= st.n) return;
-    const int O = obs_dim_ext(car::OBS, 13, 11, cfg.obs_flags, cfg.lidar.num_bins);
+    const int O = row_dim<HAZ>(car::OBS, 13, 11, cfg);
     CarHot h = st.load(i);
     float2 a = act[i];
     float o[car::OBS], tobs[car::OBS];
     CarExt x, tx;
-    StepResult r = car_env_step(K, h, st.cold, i, a.x, a.y, cfg, st.contacts != 0, o, tobs, S, &x, &tx);
+    StepResult r = car_env_step<HAZ>(K, h, st.cold, i, a.x, a.y, cfg, st.contacts != 0, o, tobs, S, &x, &tx,
+                                     hazards_block<HAZ, CAR_OBS_PRE>(obs + i * O, cfg),
+                                     hazards_block<HAZ, CAR_OBS_PRE>(term_obs ? term_obs + i * O : nullptr, cfg));
     st.store(i, h);
-    emit_obs_row<car::OBS, CAR_OBS_PRE, 13, 11>(obs + i * O, o, x, cfg.obs_flags, cfg.lidar);
+    emit_obs_row<car::OBS, CAR_OBS_PRE, 13, 11, HAZ>(obs + i * O, o, x, cfg.obs_flags, cfg.lidar);
     rew[i] = r.rew;
     done[i] = r.done ? 1 : 0;
     trunc[i] = r.trunc ? 1 : 0;
     if (r.done) {
-        if (term_obs) emit_obs_row<car::OBS, CAR_OBS_PRE, 13, 11>(term_obs + i * O, tobs, tx, cfg.obs_flags, cfg.lidar);
+        if (term_obs)
+            emit_obs_row<car::OBS, CAR_OBS_PRE, 13, 11, HAZ>(term_obs + i * O, tobs, tx, cfg.obs_flags, cfg.lidar);
         if (ep_ret) ep_ret[i] = r.ep_r;
         if (ep_len) ep_len[i] = r.ep_l;
     }
 }
 
+template <bool HAZ>
 __device__ __forceinline__ void car_obs_row(const CarHot& h, int64_t i, const float (&o)[car::OBS], const EnvCfg& cfg,
                                             float* __restrict__ obs) {
-    if (cfg.obs_flags) {
+    if (HAZ || cfg.obs_flags) {
         CarExt x;
         car_obs_ext(h, x);
-        emit_obs_row<car::OBS, CAR_OBS_PRE, 13, 11>(obs + i * obs_dim_ext(car::OBS, 13, 11, cfg.obs_flags, cfg.lidar.num_bins),
-                                                    o, x, cfg.obs_flags, cfg.lidar);
+        float* row = obs + i * row_dim<HAZ>(car::OBS, 13, 11, cfg);
+        emit_obs_row<car::OBS, CAR_OBS_PRE, 13, 11, HAZ>(row, o, x, cfg.obs_flags, cfg.lidar);
+        if constexpr (HAZ) {
+            if (float* hb = hazards_block<HAZ, CAR_OBS_PRE>(row, cfg)) car_hazards_lidar(hb, h, cfg, i);
+        }
     } else {
         for (int k = 0; k < car::OBS; ++k) obs[i * car::OBS + k] = o[k];
     }
 }
 
+template <bool HAZ>
 __global__ void __launch_bounds__(CAR_THREADS)
 car_reset_kernel(CarSoA st, car::Consts K, const uint8_t* __restrict__ mask, int first, float* __restrict__ obs,
                  EnvCfg cfg) {
@@ -303,15 +323,16 @@ car_reset_kernel(CarSoA st, car::Consts K, const uint8_t* __restrict__ mask, int
     if (mask && !mask[i]) return;
     CarHot h = st.load(i);
     bool reach = point::dist2((double)h.gx, (double)h.gy, h.s.p[0], h.s.p[1]) < REACH_RADIUS;
-    car_reset(h, st.cold, i, first || !reach);
+    car_reset<HAZ>(h, st.cold, i, first || !reach, &cfg.haz);
     st.store(i, h);
     if (obs) {
         float o[car::OBS];
         car::sensors(K, h.s, (double)h.cx, (double)h.cz, h.gx, h.gy, st.contacts != 0, o, S);
-        car_obs_row(h, i, o, cfg, obs);
+        car_obs_row<HAZ>(h, i, o, cfg, obs);
     }
 }
 
+template <bool HAZ>
 __global__ void __launch_bounds__(CAR_THREADS)
 car_obs_kernel(CarSoA st, car::Consts K, float* __restrict__ obs, EnvCfg cfg) {
     MR_CAR_SCRATCH();
@@ -320,7 +341,7 @@ car_obs_kernel(CarSoA st, car::Consts K, float* __restrict__ obs, EnvCfg cfg) {
     CarHot h = st.load(i);
     float o[car::OBS];
     car::sensors(K, h.s, (double)h.cx, (double)h.cz, h.gx, h.gy, st.contacts != 0, o, S);
-    car_obs_row(h, i, o, cfg, obs);
+    car_obs_row<HAZ>(h, i, o, cfg, obs);
 }
 
 // reference view: qpos(13) = p quat thL thR qb ; qvel(11) = v w sL sR wb ; ctrl goal elapsed ep_ret
@@ -328,10 +349,14 @@ car_obs_kernel(CarSoA st, car::Consts K, float* __restrict__ obs, EnvCfg cfg) {
 static int car_smem_optin() {
     static OncePerDevice once;
     if (once.first()) {
-        MR_CUDA(cudaFuncSetAttribute(car_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CAR_SMEM));
-        MR_CUDA(cudaFuncSetAttribute(car_step_ext_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CAR_SMEM));
-        MR_CUDA(cudaFuncSetAttribute(car_reset_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CAR_SMEM));
-        MR_CUDA(cudaFuncSetAttribute(car_obs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CAR_SMEM));
+        const int b = (int)CAR_SMEM;
+        MR_CUDA(cudaFuncSetAttribute(car_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, b));
+        MR_CUDA(cudaFuncSetAttribute(car_step_ext_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, b));
+        MR_CUDA(cudaFuncSetAttribute(car_step_ext_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, b));
+        MR_CUDA(cudaFuncSetAttribute(car_reset_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, b));
+        MR_CUDA(cudaFuncSetAttribute(car_reset_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, b));
+        MR_CUDA(cudaFuncSetAttribute(car_obs_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, b));
+        MR_CUDA(cudaFuncSetAttribute(car_obs_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, b));
     }
     return MR_OK;
 }
@@ -463,21 +488,23 @@ void mr_env_destroy(mr_env* env) {
     if (!env) return;
     DeviceGuard guard(env->device);
     cudaFree(env->slab);
+    if (env->haz_slab) cudaFree(env->haz_slab);
     if (env->scratch) cudaFree(env->scratch);
     delete env;
 }
 
 int mr_env_obs_dim(const mr_env* env) {
     if (!env) return 0;
-    const int bins = env->cfg.lidar.num_bins;
-    return env->kind == MR_ENV_POINT ? obs_dim_ext(point::OBS, 3, 3, env->cfg.obs_flags, bins)
-                                     : obs_dim_ext(car::OBS, 13, 11, env->cfg.obs_flags, bins);
+    const EnvCfg& c = env->cfg;
+    if (c.haz.num > 0)
+        return env->kind == MR_ENV_POINT ? row_dim<true>(point::OBS, 3, 3, c) : row_dim<true>(car::OBS, 13, 11, c);
+    return env->kind == MR_ENV_POINT ? row_dim<false>(point::OBS, 3, 3, c) : row_dim<false>(car::OBS, 13, 11, c);
 }
 
 int mr_env_set_obs_flags(mr_env* env, unsigned flags) {
     MR_REQUIRE(env, "env is NULL");
     if (flags & ~OBS_ALL_FLAGS) {
-        set_error("unknown observation flag bits 0x%x (1 goal_dist, 2 qpos, 4 qvel, 8 ctrl, 16 goal_lidar)",
+        set_error("unknown observation flag bits 0x%x (1 goal_dist, 2 qpos, 4 qvel, 8 ctrl, 16 goal_lidar, 32 hazards_lidar)",
                   flags & ~OBS_ALL_FLAGS);
         return MR_ERR_UNSUPPORTED;
     }
@@ -494,7 +521,7 @@ int mr_env_set_obs_flags(mr_env* env, unsigned flags) {
 int mr_env_set_lidar(mr_env* env, int num_bins, double max_dist, double exp_gain, int alias) {
     MR_REQUIRE(env, "env is NULL");
     MR_REQUIRE(num_bins >= 1, "lidar_num_bins must be at least 1");
-    if (env->scratch && num_bins != env->cfg.lidar.num_bins && (env->cfg.obs_flags & OBS_GOAL_LIDAR)) {
+    if (env->scratch && num_bins != env->cfg.lidar.num_bins && (env->cfg.obs_flags & (OBS_GOAL_LIDAR | OBS_HAZARDS_LIDAR))) {
         DeviceGuard guard(env->device);   // as in mr_env_set_obs_flags: the rollout scratch has the old row length
         MR_CUDA(cudaDeviceSynchronize());
         MR_CUDA(cudaFree(env->scratch));
@@ -503,6 +530,101 @@ int mr_env_set_lidar(mr_env* env, int num_bins, double max_dist, double exp_gain
     env->cfg.lidar = make_lidar_cfg(num_bins, max_dist, exp_gain, alias);
     return MR_OK;
 }
+int mr_env_set_hazards(mr_env* env, int num, double size, double keepout, double cost, int constrain, int indicator,
+                       const double* locations, int n_loc) {
+    MR_REQUIRE(env, "env is NULL");
+    MR_REQUIRE(num >= 0 && num <= MAX_HAZARDS, "hazards_num must be in 0 .. MR_MAX_HAZARDS (32)");
+    MR_REQUIRE(n_loc >= 0 && n_loc <= num, "more hazards_locations than hazards");
+    MR_REQUIRE(n_loc == 0 || locations, "locations is NULL");
+    MR_REQUIRE(size >= 0.0 && keepout >= 0.0, "hazards_size and hazards_keepout must not be negative");
+    MR_REQUIRE(!constrain || size < ROBOT_KEEPOUT + PLACEMENTS_MARGIN + keepout,
+               "constrain_hazards with hazards_size >= robot_keepout + placements_margin + hazards_keepout: the "
+               "Engine's reset asserts 'World has starting cost!'");
+    DeviceGuard guard(env->device);
+    const int before = mr_env_obs_dim(env);
+    if (env->haz_slab) {
+        MR_CUDA(cudaDeviceSynchronize());   // kernels in flight may still read the old arrays
+        MR_CUDA(cudaFree(env->haz_slab));
+        env->haz_slab = nullptr;
+    }
+    HazardCfg& c = env->cfg.haz;
+    c = HazardCfg{};
+    if (num > 0) {
+        // draw boxes, host float64 like the reference: constrain_placement(placements_extents, keepout), or for a fixed
+        // location constrain_placement((x - k, y - k, x + k, y + k), keepout) with k = keepout + 1e-9
+        double box[MAX_HAZARDS][4];
+        for (int h = 0; h < num; ++h) {
+            if (h < n_loc) {
+                const double x = locations[2 * h], y = locations[2 * h + 1], k = keepout + 1e-9;
+                box[h][0] = (x - k) + keepout; box[h][1] = (y - k) + keepout;
+                box[h][2] = (x + k) - keepout; box[h][3] = (y + k) - keepout;
+            } else {
+                box[h][0] = -2.0 + keepout; box[h][1] = -2.0 + keepout;
+                box[h][2] = 2.0 - keepout; box[h][3] = 2.0 - keepout;
+            }
+        }
+        const size_t pos_b = PointState::align_up((size_t)env->n * num * sizeof(double2));
+        const size_t box_b = PointState::align_up((size_t)num * 4 * sizeof(double));
+        const size_t cost_b = PointState::align_up((size_t)env->n * sizeof(double));
+        const size_t bytes = pos_b + box_b + cost_b + sizeof(unsigned long long);
+        void* slab = nullptr;
+        cudaError_t err = cudaMalloc(&slab, bytes);
+        if (err != cudaSuccess) {
+            set_error("cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(err));
+            return MR_ERR_ALLOC;
+        }
+        env->haz_slab = slab;
+        char* p = static_cast<char*>(slab);
+        MR_CUDA(cudaMemset(p, 0, bytes));
+        MR_CUDA(cudaMemcpy(p + pos_b, box, (size_t)num * 4 * sizeof(double), cudaMemcpyHostToDevice));
+        c.num = num;
+        c.flags = (constrain ? HAZ_CONSTRAIN : 0u) | (indicator ? HAZ_INDICATOR : 0u);
+        c.size = size; c.keepout = keepout; c.cost = cost;
+        c.pos = reinterpret_cast<double2*>(p);
+        c.box = reinterpret_cast<const double*>(p + pos_b);
+        c.cost_out = reinterpret_cast<double*>(p + pos_b + box_b);
+        c.failures = reinterpret_cast<unsigned long long*>(p + pos_b + box_b + cost_b);
+    }
+    if (env->scratch && mr_env_obs_dim(env) != before) {   // as in mr_env_set_obs_flags
+        MR_CUDA(cudaDeviceSynchronize());
+        MR_CUDA(cudaFree(env->scratch));
+        env->scratch = nullptr;
+    }
+    return MR_OK;
+}
+
+int mr_env_get_hazards(mr_env* env, double* out, void* stream) {
+    MR_REQUIRE(env && out, "NULL argument");
+    const HazardCfg& c = env->cfg.haz;
+    if (c.num > 0)
+        MR_CUDA(cudaMemcpyAsync(out, c.pos, (size_t)env->n * c.num * sizeof(double2), cudaMemcpyDeviceToDevice,
+                                (cudaStream_t)stream));
+    return MR_OK;
+}
+
+int mr_env_get_cost(mr_env* env, double* out, void* stream) {
+    MR_REQUIRE(env && out, "NULL argument");
+    const HazardCfg& c = env->cfg.haz;
+    if (c.num > 0)
+        MR_CUDA(cudaMemcpyAsync(out, c.cost_out, (size_t)env->n * sizeof(double), cudaMemcpyDeviceToDevice,
+                                (cudaStream_t)stream));
+    else
+        MR_CUDA(cudaMemsetAsync(out, 0, (size_t)env->n * sizeof(double), (cudaStream_t)stream));
+    return MR_OK;
+}
+
+int mr_env_layout_failures(mr_env* env, int64_t* out) {
+    MR_REQUIRE(env && out, "NULL argument");
+    *out = 0;
+    if (env->cfg.haz.num == 0) return MR_OK;
+    DeviceGuard guard(env->device);
+    unsigned long long v = 0;
+    MR_CUDA(cudaDeviceSynchronize());
+    MR_CUDA(cudaMemcpy(&v, env->cfg.haz.failures, sizeof(v), cudaMemcpyDeviceToHost));
+    *out = (int64_t)v;
+    return MR_OK;
+}
+
 int mr_env_state_dim(const mr_env* env) {
     return env ? (env->kind == MR_ENV_POINT ? POINT_STATE_DIM : CAR_STATE_DIM) : 0;
 }
@@ -530,13 +652,15 @@ int mr_env_seed(mr_env* env, const uint64_t* h_pcg_init, const uint64_t* h_pcg_g
 int mr_env_reset(mr_env* env, const uint8_t* mask, int first, float* obs_out, void* stream) {
     MR_REQUIRE(env, "env is NULL");
     cudaStream_t s = (cudaStream_t)stream;
-    if (env->kind == MR_ENV_POINT)
-        point_reset_kernel<<<ceil_div(env->n, STEP_THREADS), STEP_THREADS, 0, s>>>(env->point, mask, first, obs_out,
-                                                                                   env->cfg);
-    else {
+    const bool haz = env->cfg.haz.num > 0;
+    if (env->kind == MR_ENV_POINT) {
+        auto kern = haz ? point_reset_kernel<true> : point_reset_kernel<false>;
+        kern<<<ceil_div(env->n, STEP_THREADS), STEP_THREADS, 0, s>>>(env->point, mask, first, obs_out, env->cfg);
+    } else {
         if (car_smem_optin() != MR_OK) return MR_ERR_CUDA;
-        car_reset_kernel<<<ceil_div(env->n, CAR_THREADS), CAR_THREADS, CAR_SMEM, s>>>(env->car, env->carK, mask, first, obs_out,
-                                                                                      env->cfg);
+        auto kern = haz ? car_reset_kernel<true> : car_reset_kernel<false>;
+        kern<<<ceil_div(env->n, CAR_THREADS), CAR_THREADS, CAR_SMEM, s>>>(env->car, env->carK, mask, first, obs_out,
+                                                                          env->cfg);
     }
     MR_CHECK_LAUNCH();
     return MR_OK;
@@ -546,15 +670,19 @@ int mr_env_step(mr_env* env, const float* act, float* obs, float* rew, uint8_t* 
                 uint8_t* trunc, float* term_obs, double* ep_ret, int32_t* ep_len, void* stream) {
     MR_REQUIRE(env && act && obs && rew && done && trunc, "NULL argument");
     cudaStream_t s = (cudaStream_t)stream;
-    if (env->cfg.obs_flags) {
+    const bool haz = env->cfg.haz.num > 0;   // the layout changes the heading: never the default kernels
+    if (env->cfg.obs_flags || haz) {
         const float2* a2 = reinterpret_cast<const float2*>(act);
         if (env->kind == MR_ENV_POINT) {
-            point_step_ext_kernel<<<ceil_div(env->n, STEP_THREADS), STEP_THREADS, 0, s>>>(
-                env->point, env->cfg, a2, obs, rew, done, trunc, term_obs, ep_ret, ep_len);
+            auto kern = haz ? point_step_ext_kernel<true> : point_step_ext_kernel<false>;
+            kern<<<ceil_div(env->n, STEP_THREADS), STEP_THREADS, 0, s>>>(env->point, env->cfg, a2, obs, rew, done,
+                                                                         trunc, term_obs, ep_ret, ep_len);
         } else {
             if (car_smem_optin() != MR_OK) return MR_ERR_CUDA;
-            car_step_ext_kernel<<<ceil_div(env->n, CAR_THREADS), CAR_THREADS, CAR_SMEM, s>>>(
-                env->car, env->carK, env->cfg, a2, obs, rew, done, trunc, term_obs, ep_ret, ep_len);
+            auto kern = haz ? car_step_ext_kernel<true> : car_step_ext_kernel<false>;
+            kern<<<ceil_div(env->n, CAR_THREADS), CAR_THREADS, CAR_SMEM, s>>>(env->car, env->carK, env->cfg, a2, obs,
+                                                                              rew, done, trunc, term_obs, ep_ret,
+                                                                              ep_len);
         }
     } else if (env->kind == MR_ENV_POINT) {
         // tuning knobs (measured on B200 at 4M envs, profiles/r01_env_step_sweep.txt): 5 blocks per SM
@@ -583,15 +711,20 @@ int mr_env_step(mr_env* env, const float* act, float* obs, float* rew, uint8_t* 
 int mr_env_get_obs(mr_env* env, float* obs_out, void* stream) {
     MR_REQUIRE(env && obs_out, "NULL argument");
     cudaStream_t s = (cudaStream_t)stream;
+    const bool haz = env->cfg.haz.num > 0;
     if (env->kind == MR_ENV_POINT) {
-        if (env->cfg.obs_flags)
-            point_obs_ext_kernel<<<ceil_div(env->n, STEP_THREADS), STEP_THREADS, 0, s>>>(env->point, obs_out, env->cfg);
+        if (haz)
+            point_obs_ext_kernel<true><<<ceil_div(env->n, STEP_THREADS), STEP_THREADS, 0, s>>>(env->point, obs_out,
+                                                                                              env->cfg);
+        else if (env->cfg.obs_flags)
+            point_obs_ext_kernel<false><<<ceil_div(env->n, STEP_THREADS), STEP_THREADS, 0, s>>>(env->point, obs_out,
+                                                                                               env->cfg);
         else
             point_obs_kernel<<<ceil_div(env->n, STEP_THREADS), STEP_THREADS, 0, s>>>(env->point, obs_out);
     } else {
         if (car_smem_optin() != MR_OK) return MR_ERR_CUDA;
-        car_obs_kernel<<<ceil_div(env->n, CAR_THREADS), CAR_THREADS, CAR_SMEM, s>>>(env->car, env->carK, obs_out,
-                                                                                    env->cfg);
+        auto kern = haz ? car_obs_kernel<true> : car_obs_kernel<false>;
+        kern<<<ceil_div(env->n, CAR_THREADS), CAR_THREADS, CAR_SMEM, s>>>(env->car, env->carK, obs_out, env->cfg);
     }
     MR_CHECK_LAUNCH();
     return MR_OK;

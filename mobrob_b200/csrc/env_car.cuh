@@ -71,7 +71,10 @@ struct CarSoA {
     }
 };
 
-__host__ __device__ inline void car_reset(CarHot& h, const EnvCold& cold, int64_t i, bool full) {
+// see point_reset
+template <bool HAZ = false>
+__host__ __device__ inline void car_reset(CarHot& h, const EnvCold& cold, int64_t i, bool full,
+                                          const HazardCfg* hz = nullptr) {
     if (full) {
         // Engine.reset() once (wrapper.py:190); CarEnv.set_pos only rewrites qpos[0:2] (wrapper.py:320-326)
         int64_t seed = cold.engine_seed[i] + 1;
@@ -80,7 +83,9 @@ __host__ __device__ inline void car_reset(CarHot& h, const EnvCold& cold, int64_
         float x = (float)g.uniform((double)cold.spaces[0], (double)cold.spaces[2]);
         float y = (float)g.uniform((double)cold.spaces[1], (double)cold.spaces[3]);
         store_pcg(cold.pcg_init, i, g);
-        double heading = engine_heading((uint32_t)seed);
+        double heading;
+        if constexpr (HAZ) heading = hazard_reset_heading(*hz, (uint32_t)seed, i);
+        else heading = engine_heading((uint32_t)seed);
         car::State& s = h.s;
         s.p[0] = (double)x; s.p[1] = (double)y; s.p[2] = 0.1;  // body pos z (car.xml:12)
         double sh, ch;
@@ -129,10 +134,21 @@ __host__ __device__ inline void car_obs_ext(const CarHot& h, CarExt& x) {
     x.qvel[6] = (float)s.s[0]; x.qvel[7] = (float)s.s[1];
 }
 
+// the hazards_lidar block of the car at its current pose: R^T (h_x - p_x, h_y - p_y, -p_z), as car_obs_ext's goal
+__host__ __device__ inline void car_hazards_lidar(float* dst, const CarHot& h, const EnvCfg& cfg, int64_t i) {
+    double R[9];
+    car::quat2mat(h.s.q, R);
+    const double m[6] = {R[0], R[3], R[6], R[1], R[4], R[7]};
+    hazards_lidar(dst, cfg.haz.pos + i * cfg.haz.num, cfg.haz.num, m, h.s.p[0], h.s.p[1], h.s.p[2], cfg.lidar);
+}
+
+// see point_env_step
+template <bool HAZ = false>
 __host__ __device__ inline StepResult car_env_step(const car::Consts& K, CarHot& h, const EnvCold& cold, int64_t i,
                                           float a0, float a1, const EnvCfg& cfg, bool contacts, float* obs,
                                           float* term_obs, const car::Scratch& S, CarExt* ext = nullptr,
-                                          CarExt* term_ext = nullptr) {
+                                          CarExt* term_ext = nullptr, float* haz_obs = nullptr,
+                                          float* haz_term = nullptr) {
     StepResult r;
     h.cx = fminf(fmaxf(a0, -1.f), 1.f);
     h.cz = fminf(fmaxf(a1, -1.f), 1.f);
@@ -157,12 +173,22 @@ __host__ __device__ inline StepResult car_env_step(const car::Consts& K, CarHot&
     r.ep_l = h.elapsed;
     car::sensors(K, h.s, (double)h.cx, (double)h.cz, h.gx, h.gy, contacts, obs, S);
     if (ext) car_obs_ext(h, *ext);
+    if constexpr (HAZ) {
+        if (cfg.haz.flags & HAZ_CONSTRAIN)
+            cfg.haz.cost_out[i] = hazard_cost(cfg.haz, cfg.haz.pos + i * cfg.haz.num, h.s.p[0], h.s.p[1]);
+    }
     if (r.done) {
         for (int k = 0; k < car::OBS; ++k) term_obs[k] = obs[k];
         if (ext) *term_ext = *ext;
-        car_reset(h, cold, i, !r.reach);
+        if constexpr (HAZ) {
+            if (haz_term) car_hazards_lidar(haz_term, h, cfg, i);
+        }
+        car_reset<HAZ>(h, cold, i, !r.reach, &cfg.haz);
         car::sensors(K, h.s, (double)h.cx, (double)h.cz, h.gx, h.gy, contacts, obs, S);
         if (ext) car_obs_ext(h, *ext);
+    }
+    if constexpr (HAZ) {
+        if (haz_obs) car_hazards_lidar(haz_obs, h, cfg, i);
     }
     return r;
 }

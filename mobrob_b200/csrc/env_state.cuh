@@ -131,6 +131,7 @@ struct mr_env {
     mr::CarSoA car;
     mr::car::Consts carK;
     void* scratch = nullptr;  // lazily allocated by mr_rollout_unfused
+    void* haz_slab = nullptr; // mr_env_set_hazards: EnvCfg::haz's arrays
     int step_flip = 0;        // env-step kernels alternate the block order (L2 keeps the tail of the last step)
 };
 

@@ -437,7 +437,7 @@ extern "C" int mr_evaluate(mr_env* env, const float* params, int deterministic, 
     A.S = reinterpret_cast<unsigned long long*>(steps_taken);
     A.status = status;
     A.seed = seed; A.noise_offset = noise_offset; A.env_offset = env_offset;
-    if (env->kind == MR_ENV_POINT && env->cfg.obs_flags == 0) {
+    if (env->kind == MR_ENV_POINT && env->cfg.obs_flags == 0 && env->cfg.haz.num == 0) {
         MR_CUDA(cudaMemsetAsync(steps_taken, 0, sizeof(int64_t), s));
         MR_CUDA(cudaMemsetAsync(status, 0, sizeof(int), s));
         return eval_fused(env, A, s);
@@ -533,7 +533,7 @@ extern "C" int mr_follow_waypoints(mr_env* env, const float* params, int determi
     MR_CUDA(cudaMemsetAsync(ret, 0, (size_t)N * sizeof(double), s));
     MR_CUDA(cudaMemsetAsync(steps_taken, 0, (size_t)N * sizeof(int32_t), s));
     const int stochastic = deterministic ? 0 : 1;
-    if (env->kind != MR_ENV_POINT || env->cfg.obs_flags != 0)
+    if (env->kind != MR_ENV_POINT || env->cfg.obs_flags != 0 || env->cfg.haz.num != 0)
         return waypoints_per_step(env, params, stochastic, waypoints, K, max_steps, seed, noise_offset, env_offset,
                                   last_obs, arrival, ret, steps_taken, positions, s);
     WaypointArgs A;

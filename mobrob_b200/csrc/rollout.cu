@@ -316,7 +316,8 @@ extern "C" int mr_rollout(mr_env* env, const float* params, int64_t T, float* la
                    logp && last_val && last_done && ep_ret && ep_len && ep_steps && ep_r && ep_l && ep_count,
                "NULL argument");
     MR_REQUIRE(env->kind == MR_ENV_POINT, "fused rollout is built for the point env");
-    MR_REQUIRE(env->cfg.obs_flags == 0, "fused rollout is built for the default observation (use mr_rollout_unfused)");
+    MR_REQUIRE(env->cfg.obs_flags == 0 && env->cfg.haz.num == 0,
+               "fused rollout is built for the default observation without hazards (use mr_rollout_unfused)");
     MR_REQUIRE(T > 0 && T <= INT32_MAX && ring_cap > 0, "T must be in 1 .. 2^31 - 1 and ring_cap positive");
     RolloutArgs A;
     A.st = env->point;

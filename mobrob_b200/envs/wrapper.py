@@ -14,6 +14,7 @@ from abc import ABC, abstractmethod
 import numpy as np
 import torch
 
+from .. import _lib
 from ..spaces import Box
 from ..vec_env import GpuVecEnv
 
@@ -90,7 +91,10 @@ class EnvWrapper(ABC):
         obs = self._physics_step(action)
         reward = self.reward_fn()
         terminated = self.terminate_on_goal and self.reached()
-        return obs, reward, terminated, False, {"cost": 0.0}
+        return obs, reward, terminated, False, self._cost_info()
+
+    def _cost_info(self) -> dict:
+        return {"cost": 0.0}
 
     def reset(self, init_pos=None, *args, **kwargs):
         if "seed" in kwargs:
@@ -129,7 +133,8 @@ class MujocoGoalEnv(EnvWrapper, ABC):
     def get_robot_config(self) -> dict:
         """Engine config of the robot (wrapper.py:235-240, 293-317).  A subclass may switch on observe_goal_dist /
         observe_qpos / observe_qvel / observe_ctrl (engine.py:125, 140-142) and observe_goal_lidar with its
-        lidar_num_bins / lidar_max_dist / lidar_exp_gain / lidar_alias settings; other observation keys are fixed."""
+        lidar_num_bins / lidar_max_dist / lidar_exp_gain / lidar_alias settings, and add hazards (hazards_num and
+        the other hazard keys of vec_env.HAZARD_DEFAULTS, observe_hazards); other observation keys are fixed."""
         return {"robot_base": f"xmls/{self.ENV_NAME}.xml", "sensors_obs": self.BASE_SENSORS,
                 "observe_com": False, "observe_goal_comp": True}
 
@@ -172,6 +177,27 @@ class MujocoGoalEnv(EnvWrapper, ABC):
     def get_pos(self) -> np.ndarray:
         return self.env.get_pos().cpu().numpy()[0].copy()
 
+    # device full resets add this to Engine._seed: PointEnv.set_pos resets the Engine a second time
+    LAYOUT_SEED_STEP = 1
+
+    def _engine_layout(self, engine_seed: int) -> np.ndarray:
+        """Engine.reset with hazards: lays out this env's hazards with Engine._seed = engine_seed on the device (the
+        batched env's full reset) and returns the reference-view state that reset leaves, whose heading is the
+        layout's.  The caller writes the state it wants back."""
+        e, stream = self.env, self.env._stream()
+        zeros = np.zeros((1, 4), np.uint64)
+        eng = np.array([engine_seed - self.LAYOUT_SEED_STEP], np.int64)
+        _lib.check(e.lib.mr_env_seed(e._h, zeros.ctypes.data, zeros.ctypes.data, eng.ctypes.data, stream))
+        _lib.check(e.lib.mr_env_reset(e._h, None, 1, None, stream))
+        e._check_layouts()
+        return self._state()
+
+    def _cost_info(self) -> dict:
+        if not self.env._constrain:
+            return {"cost": 0.0}
+        c = float(self.env.cost.cpu().numpy()[0])
+        return {"cost": c, "cost_hazards": c}
+
     def get_obs(self) -> np.ndarray:
         return self.env.get_obs_tensor().cpu().numpy()[0]
 
@@ -204,13 +230,17 @@ class PointEnv(MujocoGoalEnv):
     def _engine_reset(self):
         self._engine_seed += 1
 
+    LAYOUT_SEED_STEP = 2
+
     def set_pos(self, pos):
-        # PointEnv.set_pos rebuilds the Engine (wrapper.py:301-305): fresh sim, new heading
+        # PointEnv.set_pos rebuilds the Engine (wrapper.py:301-305): fresh sim, new heading (and hazards)
         self._engine_seed += 1
         s = self._state()
+        heading = (self._engine_layout(self._engine_seed)[8] if self.env.hazards_num
+                   else _engine_heading(self._engine_seed))
         s[0:6] = 0.0
         s[6:8] = np.asarray(pos, dtype=np.float64)[:2]
-        s[8] = _engine_heading(self._engine_seed)
+        s[8] = heading
         s[9:11] = 0.0
         self._write_state(s)
 
@@ -240,11 +270,15 @@ class CarEnv(MujocoGoalEnv):
         # Engine.reset(): new MjSim -- default pose at the origin, body z from car.xml:12, heading
         # drawn from RandomState(_seed), zero velocities and ctrl (engine.py:1000-1021, world.py:52-54)
         self._engine_seed += 1
-        heading = _engine_heading(self._engine_seed)
         s = self._state()
+        if self.env.hazards_num:
+            quat = self._engine_layout(self._engine_seed)[3:7]
+        else:
+            heading = _engine_heading(self._engine_seed)
+            quat = (np.cos(0.5 * heading), 0.0, 0.0, np.sin(0.5 * heading))
         s[0:24] = 0.0
         s[2] = 0.1
-        s[3], s[6] = np.cos(0.5 * heading), np.sin(0.5 * heading)
+        s[3], s[6] = quat[0], quat[3]
         s[9] = 1.0            # ball joint quaternion
         s[24:26] = 0.0        # data.ctrl
         self._write_state(s)

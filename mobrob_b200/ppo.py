@@ -248,7 +248,8 @@ class PPO:
             self._last_obs = env.reset_tensor().clone()
             self._last_episode_starts = torch.ones(env.num_envs, dtype=torch.float32, device=self.device)
         seed = int(self.seed if self.seed is not None else 0)
-        fused = env.env_name == "point" and self.rollout_mode == "fused" and not getattr(env, "obs_flags", 0)
+        fused = (env.env_name == "point" and self.rollout_mode == "fused" and not getattr(env, "obs_flags", 0)
+                 and not getattr(env, "hazards_num", 0))
         fn = self.lib.mr_rollout if fused else self.lib.mr_rollout_unfused
         _lib.check(fn(
             env._h, self.updater.params.data_ptr(), self.n_steps, self._last_obs.data_ptr(),

@@ -20,10 +20,11 @@ ENV_KINDS = {"point": 0, "car": 1}
 OBS_DIMS = {"point": 14, "car": 26}
 # Engine config keys (engine.py:124-144) the batched env implements -> mr_env_set_obs_flags bits; every other
 # observe_* key must keep the value the reference's get_robot_config leaves it at
-OBS_FLAG_BITS = {"observe_goal_dist": 1, "observe_qpos": 2, "observe_qvel": 4, "observe_ctrl": 8, "observe_goal_lidar": 16}
+OBS_FLAG_BITS = {"observe_goal_dist": 1, "observe_qpos": 2, "observe_qvel": 4, "observe_ctrl": 8, "observe_goal_lidar": 16,
+                 "observe_hazards": 32}
 _FIXED_OBSERVE = {"observe_sensors": True, "observe_goal_comp": True, "observe_com": False,
                   "observe_box_comp": False, "observe_box_lidar": False, "observe_circle": False,
-                  "observe_remaining": False, "observe_walls": False, "observe_hazards": False, "observe_vases": False,
+                  "observe_remaining": False, "observe_walls": False, "observe_vases": False,
                   "observe_pillars": False, "observe_buttons": False, "observe_gremlins": False,
                   "observe_vision": False, "observe_freejoint": False}
 
@@ -33,6 +34,8 @@ def obs_flags_of(robot_config: dict | None) -> int:
     sensors_obs, box_*) are the reference's constants for the robot and are ignored."""
     flags = 0
     for key, value in (robot_config or {}).items():
+        if key == "observe_hazards" and value and not (robot_config.get("hazards_num") or 0):
+            raise NotImplementedError("observe_hazards=True needs hazards_num > 0 (the lidar of no hazards is not built)")
         if key in OBS_FLAG_BITS:
             flags |= OBS_FLAG_BITS[key] if value else 0
         elif key in _FIXED_OBSERVE and bool(value) != _FIXED_OBSERVE[key]:
@@ -63,6 +66,45 @@ def lidar_of(robot_config: dict | None) -> tuple[int, float | None, float, bool]
             bool(cfg["lidar_alias"]))
 
 
+# Safety Gym's Engine.DEFAULT hazard settings (parity unpinned: restated like LIDAR_DEFAULTS).  observe_hazards is read
+# by obs_flags_of; the lidar settings are LIDAR_DEFAULTS'.
+HAZARD_DEFAULTS = {"hazards_num": 0, "hazards_size": 0.3, "hazards_keepout": 0.4, "hazards_cost": 1.0,
+                   "hazards_locations": [], "hazards_placements": None, "observe_hazards": False,
+                   "constrain_hazards": False, "constrain_indicator": True}
+MAX_HAZARDS = 32                                   # MR_MAX_HAZARDS
+ROBOT_KEEPOUT, PLACEMENTS_MARGIN = 0.4, 0.0        # Engine.DEFAULT
+
+
+class ResamplingError(AssertionError):
+    """Engine.build_layout found no layout of the objects in 10 000 attempts (safety_gym's ResamplingError)."""
+
+
+def hazards_of(robot_config: dict | None) -> dict | None:
+    """Engine(config) hazard keys -> the mr_env_set_hazards settings, defaults filled in; None without hazards."""
+    cfg = {**HAZARD_DEFAULTS, **{k: v for k, v in (robot_config or {}).items() if k in HAZARD_DEFAULTS}}
+    num = cfg["hazards_num"]
+    if isinstance(num, bool) or not isinstance(num, (int, np.integer)) or not 0 <= num <= MAX_HAZARDS:
+        raise ValueError(f"hazards_num={num!r}: must be an integer in 0 .. {MAX_HAZARDS}")
+    if cfg["hazards_placements"] is not None:
+        raise NotImplementedError("hazards_placements regions are not available on the B200 path; use "
+                                  "hazards_locations or the default placement over the whole floor")
+    if num == 0:
+        return None
+    locs = np.asarray(cfg["hazards_locations"], dtype=np.float64).reshape(-1, 2)
+    if len(locs) > num:
+        raise ValueError(f"{len(locs)} hazards_locations for hazards_num={num}")
+    size, keepout = float(cfg["hazards_size"]), float(cfg["hazards_keepout"])
+    if size < 0 or keepout < 0:
+        raise ValueError("hazards_size and hazards_keepout must not be negative")
+    constrain = bool(cfg["constrain_hazards"])
+    if constrain and size >= ROBOT_KEEPOUT + PLACEMENTS_MARGIN + keepout:
+        # the robot's layout position keeps robot_keepout + margin + hazards_keepout from every hazard
+        raise ValueError(f"hazards_size={size} >= robot_keepout + placements_margin + hazards_keepout with "
+                         f"constrain_hazards: the Engine's reset would fail its assertion 'World has starting cost!'")
+    return {"num": int(num), "size": size, "keepout": keepout, "cost": float(cfg["hazards_cost"]),
+            "constrain": constrain, "indicator": bool(cfg["constrain_indicator"]), "locations": locs}
+
+
 class GpuVecEnv:
     def __init__(self, env_name: str = "point", n_envs: int = 1, seed: int | None = 0,
                  time_limit: int | None = 1000, terminate_on_goal: bool = True,
@@ -89,11 +131,21 @@ class GpuVecEnv:
         self.obs_flags = obs_flags_of(robot_config)
         if self.obs_flags:
             _lib.check(self.lib.mr_env_set_obs_flags(h, self.obs_flags))
-        # the lidar keys are read only with observe_goal_lidar on (the Engine ignores them otherwise)
-        self.lidar = lidar_of(robot_config) if self.obs_flags & OBS_FLAG_BITS["observe_goal_lidar"] else None
+        # the lidar keys are read only with a lidar on (the Engine ignores them otherwise)
+        lidars = OBS_FLAG_BITS["observe_goal_lidar"] | OBS_FLAG_BITS["observe_hazards"]
+        self.lidar = lidar_of(robot_config) if self.obs_flags & lidars else None
         if self.lidar:
             bins, max_dist, gain, alias = self.lidar
             _lib.check(self.lib.mr_env_set_lidar(h, bins, max_dist or 0.0, gain, int(alias)))
+        self.hazards = hazards_of(robot_config)
+        self.hazards_num = self.hazards["num"] if self.hazards else 0
+        if self.hazards:
+            hz = self.hazards
+            locs = np.ascontiguousarray(hz["locations"])
+            _lib.check(self.lib.mr_env_set_hazards(h, hz["num"], hz["size"], hz["keepout"], hz["cost"],
+                                                   int(hz["constrain"]), int(hz["indicator"]),
+                                                   locs.ctypes.data if len(locs) else None, len(locs)))
+        self._constrain = bool(self.hazards and self.hazards["constrain"])
         self.obs_dim = int(self.lib.mr_env_obs_dim(h))
         self.state_dim = int(self.lib.mr_env_state_dim(h))
         self.observation_space = Box(-np.inf, np.inf, (self.obs_dim,), np.float32)
@@ -153,7 +205,17 @@ class GpuVecEnv:
         return self.obs
 
     def reset(self) -> np.ndarray:
-        return self.reset_tensor().cpu().numpy()
+        obs = self.reset_tensor().cpu().numpy()
+        self._check_layouts()
+        return obs
+
+    def _check_layouts(self):
+        if self.hazards_num:
+            n = ctypes.c_int64()
+            _lib.check(self.lib.mr_env_layout_failures(self._h, ctypes.byref(n)))
+            if n.value:
+                raise ResamplingError(f"Failed to sample layout of objects ({n.value} full resets found no layout "
+                                      f"in 10000 attempts)")
 
     # -- stepping ---------------------------------------------------------------------------
     def step_tensor(self, actions: torch.Tensor):
@@ -195,6 +257,11 @@ class GpuVecEnv:
         else:
             for d in infos:
                 d["TimeLimit.truncated"] = False
+        if self.hazards_num:
+            self._check_layouts()
+        if self._constrain:   # Engine.cost: only cost_hazards contributes, so cost == cost_hazards
+            for d, c in zip(infos, self.cost.cpu().numpy().tolist()):
+                d["cost"] = d["cost_hazards"] = c
         return obs_h, rew_h, done_h, infos
 
     def step(self, actions):
@@ -249,6 +316,21 @@ class GpuVecEnv:
         """[num_envs, 2] float32 on the device: each env's current goal (EnvWrapper.get_goal)."""
         slot = 11 if self.env_name == "point" else 26   # goal_xy in the reference-view state
         return self.get_state()[:, slot:slot + 2].to(torch.float32)
+
+    # -- hazards -------------------------------------------------------------------------------------------------------
+    @property
+    def cost(self) -> torch.Tensor:
+        """[num_envs] float64 on the device: info["cost"] of each env's last step (0 before the first step and without
+        constrain_hazards)."""
+        out = torch.empty(self.num_envs, dtype=torch.float64, device=self.device)
+        _lib.check(self.lib.mr_env_get_cost(self._h, out.data_ptr(), self._stream()))
+        return out
+
+    def get_hazards(self) -> torch.Tensor:
+        """[num_envs, hazards_num, 2] float64 on the device: each env's hazard xy, laid out at its last full reset."""
+        out = torch.zeros((self.num_envs, self.hazards_num, 2), dtype=torch.float64, device=self.device)
+        _lib.check(self.lib.mr_env_get_hazards(self._h, out.data_ptr(), self._stream()))
+        return out
 
     def set_contacts(self, enabled: bool):
         """car only: switch the floor contacts off for contact-free parity trajectories."""
